@@ -27,10 +27,7 @@ struct AsHandle {
                        // kernel after the gather kernel (ALLSTEPS_PDL, default 2; 0 = plain stream order)
   const void* lean_probe_ptr;  // last contact matrix whose memory type was looked up (pinned host => lean k_prepare)
   bool lean_probe_host;
-  int64_t prepare_min_envs;  // from this many envs on the scattered reads of a step go to k_prepare*
-  int allow_self_finish, allow_pre;  // A/B knobs (ALLSTEPS_SELF_FINISH, ALLSTEPS_PRE; default 1)
   int regen_mode;      // shape of the regeneration kernel: 0 = by list length, 1 = warp per env, 2 = thread per env (ALLSTEPS_REGEN_MODE)
-  int prefetch_tiles;  // L2 prefetch distance of the step kernel, in 128-env tiles (about one wave of CTAs)
   cudaEvent_t ev_start, ev_stop;  // optional timing hook around k_step<fused>
   PeerArgs peer;        // world > 0 after as_peer_create; buf[] complete after as_peer_connect
   bool peer_connected;
@@ -84,11 +81,12 @@ int check_peer(const AsHandle* h) {
 
 int num_tiles(int64_t n) { return static_cast<int>((n + kTile - 1) / kTile); }
 
-// Below this batch size the step is launch-latency bound (working set in L2, a handful of CTAs per SM): one launch
-// fewer beats the better latency hiding of the separate gather kernel (measured, us per step with / without k_prepare*:
-// 32 768 envs 22.1 / 22.0, 65 536 envs 25.9 / 27.6, 131 072 envs 40.9 / 47.5, 524 288 envs 107 / 130).
 constexpr int64_t kRegenByWarpMaxEnvs = 1 << 15;  // k_reset_rows: a warp per env up to this batch size (profiles/r02_experiments.txt, 12)
-constexpr int64_t kSeparateGatherMinEnvsDefault = 1 << 16;  // (ALLSTEPS_PREPARE_MIN_ENVS overrides: tuning knob)
+// From this batch size on the scattered reads of a step go to k_prepare*.  Below it the step is launch-latency bound
+// (working set in L2, a handful of CTAs per SM): one launch fewer beats the better latency hiding of the separate gather
+// kernel (measured, us per step with / without k_prepare*: 32 768 envs 22.1 / 22.0, 65 536 envs 25.9 / 27.6,
+// 131 072 envs 40.9 / 47.5, 524 288 envs 107 / 130).
+constexpr int64_t kSeparateGatherMinEnvs = 1 << 16;
 
 // Contact matrices in pinned host memory (zero-copy ingest): every load of the gather is a PCIe request, so k_prepare*
 // fetches the current stone's vectors only and the step kernel instantiation with its own gathers is used.
@@ -105,8 +103,8 @@ bool contact_in_host_memory(AsHandle* h, const AsStateIn* in) {
 
 // k_prepare*: contact norms of the current / following stone, stale stone windows, optionally the three body rows out
 // of a strided body tensor (`gather_body`), for batches that are not launch-bound.
-int launch_prepare(AsHandle* h, const AsStateIn* in, cudaStream_t s, bool gather_body = false) {
-  if (h->num_envs < h->prepare_min_envs) return AS_OK;
+int launch_prepare(AsHandle* h, const AsStateIn* in, cudaStream_t s, bool gather_body) {
+  if (h->num_envs < kSeparateGatherMinEnvs) return AS_OK;
   PrepareArgs p;
   p.in = *in;
   p.ws = h->ws;
@@ -244,8 +242,7 @@ StepArgs make_step_args(AsHandle* h, const AsStateIn* in, const float* actions, 
   if (dense(actions, actions_stride, kJ)) bits |= kDenseAct;
   if (out && dense(out->obs, kObs, kObs)) bits |= kDenseObs;
   a.dense16 = bits;
-  a.use_pre = h->num_envs >= h->prepare_min_envs ? 1 : 0;
-  a.prefetch_tiles = h->prefetch_tiles;
+  a.use_pre = h->num_envs >= kSeparateGatherMinEnvs ? 1 : 0;
   return a;
 }
 
@@ -285,23 +282,114 @@ cudaError_t launch_dependent(void (*kernel)(KArgs...), unsigned grid, unsigned b
   return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
+using StepKernel = void (*)(StepArgs);
+
+// The families of k_step instantiations (process_tile describes FAST, PACKED and PRE).
+enum StepKind {
+  kRagged,      // the one-CTA launch of a ragged last tile; division flavour read at run time (EXACT = 2)
+  kRuntimeDiv,  // full tiles, division flavour read at run time: pass 2, true divisions, pass 1 not prepared
+  kTwoFma,      // full tiles of a fused step that gathers its contact vectors itself, two-FMA quotients; FAST / PACKED
+  kPrepared,    // full tiles behind k_prepare*, two-FMA quotients (PRE); FAST / PACKED variants
+};
+
+// Every k_step instantiation the library launches.  select_step picks from this table alone and as_create sets the
+// dynamic shared-memory limit of every entry, so whatever can be selected can be launched.
+struct StepVariant {
+  int mode;  // StepMode
+  StepKind kind;
+  bool fast, packed;
+  StepKernel kernel;
+};
+const StepVariant kStepVariants[] = {
+    {kModeFused, kRagged, false, false, k_step<kModeFused, 2, false>},
+    {kModeFused, kRuntimeDiv, false, false, k_step<kModeFused, 2, true>},
+    {kModeFused, kTwoFma, false, false, k_step<kModeFused, 0, true, false, false>},
+    {kModeFused, kTwoFma, false, true, k_step<kModeFused, 0, true, false, true>},
+    {kModeFused, kTwoFma, true, false, k_step<kModeFused, 0, true, true, false>},
+    {kModeFused, kTwoFma, true, true, k_step<kModeFused, 0, true, true, true>},
+    {kModeFused, kPrepared, false, false, k_step<kModeFused, 0, true, false, false, true>},
+    {kModeFused, kPrepared, false, true, k_step<kModeFused, 0, true, false, true, true>},
+    {kModeFused, kPrepared, true, false, k_step<kModeFused, 0, true, true, false, true>},
+    {kModeFused, kPrepared, true, true, k_step<kModeFused, 0, true, true, true, true>},
+    {kModePass1, kRagged, false, false, k_step<kModePass1, 2, false>},
+    {kModePass1, kRuntimeDiv, false, false, k_step<kModePass1, 2, true>},
+    {kModePass1, kPrepared, false, false, k_step<kModePass1, 0, true, false, false, true>},
+    {kModePass1, kPrepared, false, true, k_step<kModePass1, 0, true, false, true, true>},
+    {kModePass1, kPrepared, true, false, k_step<kModePass1, 0, true, true, false, true>},
+    {kModePass1, kPrepared, true, true, k_step<kModePass1, 0, true, true, true, true>},
+    {kModePass2, kRagged, false, false, k_step<kModePass2, 2, false>},
+    {kModePass2, kRuntimeDiv, false, false, k_step<kModePass2, 2, true>},
+};
+
+size_t step_smem(const StepVariant& v) { return v.packed ? kSmemBytesPacked : kSmemBytes; }
+
+const StepVariant* find_step_variant(int mode, StepKind kind, bool fast, bool packed) {
+  for (const StepVariant& v : kStepVariants)
+    if (v.mode == mode && v.kind == kind && v.fast == fast && v.packed == packed) return &v;
+  return nullptr;
+}
+
+struct StepLaunch {
+  const StepVariant* full;
+  const StepVariant* ragged;
+};
+
+// Chooses the k_step instantiations of a step in `mode` and sets what the kernel has to know about that choice in `a`.
+StepLaunch select_step(AsHandle* h, int mode, const AsStateIn* in, StepArgs& a) {
+  // pass 2 of the 3-call path outside a speculating pass 1 (a reset outside a step) is off the hot path: the generic
+  // instantiation, in stream order, with the body rows read where they are
+  const bool hot = mode != kModePass2;
+  if (hot && a.use_pre && !(a.dense16 & kDenseBody)) {
+    // The three body rows the task reads (12 bytes each out of Isaac Lab's (N,B,13) body_state_w) are scattered
+    // reads like the contact vectors: k_prepare* gathers them into a dense (N,3,3) array, which the step kernel (and
+    // the fix-up, which re-reads the inputs) then takes by bulk copy.
+    a.body_from_prepare = 1;
+    a.in.body_pos = h->ws.body_dense;
+    a.in.body_env_stride = 9;
+    a.in.body_row_stride = 3;
+    a.in.right_foot_row = 0;
+    a.in.left_foot_row = 1;
+    a.in.torso_row = 2;
+    a.dense16 |= kDenseBody;
+  }
+  // dependent of the gather kernel: tiles, state words and windows are loaded while the gather's last wave runs; the
+  // MDP role waits for the gather (griddepcontrol.wait) right before it reads the contact norms.  Not between the timing
+  // events of a fused step, which time the step kernel alone.
+  a.pdl_wait = (hot && h->pdl >= 2 && a.use_pre && !(mode == kModeFused && h->ev_start)) ? 1 : 0;
+  // the common launch shape has its own instantiation (process_tile: FAST)
+  const bool fast = !a.in.quat_xyzw && !a.out.reward_terms && a.out.obs_clip == 0.0f;
+  // root pos / quat / lin vel handed over as slices of one (N,13) root_state_w tensor (Isaac Lab's own layout): the
+  // full tiles take the whole rows with one bulk copy (process_tile: PACKED)
+  const bool packed = in->root_pos_stride == AS_ROOT_STATE_DIM && in->root_quat_stride == AS_ROOT_STATE_DIM &&
+                      in->root_lin_vel_stride == AS_ROOT_STATE_DIM && in->root_quat == in->root_pos + 3 &&
+                      in->root_lin_vel == in->root_pos + 7 && (reinterpret_cast<uintptr_t>(in->root_pos) & 15u) == 0;
+  // (the host knows whether any divisor needs a true division: the two-FMA instantiations have no branch for it)
+  StepKind kind = kRuntimeDiv;
+  if (hot && !h->jc.exact_div && a.use_pre && !contact_in_host_memory(h, in)) kind = kPrepared;
+  else if (mode == kModeFused && !h->jc.exact_div) kind = kTwoFma;
+  const bool variants = kind != kRuntimeDiv;
+  return {find_step_variant(mode, kind, variants && fast, variants && packed),
+          find_step_variant(mode, kRagged, false, false)};
+}
+
 // Launches k_step over all tiles: a one-CTA launch of the ragged instantiation for a tail tile (first, so that in a
 // programmatic chain the full-tile kernel, whose CTAs wait for their primary before they read the contact norms,
-// cannot complete before it), then the full-tile instantiation.  `full` / `ragged` are the two instantiations.
-template <typename K>
-cudaError_t launch_step(AsHandle* h, K full, K ragged, StepArgs& a, cudaStream_t s, bool programmatic,
-                        size_t full_smem = kSmemBytes) {
+// cannot complete before it), then the full-tile instantiation.
+cudaError_t launch_step(AsHandle* h, const StepLaunch& k, StepArgs& a, cudaStream_t s) {
+  if (!k.full || !k.ragged) return cudaErrorInvalidDeviceFunction;  // (a combination missing from kStepVariants)
+  const bool programmatic = a.pdl_wait != 0;
   const int n_full = static_cast<int>(a.num_envs / kTile);
   if (n_full < a.num_tiles) {
     a.tile_base = n_full;
-    cudaError_t rc = launch_dependent(ragged, 1u, static_cast<unsigned>(kThreads), kSmemBytes, s, programmatic, a);
+    cudaError_t rc = launch_dependent(k.ragged->kernel, 1u, static_cast<unsigned>(kThreads), step_smem(*k.ragged), s,
+                                      programmatic, a);
     if (rc != cudaSuccess) return rc;
     if (n_full > 0) h->launches += 1;  // (check_launch counts one launch per call)
   }
   a.tile_base = 0;
   if (n_full == 0) return cudaSuccess;
-  return launch_dependent(full, static_cast<unsigned>(n_full), static_cast<unsigned>(kThreads), full_smem, s,
-                          programmatic, a);
+  return launch_dependent(k.full->kernel, static_cast<unsigned>(n_full), static_cast<unsigned>(kThreads),
+                          step_smem(*k.full), s, programmatic, a);
 }
 }  // namespace
 
@@ -343,27 +431,8 @@ int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, i
                                  std::to_string(prop.minor));
   }
   // the step kernels stage more than the default 48 KB of dynamic shared memory
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 1, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 1, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 1, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModeFused, 0, true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass1, 0, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass1, 0, true, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass1, 0, true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass1, 0, true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesPacked));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass1, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass1, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass2, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  AS_CUDA(cudaFuncSetAttribute(k_step<kModePass2, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+  for (const StepVariant& v : kStepVariants)
+    AS_CUDA(cudaFuncSetAttribute(v.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(step_smem(v))));
   AS_CUDA(cudaFuncSetAttribute(k_fixup_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   AS_CUDA(cudaFuncSetAttribute(k_mirror_batch, cudaFuncAttributeMaxDynamicSharedMemorySize, kMirrorSmemBytes));
   AsHandle* h = new (std::nothrow) AsHandle();
@@ -387,18 +456,8 @@ int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, i
   h->pending_valid = false;
   h->ev_start = h->ev_stop = nullptr;
   {
-    // tuning knob, off by default: measured on B200 at 1M envs, a quarter wave ahead (148 tiles) gains 1 %, one wave
-    // or more loses (the lines are evicted before use) -- DESIGN.md section 6
-    const char* pf = std::getenv("ALLSTEPS_PREFETCH_TILES");
-    h->prefetch_tiles = pf ? std::atoi(pf) : 0;
     const char* pdl = std::getenv("ALLSTEPS_PDL");
     h->pdl = pdl ? std::atoi(pdl) : 2;
-    const char* pm = std::getenv("ALLSTEPS_PREPARE_MIN_ENVS");
-    h->prepare_min_envs = pm ? std::atoll(pm) : kSeparateGatherMinEnvsDefault;
-    const char* sf = std::getenv("ALLSTEPS_SELF_FINISH");
-    h->allow_self_finish = sf ? std::atoi(sf) : 1;
-    const char* pre = std::getenv("ALLSTEPS_PRE");
-    h->allow_pre = pre ? std::atoi(pre) : 1;
     const char* rm = std::getenv("ALLSTEPS_REGEN_MODE");
     h->regen_mode = rm ? std::atoi(rm) : 0;
   }
@@ -426,30 +485,22 @@ int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, i
     return cuda_fail(e, "cudaMemsetAsync(workspace)");
   }
   // no stone window is valid yet (k_prepare* refreshes the records whose bit is set)
-  if (e == cudaSuccess)
-    e = cudaMemsetAsync(h->ws.win_stale, 0xFF, static_cast<size_t>((num_envs + 31) / 32 * 4), s);
+  e = cudaMemsetAsync(h->ws.win_stale, 0xFF, static_cast<size_t>((num_envs + 31) / 32 * 4), s);
   if (e != cudaSuccess) {
     delete h;
     return cuda_fail(e, "cudaMemsetAsync(win_stale)");
   }
-  // initial MDP state of AllstepsEnv.__init__ (ENV:74-78): index 1, right leg swings, everything else zero
-  AsMdpState none;
-  std::memset(&none, 0, sizeof(none));
-  *out = h;
-  // state words: idx = 1
-  {
-    // a zeroed word has idx 0; write idx 1 through the import kernel with a constant source is overkill --
-    // fill both buffers with the packed constant instead (low 32 bits of each 8-byte word).
-    const uint32_t word = pack_state(1, 0, 0, 0, 0);
-    e = cudaMemset2DAsync(h->ws.state[0], 8, static_cast<int>(word & 0xFFu), 1, static_cast<size_t>(num_envs), s);
-    if (e == cudaSuccess)
-      e = cudaMemset2DAsync(h->ws.state[1], 8, static_cast<int>(word & 0xFFu), 1, static_cast<size_t>(num_envs), s);
-    if (e != cudaSuccess) {
-      delete h;
-      *out = nullptr;
-      return cuda_fail(e, "cudaMemset2DAsync(state)");
-    }
+  // initial MDP state of AllstepsEnv.__init__ (ENV:74-78): index 1, right leg swings, everything else zero -- in both
+  // state buffers the packed word, which is nonzero in its lowest byte only
+  const uint32_t word = pack_state(1, 0, 0, 0, 0);
+  e = cudaMemset2DAsync(h->ws.state[0], 8, static_cast<int>(word & 0xFFu), 1, static_cast<size_t>(num_envs), s);
+  if (e == cudaSuccess)
+    e = cudaMemset2DAsync(h->ws.state[1], 8, static_cast<int>(word & 0xFFu), 1, static_cast<size_t>(num_envs), s);
+  if (e != cudaSuccess) {
+    delete h;
+    return cuda_fail(e, "cudaMemset2DAsync(state)");
   }
+  *out = h;
   return AS_OK;
 }
 
@@ -499,54 +550,14 @@ int as_step_fused(AsHandle* h, const AsStateIn* in, const float* actions, int64_
   const bool regen_enabled = grid || (h->params.flags & AS_FLAG_INTENDED_REGEN) != 0;
   a.want_reset_list = (reset_out && reset_out->reset_ids) ? 1 : 0;
   if (want_rows) a.rows = *reset_out;  // start-pose rows are written by the step kernel itself
-  bool gather_body = false;
-  if (!(a.dense16 & kDenseBody) && h->num_envs >= h->prepare_min_envs) {
-    // The three body rows the task reads (12 bytes each out of Isaac Lab's (N,B,13) body_state_w) are scattered
-    // reads like the contact vectors: k_prepare* gathers them into a dense (N,3,3) array, which the step kernel (and
-    // the fix-up, which re-reads the inputs) then takes by bulk copy.
-    gather_body = true;
-    a.body_from_prepare = 1;
-    a.in.body_pos = h->ws.body_dense;
-    a.in.body_env_stride = 9;
-    a.in.body_row_stride = 3;
-    a.in.right_foot_row = 0;
-    a.in.left_foot_row = 1;
-    a.in.torso_row = 2;
-    a.dense16 |= kDenseBody;
-  }
-  if (int rc = launch_prepare(h, in, s, gather_body)) return rc;
+  const StepLaunch k = select_step(h, kModeFused, in, a);
+  if (int rc = launch_prepare(h, in, s, a.body_from_prepare != 0)) return rc;
   if (h->ev_start) AS_CUDA(cudaEventRecord(h->ev_start, s));
-  // dependent of the gather kernel: tiles, state words and windows are loaded while the gather's last wave runs;
-  // the MDP role waits for the gather (griddepcontrol.wait) right before it reads the contact norms
-  const bool dep = h->pdl >= 2 && a.use_pre && !h->ev_start;
-  a.pdl_wait = dep ? 1 : 0;
-  // (the host knows whether any divisor needs a true division: the hot kernel has no branch for it)
-  // the common launch shape has its own instantiation (process_tile: FAST)
-  const bool fast = !a.in.quat_xyzw && !a.out.reward_terms && a.out.obs_clip == 0.0f && a.prefetch_tiles == 0;
-  // root pos / quat / lin vel handed over as slices of one (N,13) root_state_w tensor (Isaac Lab's own layout): the
-  // full tiles take the whole rows with one bulk copy (process_tile: PACKED)
-  const bool packed = in->root_pos_stride == AS_ROOT_STATE_DIM && in->root_quat_stride == AS_ROOT_STATE_DIM &&
-                      in->root_lin_vel_stride == AS_ROOT_STATE_DIM && in->root_quat == in->root_pos + 3 &&
-                      in->root_lin_vel == in->root_pos + 7 && (reinterpret_cast<uintptr_t>(in->root_pos) & 15u) == 0;
-  using StepKernel = void (*)(StepArgs);
-  const int ex = h->jc.exact_div ? 1 : 0;
-  static const StepKernel kFull[2][2][2] = {  // [exact][fast][packed]
-      {{k_step<kModeFused, 0, true, false, false>, k_step<kModeFused, 0, true, false, true>},
-       {k_step<kModeFused, 0, true, true, false>, k_step<kModeFused, 0, true, true, true>}},
-      {{k_step<kModeFused, 1, true, false, false>, k_step<kModeFused, 1, true, false, true>},
-       {k_step<kModeFused, 1, true, true, false>, k_step<kModeFused, 1, true, true, true>}}};
-  // behind k_prepare* (large batches, two-FMA quotients): the instantiation without any scattered access of its own
-  static const StepKernel kFullPre[2][2] = {  // [fast][packed]
-      {k_step<kModeFused, 0, true, false, false, true>, k_step<kModeFused, 0, true, false, true, true>},
-      {k_step<kModeFused, 0, true, true, false, true>, k_step<kModeFused, 0, true, true, true, true>}};
-  const StepKernel ragged_kernel = k_step<kModeFused, 2, false>;
-  const bool pre = a.use_pre && ex == 0 && h->allow_pre && !contact_in_host_memory(h, in);
   // the last CTA closes the step itself unless somebody else has to see the open step: the cross-shard exchange, an
   // all-reduce the caller announced (AS_STEP_DEFER_FINISH), or the regeneration kernels launched below
-  a.self_finish = (h->allow_self_finish && !regen_enabled && !(out->flags & AS_STEP_DEFER_FINISH)) ? 1 : 0;
+  a.self_finish = (!regen_enabled && !(out->flags & AS_STEP_DEFER_FINISH)) ? 1 : 0;
   if (h->peer_connected) a.peer = h->peer;  // (world > 0: the closing CTA sums the counters over the shards itself)
-  AS_CUDA(launch_step(h, pre ? kFullPre[fast ? 1 : 0][packed ? 1 : 0] : kFull[ex][fast ? 1 : 0][packed ? 1 : 0],
-                      ragged_kernel, a, s, dep, packed ? kSmemBytesPacked : kSmemBytes));
+  AS_CUDA(launch_step(h, k, a, s));
   if (int rc = check_launch(h, "k_step<fused>")) return rc;
   if (h->ev_stop) AS_CUDA(cudaEventRecord(h->ev_stop, s));
   if (regen_enabled) {
@@ -705,33 +716,9 @@ int as_step_pass1(AsHandle* h, const AsStateIn* in, const float* actions, int64_
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   AS_CUDA(cudaMemsetAsync(&h->ws.ctrl->n_reset_list, 0, sizeof(uint32_t), s));  // pass 1 compacts the flagged envs
   h->device_list = false;
-  bool gather_body = false;
-  if (!(a.dense16 & kDenseBody) && h->num_envs >= h->prepare_min_envs) {  // (as in as_step_fused)
-    gather_body = true;
-    a.body_from_prepare = 1;
-    a.in.body_pos = h->ws.body_dense;
-    a.in.body_env_stride = 9;
-    a.in.body_row_stride = 3;
-    a.in.right_foot_row = 0;
-    a.in.left_foot_row = 1;
-    a.in.torso_row = 2;
-    a.dense16 |= kDenseBody;
-  }
-  if (int rc = launch_prepare(h, in, s, gather_body)) return rc;
-  const bool dep = h->pdl >= 2 && a.use_pre;
-  a.pdl_wait = dep ? 1 : 0;
-  const bool fast = !a.in.quat_xyzw && !a.out.reward_terms && a.out.obs_clip == 0.0f && a.prefetch_tiles == 0;
-  const bool packed = in->root_pos_stride == AS_ROOT_STATE_DIM && in->root_quat_stride == AS_ROOT_STATE_DIM &&
-                      in->root_lin_vel_stride == AS_ROOT_STATE_DIM && in->root_quat == in->root_pos + 3 &&
-                      in->root_lin_vel == in->root_pos + 7 && (reinterpret_cast<uintptr_t>(in->root_pos) & 15u) == 0;
-  using StepKernel = void (*)(StepArgs);
-  static const StepKernel kFullPre[2][2] = {  // [fast][packed]
-      {k_step<kModePass1, 0, true, false, false, true>, k_step<kModePass1, 0, true, false, true, true>},
-      {k_step<kModePass1, 0, true, true, false, true>, k_step<kModePass1, 0, true, true, true, true>}};
-  const bool pre = a.use_pre && !h->jc.exact_div && h->allow_pre && !contact_in_host_memory(h, in);
-  const StepKernel full = pre ? kFullPre[fast ? 1 : 0][packed ? 1 : 0] : k_step<kModePass1, 2, true>;
-  AS_CUDA(launch_step(h, full, k_step<kModePass1, 2, false>, a, s, dep,
-                      (pre && packed) ? kSmemBytesPacked : kSmemBytes));
+  const StepLaunch k = select_step(h, kModePass1, in, a);
+  if (int rc = launch_prepare(h, in, s, a.body_from_prepare != 0)) return rc;
+  AS_CUDA(launch_step(h, k, a, s));
   h->pass1_done = true;   // (its last CTA folds the statistics and advances the Philox step counter)
   h->spec_valid = true;
   h->spec_obs = out->obs;
@@ -809,8 +796,9 @@ int as_step_pass2(AsHandle* h, const AsStateIn* in, float* obs, void* stream) {
   out.obs = obs;
   out.obs_clip = h->obs_clip_pass1;
   StepArgs a = make_step_args(h, in, nullptr, 0, &out);
-  if (int rc = launch_prepare(h, in, s)) return rc;
-  AS_CUDA(launch_step(h, k_step<kModePass2, 2, true>, k_step<kModePass2, 2, false>, a, s, false));
+  const StepLaunch k = select_step(h, kModePass2, in, a);
+  if (int rc = launch_prepare(h, in, s, a.body_from_prepare != 0)) return rc;
+  AS_CUDA(launch_step(h, k, a, s));
   return check_launch(h, "k_step<pass2>");
 }
 

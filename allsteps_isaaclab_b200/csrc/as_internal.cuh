@@ -201,7 +201,6 @@ struct StepArgs {
   int32_t self_finish;                // fused: the last CTA closes the step when at least one env reset (no peers, no regeneration)
   int32_t pdl_wait;                   // 1: launched as a programmatic dependent of k_prepare*
   int32_t body_from_prepare;          // 1: in.body_pos is the dense array k_prepare* of this step writes
-  int32_t prefetch_tiles;             // the step kernel pulls the inputs of tile + prefetch_tiles into L2 (0 = off)
   uint32_t dense16;                   // per-array "dense and 16-byte aligned" bits (DenseBit), evaluated by the host
   float inv_step_dt;                  // RN(1 / P.step_dt) for the two-FMA quotient of ENV:416 (see JointConsts::exact_div)
   AsResetOut rows;                    // fused: start-pose rows for PhysX, written at the env's own row (optional)

@@ -148,10 +148,6 @@ __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
 __device__ __forceinline__ void cp_async_wait_all() {
   asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
 }
-// TMA prefetch of a contiguous global range into L2 (no shared memory involved).
-__device__ __forceinline__ void bulk_prefetch_l2(const void* src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 
 // ------------------------------------------------------------------------------------------------ staging
@@ -194,18 +190,8 @@ __device__ __forceinline__ float4 ldg64_f4(const float4* p) {
 // that the gather's fills do not push out what the step kernel is about to read (state words, contact records, stone
 // windows written / touched by the same kernel).  Measured at 1 M envs (profiles/r02_experiments.txt): no hints 188.5 us
 // per step; this + "evict last" on the contact record 185.3; + "evict last" on the step kernel's state-word store (the
-// next k_prepare* reads it first thing; AS_HINT_STATE) 184.0-184.4; "evict last" on the window refresh (AS_HINT_WINDOW)
-// helps at 262 144 envs (62.5 against 64.3) and costs at 1 M (187.7), off.  -D...=0 / 1 build the variants.
-#ifndef AS_GATHER_EVICT_FIRST
-#define AS_GATHER_EVICT_FIRST 1
-#endif
-#ifndef AS_HINT_WINDOW
-#define AS_HINT_WINDOW 0
-#endif
-#ifndef AS_HINT_STATE
-#define AS_HINT_STATE 1
-#endif
-
+// next k_prepare* reads it first thing) 184.0-184.4.  "Evict last" on the window refresh helps at 262 144 envs (62.5
+// against 64.3) and costs at 1 M (187.7): the refresh stores without a hint.
 __device__ __forceinline__ uint64_t policy_evict_first() {
   uint64_t pol;
   asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
@@ -217,35 +203,16 @@ __device__ __forceinline__ uint64_t policy_evict_last() {
   return pol;
 }
 __device__ __forceinline__ float4 ldg64_once_f4(const float4* p, uint64_t pol) {
-#if AS_GATHER_EVICT_FIRST
   float4 r;
   asm("ld.global.nc.L2::cache_hint.L2::64B.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
       : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p), "l"(pol));
   return r;
-#else
-  return ldg64_f4(p);
-#endif
-}
-__device__ __forceinline__ void st_keep_f4(float4* p, const float4& v, uint64_t pol) {
-#if AS_GATHER_EVICT_FIRST
-  asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1,%2,%3,%4}, %5;" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "l"(pol) : "memory");
-#else
-  *p = v;
-#endif
 }
 __device__ __forceinline__ void st_keep_u8(uint8_t* p, unsigned v, uint64_t pol) {
-#if AS_GATHER_EVICT_FIRST
   asm volatile("st.global.L2::cache_hint.u8 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
-#else
-  *p = static_cast<uint8_t>(v);
-#endif
 }
 __device__ __forceinline__ void st_keep_u2(uint2* p, const uint2& v, uint64_t pol) {
-#if AS_GATHER_EVICT_FIRST
   asm volatile("st.global.L2::cache_hint.v2.u32 [%0], {%1,%2}, %3;" ::"l"(p), "r"(v.x), "r"(v.y), "l"(pol) : "memory");
-#else
-  *p = v;
-#endif
 }
 __device__ __forceinline__ float ldg64_f(const float* p) {
   float r;
@@ -369,10 +336,10 @@ __device__ __forceinline__ void first_three_stones(const AsParams& P, const Vec3
 // (2*(x - offset)) / range is produced by the two-FMA correction q = fma(fma(-q0, range, n), inv, q0), which is the
 // correctly rounded quotient when inv = RN(1/range) (Markstein); as_create falls back to a true division for a
 // joint whose range has an all-ones significand (the theorem's excluded case).
-// `exact` (true division) is a compile-time choice in the fused kernel: the host knows whether any divisor is an
-// excluded case and launches the matching instantiation, so the hot code has no branch for it -- every branch ends a
+// `exact` (true division) is never decided per joint: the host knows whether any divisor is an excluded case and
+// launches the hot instantiations (EXACT = 0) only when none is, so they have no branch for it -- every branch ends a
 // basic block and, when taken, costs an instruction refetch; with one inside each of the 21 unrolled joint
-// iterations the joint loop ran 2.5x slower.
+// iterations the joint loop ran 2.5x slower.  The others (EXACT = 2) choose once, ahead of the joint loop.
 // The factor 2 of MATH:39 is folded into the constants (c = offset, range / 2, 2 / range): scaling by a power of two is
 // exact, so (2 d) / range and d / (range / 2) are the same real quotient and every rounding of the two-FMA sequence
 // lands on the same value (outside the denormal range) -- one multiplication per joint less.
@@ -380,11 +347,11 @@ __device__ __forceinline__ float scale_joint(const float4& c, float x, bool exac
   const float d = x - c.x;
   return exact ? d / c.y : div_by_const(d, c.y, c.z);
 }
-// EXACT template argument of process_tile / k_step: 0 two-FMA quotients, 1 true divisions, 2 decided at run time
-// (the modes off the hot path, to keep the number of instantiations down).
+// EXACT template argument of process_tile / k_step: 0 two-FMA quotients, 2 decided at run time from
+// JointConsts::exact_div (the launches off the hot path, to keep the number of instantiations down).
 template <int EXACT>
 __device__ __forceinline__ bool use_exact_div(const JointConsts& C) {
-  return EXACT == 2 ? C.exact_div != 0 : EXACT == 1;
+  return EXACT == 2 && C.exact_div != 0;
 }
 
 // Start-pose joint value of a reset env (ENV:505-560): running-start pose (already mirrored or not), uniform
@@ -697,14 +664,14 @@ __device__ __forceinline__ void close_pass1_by_last_cta(const StepArgs& a, Ctrl*
 // FULL: the tile has all kTile envs (every tile but a ragged last one).  A template parameter because the
 // `active` guards it removes are not free: each one ends a basic block, and the step is bound by how well the
 // instruction streams of its two roles schedule, not by DRAM (DESIGN.md section 6).
-// FAST: the launch uses none of the options -- w,x,y,z quaternions, no per-term reward output, no observation clamp,
-// no L2 prefetch.  The host checks that (as_step_fused) and the instantiation drops their uniform branches.
+// FAST: the launch uses none of the options -- w,x,y,z quaternions, no per-term reward output, no observation clamp.
+// The host checks that (select_step in as_api.cu) and the instantiation drops their uniform branches.
 // (Measured: 179.3 -> 176.7 us per 1M-env step.  Also making the per-array "dense" bits compile-time constants
 // removes 45 more instructions per warp but ptxas then spills 56 instead of 20 bytes in the MDP role: 184 us.)
-// PRE: the launch follows k_prepare* (large batches): the contact norms of the current stone AND of the stone after it
-// come as one coalesced 16-byte record, the stone window is known to be valid and is never written here (k_prepare* of
-// the next step refreshes the records whose tag went stale) -- no scattered access is left in the hot kernel but the
-// stones 0..2 of an env that resets.
+// PRE: the launch follows k_prepare* (large batches, two-FMA quotients, contact matrices in device memory): the
+// "foot presses" bits of the current stone AND of the stone after it come as one coalesced one-byte record, the stone
+// window is known to be valid and is never written here (k_prepare* of the next step refreshes the records whose tag
+// went stale) -- no scattered access is left in the hot kernel but the stones 0..2 of an env that resets.
 template <int MODE, bool FULL, int EXACT, bool FAST = false, bool PACKED = false, bool PRE = false>
 __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32_t& phase_root,
                                              uint32_t& phase_joint, unsigned char* smem) {
@@ -789,29 +756,6 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
       // dependent launch): everything else is in flight, this one copy waits for the primary to complete
       if (a.pdl_wait) asm volatile("griddepcontrol.wait;" ::: "memory");
       bulk_g2s(smem_u32(s_body), a.in.body_pos + env0 * 9, nv * 36, bar_root);
-    }
-  }
-
-  // ---------------------------------------------------------------- L2 prefetch for a LATER tile
-  // A CTA's shared memory is held for its whole lifetime, a third of which was spent waiting for its first loads
-  // to come back from DRAM (profiles/r01_cta_phase_timeline.txt).  L2 is 126 MB and idle: one thread asks the copy
-  // engine to pull the inputs of the tile that will be processed about one wave of CTAs later into L2, so that
-  // the CTA owning that tile finds them at L2 latency.  (Tiles, state words, stone windows and contact norms are all
-  // contiguous per tile.)
-  if (!FAST && tid == 0 && a.prefetch_tiles > 0) {
-    const int64_t ptile = static_cast<int64_t>(tile) + a.prefetch_tiles;
-    const int64_t penv0 = ptile * kTile;
-    if (penv0 + kTile <= a.num_envs) {  // full tiles only
-      if (dense & kDenseRp) bulk_prefetch_l2(a.in.root_pos + penv0 * 3, kTile * 12);
-      if (dense & kDenseRv) bulk_prefetch_l2(a.in.root_lin_vel + penv0 * 3, kTile * 12);
-      if (dense & kDenseBody) bulk_prefetch_l2(a.in.body_pos + penv0 * 9, kTile * 36);
-      if (dense & kDenseRq) bulk_prefetch_l2(a.in.root_quat + penv0 * 4, kTile * 16);
-      if (dense & kDenseJp) bulk_prefetch_l2(a.in.joint_pos + penv0 * kJ, kTile * kJ * 4);
-      if (dense & kDenseJv) bulk_prefetch_l2(a.in.joint_vel + penv0 * kJ, kTile * kJ * 4);
-      if (kNeedActions && (dense & kDenseAct)) bulk_prefetch_l2(a.actions + penv0 * kJ, kTile * kJ * 4);
-      bulk_prefetch_l2(a.ws.state[ctrl->parity] + penv0, kTile * 8);
-      bulk_prefetch_l2(a.ws.window + penv0 * 4, kTile * 64);
-      if (a.use_pre) bulk_prefetch_l2(a.ws.contact_pre + penv0, kTile);
     }
   }
 
@@ -1075,12 +1019,8 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
       uint2 sw;
       sw.x = pack_state(m.idx, m.leg, m.count, level, ep);
       sw.y = __float_as_uint(m.pot);
-#if AS_HINT_STATE
       if (PRE) st_keep_u2(st_out + e, sw, policy_evict_last());  // (k_prepare* of the next step reads it first thing)
       else st_out[e] = sw;
-#else
-      st_out[e] = sw;
-#endif
       if (PRE) {
         // this instantiation never writes windows: tell k_prepare* of the next step which records to refresh
         const unsigned stale = __ballot_sync(0xffffffffu, win_dirty);
@@ -1477,11 +1417,7 @@ struct PrepareArgs {
 __device__ __forceinline__ void refresh_window_entry(const Workspace& ws, int64_t e, int idx, int slot) {
   float4 v = ldg64_f4(ws.stones + e * kS + window_slot_stone(idx, slot));
   if (slot == 0) v.w = __int_as_float(idx);  // tag
-#if AS_HINT_WINDOW
-  st_keep_f4(ws.window + e * 4 + slot, v, policy_evict_last());  // (read by the step kernel in a moment)
-#else
   ws.window[e * 4 + slot] = v;
-#endif
 }
 
 // One lane per env (rows that are not 16-byte aligned).

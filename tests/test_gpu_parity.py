@@ -545,7 +545,8 @@ def test_joint_scaling_is_bit_exact():
 def test_true_division_fallback_kernels():
     """A divisor with an all-ones significand is the excluded case of the two-FMA quotient (Markstein): as_create
     then selects the step-kernel instantiations that divide.  One joint is given such a range (upper - lower =
-    0x3fffffff); full tiles, a ragged tail, resets and the bit-exact joint scaling must all still match the oracle."""
+    0x3fffffff); full tiles, a ragged tail, resets and the bit-exact joint scaling must all still match the oracle.
+    Two sizes: one that gathers inside the step kernel, and one from which k_prepare* gathers for it."""
     from allsteps_isaaclab_b200.config import AllstepsCfg
     from allsteps_isaaclab_b200.mdp import AllstepsMDP, StepBuffers
     from oracle import allsteps_oracle as ao
@@ -556,39 +557,41 @@ def test_true_division_fallback_kernels():
             lim[9] = (0.0, 1.9999998807907104)  # fp32 0x3fffffff
             return lim
 
-    N, seed = 300, 53
-    cfg = Cfg()
-    sc = Scenario(N, seed=seed, cfg=cfg, fall_fraction=0.1)
-    rng = (sc.joint_limits[9, 1] - sc.joint_limits[9, 0]).view(torch.int32).item()
-    assert rng & 0x7FFFFF == 0x7FFFFF, "the test's joint range is not the excluded case"
-    st0 = sc.initial_mdp_state()
-    orc = ao.AllstepsOracle(sc.cfg, N, sc.env_origins, sc.joint_limits, sc.body_indices, sc.stone_uniforms(0))
-    mdp = AllstepsMDP(N, device="cuda:0", cfg=cfg, seed=seed)
-    origins = sc.env_origins.cuda()
-    mdp.generate_stones(origins)
-    install_mdp_state(orc, st0)
-    mdp.import_state({k: st0[k] for k in ("curr_target_index", "swing_leg", "target_reach_count",
-                                          "episode_length_buf", "potentials")})
-    mdp.import_state({"steps_pos": orc.steps_pos, "steps_dphi": orc.steps_dphi})
-    out = StepBuffers(N, "cuda:0")
-    resets = 0
-    for step in range(4):
-        phys = sc.physics(orc.steps_pos, orc.curr_target_index, orc.swing_leg)
-        mirror_u, noise_u = sc.reset_uniforms(step)
-        o_obs, o_rew, o_term, o_to, o_ids = orc.step(phys, phys["actions"], mirror_u, noise_u, sc.stone_uniforms(step))
-        views, keep = to_views(phys, origins, sc.body_indices)
-        mdp.step(views, keep["actions"], out)
-        torch.cuda.synchronize()
-        exact(out.terminated, o_term, f"step {step} terminated")
-        exact(out.time_out, o_to, f"step {step} time_out")
-        close(out.reward, o_rew, f"step {step} reward")
-        close_obs(out.obs, o_obs, f"step {step} obs")
-        compare_state(mdp, orc, f"step {step}")
-        keep_rows = ~(o_term | o_to)
-        expect = ao.scale_to_unit(phys["joint_pos"], sc.joint_limits[:, 0], sc.joint_limits[:, 1])
-        assert torch.equal(out.obs[:, 6:27].cpu()[keep_rows], expect[keep_rows]), "joint_pos_scaled is not bit-identical"
-        resets += len(o_ids)
-    assert resets > 0
+    seed, cfg = 53, Cfg()
+    for N in (300, (1 << 16) + 44):
+        sc = Scenario(N, seed=seed, cfg=cfg, fall_fraction=0.1)
+        rng = (sc.joint_limits[9, 1] - sc.joint_limits[9, 0]).view(torch.int32).item()
+        assert rng & 0x7FFFFF == 0x7FFFFF, "the test's joint range is not the excluded case"
+        st0 = sc.initial_mdp_state()
+        orc = ao.AllstepsOracle(sc.cfg, N, sc.env_origins, sc.joint_limits, sc.body_indices, sc.stone_uniforms(0))
+        mdp = AllstepsMDP(N, device="cuda:0", cfg=cfg, seed=seed)
+        origins = sc.env_origins.cuda()
+        mdp.generate_stones(origins)
+        install_mdp_state(orc, st0)
+        mdp.import_state({k: st0[k] for k in ("curr_target_index", "swing_leg", "target_reach_count",
+                                              "episode_length_buf", "potentials")})
+        mdp.import_state({"steps_pos": orc.steps_pos, "steps_dphi": orc.steps_dphi})
+        out = StepBuffers(N, "cuda:0")
+        resets = 0
+        for step in range(4):
+            phys = sc.physics(orc.steps_pos, orc.curr_target_index, orc.swing_leg)
+            mirror_u, noise_u = sc.reset_uniforms(step)
+            o_obs, o_rew, o_term, o_to, o_ids = orc.step(phys, phys["actions"], mirror_u, noise_u,
+                                                         sc.stone_uniforms(step))
+            views, keep = to_views(phys, origins, sc.body_indices)
+            mdp.step(views, keep["actions"], out)
+            torch.cuda.synchronize()
+            at = f"N {N} step {step}"
+            exact(out.terminated, o_term, f"{at} terminated")
+            exact(out.time_out, o_to, f"{at} time_out")
+            close(out.reward, o_rew, f"{at} reward")
+            close_obs(out.obs, o_obs, f"{at} obs")
+            compare_state(mdp, orc, at)
+            keep_rows = ~(o_term | o_to)
+            expect = ao.scale_to_unit(phys["joint_pos"], sc.joint_limits[:, 0], sc.joint_limits[:, 1])
+            assert torch.equal(out.obs[:, 6:27].cpu()[keep_rows], expect[keep_rows]), f"{at}: joint_pos_scaled is not bit-identical"
+            resets += len(o_ids)
+        assert resets > 0
 
 
 def test_straight_line_math_is_exact(tmp_path):
