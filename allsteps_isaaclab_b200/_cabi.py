@@ -17,7 +17,7 @@ ROOT_STATE_DIM = 13
 NUM_REWARD_TERMS = 10
 PEER_HANDLE_BYTES = 64  # AS_PEER_HANDLE_BYTES (sizeof(cudaIpcMemHandle_t))
 TILE_ENVS = 128
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 FLAG_INTENDED_REGEN = 1 << 0
 FLAG_SKIP_PASS2 = 1 << 1
@@ -67,7 +67,7 @@ class AsStateIn(C.Structure):
 
 class AsStepOut(C.Structure):
     _fields_ = [("obs", _ptr), ("reward", _ptr), ("terminated", _ptr), ("time_out", _ptr), ("reward_terms", _ptr),
-                ("dones", _ptr), ("obs_clip", _f), ("flags", C.c_uint32)]
+                ("dones", _ptr), ("obs_clip", _f), ("flags", C.c_uint32), ("final_obs", _ptr)]
 
 
 class AsResetOut(C.Structure):

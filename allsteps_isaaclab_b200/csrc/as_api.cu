@@ -125,6 +125,18 @@ int launch_prepare(AsHandle* h, const AsStateIn* in, cudaStream_t s, bool gather
   return check_launch(h, "k_prepare");
 }
 
+// AsStepOut.final_obs: optional, a full-size (N,59) buffer of its own (the kernels write its rows while the
+// observation tile goes to obs)
+int validate_final_obs(const AsHandle* h, const AsStepOut* out) {
+  if (!out->final_obs) return AS_OK;
+  const uintptr_t f = reinterpret_cast<uintptr_t>(out->final_obs);
+  const uintptr_t o = reinterpret_cast<uintptr_t>(out->obs);
+  const uintptr_t bytes = static_cast<uintptr_t>(h->num_envs) * kObs * sizeof(float);
+  AS_REQUIRE((f & 3u) == 0, "final_obs must be 4-byte aligned");
+  AS_REQUIRE(f + bytes <= o || o + bytes <= f, "final_obs must not overlap obs");
+  return AS_OK;
+}
+
 int validate_state_in(const AsStateIn* in, bool need_origins) {
   AS_REQUIRE(in != nullptr, "AsStateIn is null");
   AS_REQUIRE(in->root_pos && in->root_quat && in->root_lin_vel, "root state pointers must be set");
@@ -357,7 +369,7 @@ StepLaunch select_step(AsHandle* h, int mode, const AsStateIn* in, StepArgs& a) 
   // events of a fused step, which time the step kernel alone.
   a.pdl_wait = (hot && h->pdl >= 2 && a.use_pre && !(mode == kModeFused && h->ev_start)) ? 1 : 0;
   // the common launch shape has its own instantiation (process_tile: FAST)
-  const bool fast = !a.in.quat_xyzw && !a.out.reward_terms && a.out.obs_clip == 0.0f;
+  const bool fast = !a.in.quat_xyzw && !a.out.reward_terms && a.out.obs_clip == 0.0f && !a.out.final_obs;
   // root pos / quat / lin vel handed over as slices of one (N,13) root_state_w tensor (Isaac Lab's own layout): the
   // full tiles take the whole rows with one bulk copy (process_tile: PACKED)
   const bool packed = in->root_pos_stride == AS_ROOT_STATE_DIM && in->root_quat_stride == AS_ROOT_STATE_DIM &&
@@ -540,6 +552,7 @@ int as_step_fused(AsHandle* h, const AsStateIn* in, const float* actions, int64_
   AS_REQUIRE(actions_stride >= kJ, "actions stride too small");
   AS_REQUIRE(out->obs && out->reward && out->terminated && out->time_out, "step outputs must be set");
   AS_REQUIRE(out->obs_clip >= 0.0f, "obs_clip must be >= 0");
+  if (int rc = validate_final_obs(h, out)) return rc;
   if (h->pending_valid) return fail(AS_ERR_STATE, "previous fused step was not closed with as_finish_step");
   if (int rc = check_peer(h)) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -710,6 +723,7 @@ int as_step_pass1(AsHandle* h, const AsStateIn* in, const float* actions, int64_
   AS_REQUIRE(out->obs && out->reward && out->terminated && out->time_out, "step outputs must be set");
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
   AS_REQUIRE(out->obs_clip >= 0.0f, "obs_clip must be >= 0");
+  if (int rc = validate_final_obs(h, out)) return rc;
   StepArgs a = make_step_args(h, in, actions, actions_stride, out);
   a.ext_episode_length = episode_length;
   h->obs_clip_pass1 = out->obs_clip;  // as_step_pass2 rewrites the same observation buffer: same epilogue

@@ -714,8 +714,6 @@ struct CommitArgs {
                            // k_pass2_revert (DRL:360 would have skipped `_reset_idx`)
 };
 
-__device__ __forceinline__ float clip_obs(float v, float c) { return c > 0.0f ? (v < -c ? -c : (v > c ? c : v)) : v; }
-
 __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ CommitArgs a) {
   __shared__ float s_row[8][4][20];
   const AsParams& P = a.P;

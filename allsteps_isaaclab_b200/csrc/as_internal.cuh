@@ -189,6 +189,9 @@ struct StepArgs {
   const float* actions;
   int64_t actions_stride;
   AsStepOut out;
+  // AsStepOut.final_obs moved the fields behind `out` by 8 bytes; ptxas then allocated the FAST pass-1 instantiations
+  // differently (more spills).  Moving them by 16 keeps their 16-byte alignment as it was, and that code as it was.
+  uint64_t pad_final_obs;
   Workspace ws;
   const int64_t* ext_episode_length;  // 3-call path: DirectRLEnv-owned counter (already incremented), or null
   const AsExchange* global_stats;     // fix-up/finish: exchange record summed over ranks, or null

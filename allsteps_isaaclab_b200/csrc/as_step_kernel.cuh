@@ -249,6 +249,12 @@ __device__ __forceinline__ float contact_norm(const float* row, int idx, bool al
   return norm3(x, y, z);  // ENV:421-424
 }
 
+// The observation clamp of AsStepOut.obs_clip for one value (c == 0: raw).  Comparisons, not fminf/fmaxf: torch.clamp
+// hands NaN through.
+__device__ __forceinline__ float clip_obs(float v, float c) {
+  return c > 0.0f ? (v < -c ? -c : (v > c ? c : v)) : v;
+}
+
 // ------------------------------------------------------------------------------------------------ one pass
 struct Mdp {
   int idx, leg, count;
@@ -664,8 +670,9 @@ __device__ __forceinline__ void close_pass1_by_last_cta(const StepArgs& a, Ctrl*
 // FULL: the tile has all kTile envs (every tile but a ragged last one).  A template parameter because the
 // `active` guards it removes are not free: each one ends a basic block, and the step is bound by how well the
 // instruction streams of its two roles schedule, not by DRAM (DESIGN.md section 6).
-// FAST: the launch uses none of the options -- w,x,y,z quaternions, no per-term reward output, no observation clamp.
-// The host checks that (select_step in as_api.cu) and the instantiation drops their uniform branches.
+// FAST: the launch uses none of the options -- w,x,y,z quaternions, no per-term reward output, no observation clamp,
+// no final observations.  The host checks that (select_step in as_api.cu) and the instantiation drops their uniform
+// branches.
 // (Measured: 179.3 -> 176.7 us per 1M-env step.  Also making the per-array "dense" bits compile-time constants
 // removes 45 more instructions per warp but ptxas then spills 56 instead of 20 bytes in the MDP role: 184 us.)
 // PRE: the launch follows k_prepare* (large batches, two-FMA quotients, contact matrices in device memory): the
@@ -967,6 +974,17 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
     }
     if ((MODE == kModeFused || kSpec) && active) {
       if (MODE == kModeFused && is_reset) {
+        if (!FAST && a.out.final_obs) {
+          // final observation (AsStepOut.final_obs): head and tail of the row as pass 1 left them, before the reset
+          // below overwrites them; roll / pitch / v_b follow once the joint role has published them
+          float* fin = a.out.final_obs + e * kObs;
+          const float c = a.out.obs_clip;
+          fin[0] = clip_obs(h, c);
+          fin[48] = clip_obs(po.contact_r, c); fin[49] = clip_obs(po.contact_l, c);
+          fin[50] = clip_obs(po.tb0.x, c); fin[51] = clip_obs(po.tb0.y, c); fin[52] = clip_obs(po.tb0.z, c);
+          fin[53] = clip_obs(po.tb1.x, c); fin[54] = clip_obs(po.tb1.y, c); fin[55] = clip_obs(po.tb1.z, c);
+          fin[56] = clip_obs(po.tb2.x, c); fin[57] = clip_obs(po.tb2.y, c); fin[58] = clip_obs(po.tb2.z, c);
+        }
         mirror = misc->coin[t] != 0;  // drawn by the joint role in its idle time (ordered by the orientation barrier)
         // ---- masked reset, ENV:487-538.  Pass 2 on the post-reset state: identity orientation (vector part +-0),
         // zero velocity, zero contacts (contact_sensor.py:155), stale body positions; so roll = pitch = v_b = 0 and
@@ -1209,6 +1227,11 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
           const float u = u32_to_unit(phx_w[(k5 * 6 + (d >> 2)) * 4 + (d & 3)]);
           const float val = reset_joint_value(P, mirror_r ? pose_m_l : pose_l, jc_l, u, exact);
           float* row = s_obs + (row0 + r) * kObs;
+          if (!FAST && a.out.final_obs) {  // final observation: the pass-1 joint columns, before the start pose replaces them
+            float* fin = a.out.final_obs + e_r * kObs;
+            fin[6 + lane] = clip_obs(row[6 + lane], a.out.obs_clip);
+            fin[6 + kJ + lane] = clip_obs(row[6 + kJ + lane], a.out.obs_clip);
+          }
           row[6 + lane] = scale_joint(jc_l, val, exact);
           const float jv0 = mirror_r ? vel_m_l : 0.0f;
           row[6 + kJ + lane] = clamp_nan(jv0 * P.dof_vel_scale, -5.0f, 5.0f);
@@ -1270,6 +1293,15 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
         float* rt = a.out.reward_terms + e * AS_NUM_REWARD_TERMS;
         rt[2] = r_roll; rt[3] = r_pitch;
         rt[5] = r_energy; rt[6] = r_action; rt[7] = r_limit; rt[8] = r_step; rt[9] = r_bonus;
+      }
+      if (MODE == kModeFused && !FAST && a.out.final_obs && is_reset) {  // the rest of the final observation's head
+        float* fin = a.out.final_obs + e * kObs;
+        const float c = a.out.obs_clip;
+        fin[1] = clip_obs(roll_j, c);
+        fin[2] = clip_obs(pitch_j, c);
+        fin[3] = clip_obs(misc->x_vb[0][t], c);
+        fin[4] = clip_obs(misc->x_vb[1][t], c);
+        fin[5] = clip_obs(misc->x_vb[2][t], c);
       }
     }
     if (active) {  // head and tail of the observation row, ENV:330-343
@@ -1341,6 +1373,19 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
   } else {
     __syncthreads();
     for (int i = tid; i < n_valid * kObs; i += kThreads) obs_dst[i] = s_obs[i];
+  }
+  if (kSpec && !FAST && a.out.final_obs && !joint_role) {
+    // final observations: pass 1 skipped pass 2 for the envs it flagged, so their finished (clamped) rows of the tile
+    // are the rows to keep -- copied by the env's MDP-role warp, one coalesced row at a time
+    unsigned todo = __ballot_sync(0xffffffffu, is_reset);
+    while (todo) {
+      const int r = warp * 32 + __ffs(todo) - 1;
+      todo &= todo - 1u;
+      const float* src = s_obs + r * kObs;
+      float* fin = a.out.final_obs + (env0 + r) * kObs;
+      fin[lane] = src[lane];
+      if (lane < kObs - 32) fin[32 + lane] = src[32 + lane];
+    }
   }
   unsigned ticket = 0;
   if (kStats && warp == 0) {  // CTA totals -> one replicated global slot (fire and forget), by the first warp

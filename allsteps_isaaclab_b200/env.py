@@ -51,14 +51,19 @@ def resolve_robot_tables(robot, cfg: AllstepsCfg):
 class AllstepsHooksB200:
     """Hook methods of `AllstepsEnv(DirectRLEnv)` (ENV:34) backed by `AllstepsMDP`."""
 
-    def _init_allsteps_b200(self, task_cfg: Optional[AllstepsCfg] = None, seed: int = 0, **mdp_kwargs):
-        """Call at the end of `__init__` (replaces ENV:40-102)."""
+    def _init_allsteps_b200(self, task_cfg: Optional[AllstepsCfg] = None, seed: int = 0, final_obs: bool = False,
+                            **mdp_kwargs):
+        """Call at the end of `__init__` (replaces ENV:40-102).
+
+        final_obs: publish `extras["final_obs"]` (N,59) every step: for the envs that reset in the step (`reset_buf`),
+        the observation of the state their episode ended in -- `obs` holds their start pose -- so that a time-out can
+        be bootstrapped with `gamma * V(final_obs)`.  Rows of the other envs hold whatever an earlier step left there."""
         self.task_cfg = task_cfg or AllstepsCfg()
         dev = torch.device(self.device)
         body_rows, joint_limits = resolve_robot_tables(self.robot, self.task_cfg)
         self.mdp = AllstepsMDP(self.num_envs, device=dev, cfg=self.task_cfg, seed=seed, joint_limits=joint_limits,
                                **mdp_kwargs)
-        self.buf = StepBuffers(self.num_envs, dev, reward_terms=True)
+        self.buf = StepBuffers(self.num_envs, dev, reward_terms=True, final_obs=final_obs)
         self.foot_indices = [body_rows[0], body_rows[1]]  # ENV:87
         self.torso_index = body_rows[2]  # ENV:88
         jn = list(self.robot.data.joint_names)
@@ -132,6 +137,8 @@ class AllstepsHooksB200:
         if getattr(self, "_pass1_open", False):  # DRL:360 skipped `_reset_idx`: no pass 2 this step
             self.mdp.no_reset()
             self._pass1_open = False
+        if self.buf.final_obs is not None:
+            self.extras["final_obs"] = self.buf.final_obs
         return {"policy": self.buf.obs}
 
     # ------------------------------------------------------------------ the reference's public buffers, on demand

@@ -119,9 +119,12 @@ class StepBuffers:
     """Output tensors of a step; allocated once, overwritten every step (the caller clones what it keeps)."""
 
     def __init__(self, num_envs: int, device, reward_terms: bool = False, reset_rows: bool = True,
-                 obs_clip: float = 0.0):
+                 obs_clip: float = 0.0, final_obs: bool = False):
         """obs_clip > 0: `obs` comes out clamped to +-obs_clip, the `clip_obs` of RlGamesVecEnvWrapper._process_obs
-        (isaaclab_rl/rl_games.py:293) folded into the kernel's observation write; 0 keeps the raw ENV:326-345 values."""
+        (isaaclab_rl/rl_games.py:293) folded into the kernel's observation write; 0 keeps the raw ENV:326-345 values.
+        final_obs: also allocate `final_obs` (N,59), where every step writes the observation of the state an env's
+        episode ended in, at the rows of the envs that reset (`dones`) and clamped like `obs` -- what bootstrapping a
+        time-out needs, since `obs` holds the start pose of those envs.  Other rows keep what they held."""
         kw = dict(device=device)
         self.obs_clip = float(obs_clip)
         self.obs = torch.empty(num_envs, OBS_DIM, dtype=torch.float32, **kw)
@@ -139,9 +142,10 @@ class StepBuffers:
             self.reset_joint_vel = torch.zeros(num_envs, NUM_JOINTS, dtype=torch.float32, **kw)
             self.reset_ids = torch.zeros(num_envs, dtype=torch.int32, **kw)
             self.n_reset = torch.zeros(1, dtype=torch.int32, **kw)
+        self.final_obs = torch.zeros(num_envs, OBS_DIM, dtype=torch.float32, **kw) if final_obs else None
         self.step_out = _cabi.AsStepOut(_ptr(self.obs), _ptr(self.reward), _ptr(self.terminated),
                                         _ptr(self.time_out), _ptr(self.reward_terms), _ptr(self.dones),
-                                        self.obs_clip, 0)
+                                        self.obs_clip, 0, _ptr(self.final_obs))
         self.reset_out = _cabi.AsResetOut(_ptr(self.reset_root_state), _ptr(self.reset_joint_pos),
                                           _ptr(self.reset_joint_vel), _ptr(self.reset_ids), _ptr(self.n_reset))
 

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define AS_ABI_VERSION 3
+#define AS_ABI_VERSION 4
 
 #define AS_NUM_JOINTS 21  /* CFG:57  action_space            */
 #define AS_NUM_STONES 20  /* CFG:90  num_steps               */
@@ -132,6 +132,16 @@ typedef struct AsStepOut {
                             torch.clamp), so the wrapper can hand the buffer on as it is.  0: raw (ENV:326-345).
                             as_step_pass2 applies the value given to the as_step_pass1 before it.           */
   uint32_t flags;        /* AS_STEP_* bits                                                                 */
+  float* final_obs;      /* optional (N,59), 4-byte aligned, not overlapping obs; NULL to skip.  The final
+                            observation of every env that resets in this step (terminated | time_out): the row the
+                            reference's `_get_observations()` (ENV:326-345) returns when called between `_get_dones` /
+                            `_get_rewards` and `_reset_idx` -- h, roll, pitch, v_b, scaled joint positions and clipped
+                            joint velocities of the step's physics input, foot_contact and targets_b as pass 1 left
+                            them -- clamped by obs_clip like obs.  What `V(s_T)` of a truncated episode needs, since
+                            `obs` holds the start pose of an env that reset.  Written at the env's own row, only for the
+                            envs that reset; other rows, and the whole buffer in a step in which no env resets, are
+                            left untouched.  Honoured by as_step_fused and as_step_pass1 (the envs pass 1 flagged,
+                            whatever ids as_reset is given later); the generic kernel instantiation runs when set. */
 } AsStepOut;
 /* AsStepOut.flags */
 enum {
