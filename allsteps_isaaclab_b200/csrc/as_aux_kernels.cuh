@@ -254,7 +254,9 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
     }
   }
   if (a.out.n_reset && blockIdx.x == 0 && threadIdx.x == 0) *a.out.n_reset = static_cast<int32_t>(n_reset);
-  if (!a.fused && blockIdx.x == 0 && threadIdx.x == 0) ctrl->n_reset_list = static_cast<uint32_t>(n_reset);
+  // (the count of the list k_pass2_commit walks.  Outside a step no commit follows to clear it, and the next fused step
+  // would start its reset-id list behind it, past the end of the N-entry buffers)
+  if (a.into_other && blockIdx.x == 0 && threadIdx.x == 0) ctrl->n_reset_list = static_cast<uint32_t>(n_reset);
 }
 
 
@@ -723,6 +725,7 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
   const int64_t n = ctrl->n_reset_list;
   if (n == 0 && a.revert_if_none) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) ctrl->stats.n_advanced -= ctrl->last_adv2;  // pass 2 is discarded
     const int64_t total = a.num_envs * 11;
     for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
          i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
@@ -826,7 +829,10 @@ __global__ void __launch_bounds__(256) k_pass2_revert(Workspace ws, float* __res
     const int c = static_cast<int>(i - e * 11);
     obs[e * kObs + 48 + c] = clip_obs(reinterpret_cast<const float*>(ws.tail1 + e * 3)[c], obs_clip);
   }
-  if (blockIdx.x == 0 && threadIdx.x == 0) ws.ctrl->n_reset_list = 0;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    ws.ctrl->n_reset_list = 0;
+    ws.ctrl->stats.n_advanced -= ws.ctrl->last_adv2;  // the pass-2 advances pass 1 counted are discarded with pass 2
+  }
 }
 
 // `_reset_idx` called outside a step (as_reset without a preceding as_step_pass1): the numerator of ENV:471 from the

@@ -1025,7 +1025,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
           geom = foot_geometry(P, rf, lf, f_r, f_l, s_curr);
         }
         const bool moved = foot_update(P, geom, m, po);
-        if (MODE == kModeFused) adv2 = po.advanced;  // (3-call path: counted only if as_step_pass2 commits; left out)
+        adv2 = po.advanced;  // (taken back with pass 2 by k_fixup_finish, k_pass2_revert or k_pass2_commit)
         if (moved) {
           slide_window();
           targets_and_potential(P, a.inv_step_dt, exact, p, inv, s_prev, s_curr, s_next, m, po);

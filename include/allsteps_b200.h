@@ -165,7 +165,9 @@ typedef struct AsResetOut {
 typedef struct AsStats {
   int64_t n_envs;        /* envs that contributed                                                          */
   int64_t n_reset, n_terminated, n_time_out, n_fell, n_so_fast, n_died;
-  int64_t n_advanced;    /* stones reached (index advances) in this step, both passes                      */
+  int64_t n_advanced;    /* stones reached (index advances) in this step, both passes.  3-call path: pass 1
+                            counts the pass-2 advances it speculates; as_step_no_reset, or as_step_pass2
+                            finding the device-side list empty, takes them back with pass 2              */
   int64_t sum_target_index; /* sum of curr_target_index after pass 1: numerator of ENV:471                 */
   int64_t n_regenerated;
   int64_t level;         /* current curriculum level (max over envs when per-env levels are in use)        */
