@@ -99,6 +99,9 @@ class AsExchange(C.Structure):
 
 STATS_INT64_WORDS = C.sizeof(AsStats) // 8          # int64 words of the AsStats head of an exchange record
 EXCHANGE_INT64_WORDS = C.sizeof(AsExchange) // 8    # ... of the whole record (grid arrays: two uint32 per word)
+# The handle's difficulty-grid histograms (uint32 attempts[256], then successes[256]) sit this many bytes behind the
+# end of its exchange record in the workspace (a static_assert in csrc/as_internal.cuh holds the layout to it)
+GRID_HIST_OFFSET = 1664
 
 
 class AsMdpState(C.Structure):

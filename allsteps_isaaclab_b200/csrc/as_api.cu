@@ -294,6 +294,17 @@ cudaError_t launch_dependent(void (*kernel)(KArgs...), unsigned grid, unsigned b
   return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
+// k_reset_rows over the list of envs that regenerate (Ctrl::n_regen_list), behind the kernel that compacted it: the
+// fused step kernel or k_reset_list.  Shape: a warp per env for small batches, a thread per env for large ones
+// (ALLSTEPS_REGEN_MODE: 1 / 2).
+int launch_regeneration(AsHandle* h, const ResetArgs& r, cudaStream_t s) {
+  const bool by_warp = h->regen_mode == 1 || (h->regen_mode == 0 && h->num_envs <= kRegenByWarpMaxEnvs);
+  const int grid_ctas = grid_for(h->num_envs, 64, h->sm_count, 8);
+  AS_CUDA(launch_dependent(by_warp ? k_reset_rows<true> : k_reset_rows<false>, static_cast<unsigned>(grid_ctas), 256u,
+                           0, s, h->pdl >= 1, r));
+  return check_launch(h, "k_reset_rows");
+}
+
 using StepKernel = void (*)(StepArgs);
 
 // The families of k_step instantiations (process_tile describes FAST, PACKED and PRE).
@@ -579,12 +590,7 @@ int as_step_fused(AsHandle* h, const AsStateIn* in, const float* actions, int64_
     // the stone rows.  A programmatic dependent of the step kernel: launch and prologue hide under its last wave.
     ResetArgs r = make_reset_args(h, in->env_origins);
     r.fused = 1;
-    // shape of the kernel: a warp per env for small batches, a thread per env for large ones (ALLSTEPS_REGEN_MODE: 1 / 2)
-    const bool by_warp = h->regen_mode == 1 || (h->regen_mode == 0 && h->num_envs <= kRegenByWarpMaxEnvs);
-    const int grid_ctas = grid_for(h->num_envs, 64, h->sm_count, 8);
-    AS_CUDA(launch_dependent(by_warp ? k_reset_rows<true> : k_reset_rows<false>, static_cast<unsigned>(grid_ctas), 256u, 0, s,
-                             h->pdl >= 1, r));
-    if (int rc = check_launch(h, "k_reset_rows")) return rc;
+    if (int rc = launch_regeneration(h, r, s)) return rc;
   }
   h->pending = a;
   h->pending_valid = true;
@@ -773,10 +779,20 @@ int as_reset(AsHandle* h, const float* env_origins, const int32_t* env_ids, int6
   r.ext_episode_length = episode_length;
   r.fused = 0;
   r.into_other = h->spec_valid ? 1 : 0;  // behind a speculating pass 1 the step continues in the other state buffer
+  const bool regen_enabled = (h->params.flags & (AS_FLAG_GRID_CURRICULUM | AS_FLAG_INTENDED_REGEN)) != 0;
+  // (k_reset_list lists the envs that regenerate: the list starts empty)
+  if (regen_enabled) AS_CUDA(cudaMemsetAsync(&h->ws.ctrl->n_regen_list, 0, sizeof(uint32_t), s));
   // (four envs per warp; with the device-side list the count is only known on the device: sized for a tenth of the envs)
   const int grid = grid_for(from_device_list ? h->num_envs / 10 + 1 : n_ids, 32, h->sm_count, 3);
   k_reset_list<<<grid, 256, 0, s>>>(r);
-  return check_launch(h, "k_reset_list");
+  if (int rc = check_launch(h, "k_reset_list")) return rc;
+  if (!regen_enabled) return AS_OK;
+  // grid turnover and stones of the listed envs, by the kernel the fused step uses
+  if (int rc = launch_regeneration(h, r, s)) return rc;
+  // (k_pass2_commit clears the list when it closes the step; outside a step nothing follows that would, and a fused
+  // step must start with an empty list)
+  if (!r.into_other) AS_CUDA(cudaMemsetAsync(&h->ws.ctrl->n_regen_list, 0, sizeof(uint32_t), s));
+  return AS_OK;
 }
 
 int as_step_pass2(AsHandle* h, const AsStateIn* in, float* obs, void* stream) {

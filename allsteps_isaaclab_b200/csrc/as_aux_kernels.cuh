@@ -1,8 +1,8 @@
 // Kernels (b) and (c) plus the small adapters around the fused step:
 //   k_reset_list      3-call path: start-pose rows for PhysX (ENV:505-565) from the same Philox draws the step kernel
-//                     uses, MDP words, stone regeneration for an explicit / device-compacted id list
-//   k_reset_rows      fused path: grid-curriculum turnover + stone-sequence regeneration (ENV:106-174) for the envs the
-//                     step kernel listed
+//                     uses, MDP words, the list of envs to regenerate, for an explicit / device-compacted id list
+//   k_reset_rows      grid-curriculum turnover + stone-sequence regeneration (ENV:106-174) for the envs the fused step
+//                     kernel or k_reset_list listed
 //   k_generate_stones stone sequences for all / listed envs (init, ENV:71)
 //   k_apply_action    ENV:257-274
 //   k_mirror_batch    ENV:570-660 (mirror-symmetry augmentation; 128-row tiles through shared memory by TMA bulk copies)
@@ -152,7 +152,7 @@ __device__ __forceinline__ void stone_draws(const ResetArgs& a, unsigned long lo
 //   fused = 1: lists were compacted by the step kernel (ws.reset_ids / ws.regen_ids), MDP words already reset;
 //              PhysX rows are written at the env's own row of full-size buffers.
 //   fused = 0: explicit `env_ids` (3-call path): also resets the MDP word and the DirectRLEnv episode counter,
-//              decides regeneration, writes compact rows.
+//              decides regeneration and lists the envs that regenerate for k_reset_rows, writes compact rows.
 __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ ResetArgs a) {
   const AsParams& P = a.P;
   Ctrl* ctrl = a.ws.ctrl;
@@ -162,21 +162,13 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
   const unsigned long long step = ctrl->step_counter;
   // fused: the step kernel already wrote the start-pose rows; n_ids < 0: the list pass 1 compacted on the device
   const int64_t n_reset = a.fused ? 0 : (a.n_ids < 0 ? static_cast<int64_t>(ctrl->n_reset_list) : a.n_ids);
-  // promotion decided in THIS step is already in force when stones are regenerated (ENV:471 precedes ENV:500)
-  int promote_now;
-  if (!a.fused) {
-    // 3-call path: `_reset_idx` opens with the promotion rule (ENV:471-479) on the statistics pass 1 folded; every
-    // warp evaluates it for itself, one thread leaves the decision for the next pass 1 (nobody reads it in here)
+  if (!a.fused && blockIdx.x == 0 && threadIdx.x == 0) {
+    // 3-call path: `_reset_idx` opens with the promotion rule (ENV:471-479) on the statistics pass 1 folded.  The
+    // decision is in force from here on: k_reset_rows regenerates at the promoted level (ENV:471 precedes ENV:500),
+    // the next pass 1 applies it to the state words
     AsStats s = ctrl->stats;
     if (a.force_any_reset) s.n_reset = s.n_reset > 0 ? s.n_reset : 1;
-    promote_now = static_cast<int>(promotion_decision(P, s));
-    if (blockIdx.x == 0 && threadIdx.x == 0) ctrl->promote_cur = static_cast<uint32_t>(promote_now);
-  } else if (a.global_stats) {
-    promote_now = static_cast<int>(promotion_decision(P, a.global_stats->stats));
-  } else {  // the step kernel's counters are still in the replicated slots (folded by the finish kernel)
-    const unsigned nr = slot_sum(ctrl, kCntReset);
-    const unsigned si = slot_sum(ctrl, kCntSumIndex);
-    promote_now = static_cast<int>(promotion_rule(P, nr, si, a.num_envs));
+    ctrl->promote_cur = promotion_decision(P, s);
   }
   const uint32_t parity = ctrl->parity;
   // fused: the step wrote the other buffer; 3-call path after a speculating pass 1: so did that pass
@@ -189,17 +181,16 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
     const int64_t w = w0 + grp;
     const bool have = w < n_reset;
     int64_t e = 0;
-    int level = 0;
+    uint32_t word = 0;
     bool regen = false;
-    float ox = 0.f, oy = 0.f, oz = 0.f;
     if (have) {
       e = a.env_ids[w];
       const int64_t row = w;
       const uint32_t gid = static_cast<uint32_t>(e + a.env_id_offset);
-      const uint32_t word = st_cur[e].x;
-      ox = a.env_origins[e * 3];
-      oy = a.env_origins[e * 3 + 1];
-      oz = a.env_origins[e * 3 + 2];
+      word = st_cur[e].x;
+      const float ox = a.env_origins[e * 3];
+      const float oy = a.env_origins[e * 3 + 1];
+      const float oz = a.env_origins[e * 3 + 2];
       const uint4 b0 = philox_block(P.seed, step, kStreamReset, gid, 0);
       const bool mirror = u32_to_unit(b0.x) > 0.5f;  // ENV:518
       for (int j = g; j < kJ; j += 8) {
@@ -221,8 +212,8 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
           a.out.root_state[row * AS_ROOT_STATE_DIM + c] = val;
         }
       }
-      level = min(state_level(word) + promote_now, P.max_level);
-      regen = (P.flags & AS_FLAG_INTENDED_REGEN) && state_idx(word) > kS / 2;
+      // the rule of the fused step kernel: every env with the grid curriculum, else those past half of their stones
+      regen = (P.flags & AS_FLAG_GRID_CURRICULUM) || ((P.flags & AS_FLAG_INTENDED_REGEN) && state_idx(word) > kS / 2);
       if (g == 0) {
         if (a.out.reset_ids) a.out.reset_ids[w] = static_cast<int32_t>(e);
         a.ws.reset_ids[w] = static_cast<int32_t>(e);  // (k_pass2_commit walks this list)
@@ -233,21 +224,27 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
         if (a.ext_episode_length) a.ext_episode_length[e] = 0;
       }
     }
-    // regeneration takes the whole warp (one stone per lane): the groups that need it take turns
-    const unsigned rmask = __ballot_sync(kFullMask, have && regen);
-    for (int q = 0; q < 4; ++q) {
-      if (!((rmask >> (q * 8)) & 1u)) continue;
-      const int64_t eq = __shfl_sync(kFullMask, e, q * 8);
-      const int lq = __shfl_sync(kFullMask, level, q * 8);
-      const Vec3 org{__shfl_sync(kFullMask, ox, q * 8), __shfl_sync(kFullMask, oy, q * 8),
-                     __shfl_sync(kFullMask, oz, q * 8)};
-      float u0, u1, u2;
-      stone_draws(a, step, eq, static_cast<uint32_t>(eq + a.env_id_offset), lane, u0, u1, u2);
-      generate_stones_warp(P, lane, difficulty_of_env(P, a.ws, eq, lq), org, u0, u1, u2, a.ws.stones + eq * kS);
-      if (lane == 0) atomicAdd(reinterpret_cast<unsigned long long*>(&ctrl->stats.n_regenerated), 1ull);
+    // the envs that regenerate join the list k_reset_rows (launched behind this kernel) works through: the grid
+    // turnover and the stones, the same kernel as behind the fused step.  regen_info: the index the episode ended at
+    // (the word as pass 1 left it -- read above, before the reset overwrote it)
+    const bool listed = have && regen && g == 0;
+    const unsigned lmask = __ballot_sync(kFullMask, listed);
+    if (lmask) {
+      const int leader = __ffs(lmask) - 1;
+      unsigned base = 0;
+      if (lane == leader) {
+        base = atomicAdd(&ctrl->n_regen_list, static_cast<unsigned>(__popc(lmask)));
+        atomicAdd(reinterpret_cast<unsigned long long*>(&ctrl->stats.n_regenerated),
+                  static_cast<unsigned long long>(__popc(lmask)));
+      }
+      base = __shfl_sync(kFullMask, base, leader);
+      if (listed) {
+        const unsigned pos = base + __popc(lmask & ((1u << lane) - 1u));
+        a.ws.regen_ids[pos] = static_cast<int32_t>(e);
+        a.ws.regen_info[pos] = static_cast<uint8_t>(state_idx(word));
+      }
     }
-    __syncwarp();
-    if (have && g < 4) {  // the env restarts at index 1: its stone window
+    if (have && !regen && g < 4) {  // the env restarts at index 1 on its stones: its stone window
       float4 v = a.ws.stones[e * kS + window_slot_stone(1, g)];
       if (g == 0) v.w = __int_as_float(1);
       a.ws.window[e * 4 + g] = v;
@@ -261,7 +258,10 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
 
 
 // ------------------------------------------------------------------------------------------------ kernels (b) + (c)
-// Behind the fused step: everything that happens to the envs the step kernel listed for regeneration, in ONE launch.
+// Everything that happens to the envs listed for regeneration, in ONE launch: behind the fused step the step kernel
+// listed them (fused = 1), on the 3-call path k_reset_list did (fused = 0; there the draws are at the step counter
+// pass 1 or k_prepare_reset advanced to, the outcomes join the histograms when k_pass2_commit closes the step, and a
+// reset outside a step -- into_other = 0 -- records none).
 //   (c) grid-curriculum extension (no reference counterpart; specification = oracle/grid_curriculum.py): the outcome of
 //       the episode that just ended is recorded against the bin the env WAS playing -- a shared-memory histogram per
 //       CTA, flushed with one atomic per touched bin into the step's outcome record (Ctrl::grid_delta_*), which joins
@@ -316,13 +316,15 @@ __global__ void __launch_bounds__(256, 4) k_reset_rows(const __grid_constant__ R
     __syncthreads();
   }
   const unsigned long long step = ctrl->step_counter;
+  // a reset outside a step (3-call path without a pass 1: DirectRLEnv.reset()) ends no episode: new bins, no outcomes
+  const bool record = a.fused || a.into_other;
   // outcome of list entry w (env e) against the bin it played, then the new bin of the env
   auto grid_turnover = [&](int64_t w, int64_t e) -> int {
     const int b0 = a.ws.bin[e];
-    if (BY_WARP) {  // a short list spread over many CTAs: straight into the step's outcome record
+    if (record && BY_WARP) {  // a short list spread over many CTAs: straight into the step's outcome record
       atomicAdd(&ctrl->grid_delta_att[b0], 1u);
       if (a.ws.regen_info[w] > kS / 2) atomicAdd(&ctrl->grid_delta_succ[b0], 1u);
-    } else {
+    } else if (record) {
       atomicAdd(&s_att[b0], 1u);
       if (a.ws.regen_info[w] > kS / 2) atomicAdd(&s_succ[b0], 1u);
     }
@@ -339,14 +341,18 @@ __global__ void __launch_bounds__(256, 4) k_reset_rows(const __grid_constant__ R
   };
   // promotion decided in THIS step is already in force when stones are regenerated (ENV:471 precedes ENV:500)
   int promote_now;
-  if (a.global_stats) {
+  if (!a.fused) {  // 3-call path: k_reset_list, launched before, decided it
+    promote_now = static_cast<int>(ctrl->promote_cur);
+  } else if (a.global_stats) {
     promote_now = static_cast<int>(promotion_decision(P, a.global_stats->stats));
   } else {  // the step kernel's counters are still in the replicated slots (folded by the finish kernel)
     const unsigned nr = slot_sum(ctrl, kCntReset);
     const unsigned si = slot_sum(ctrl, kCntSumIndex);
     promote_now = static_cast<int>(promotion_rule(P, nr, si, a.num_envs));
   }
-  const uint2* st_cur = a.ws.state[ctrl->parity ^ 1u];  // (the step wrote the other buffer)
+  // the state words as reset: the fused step and a speculating pass 1 wrote the other buffer, a reset outside a step
+  // the current one
+  const uint2* st_cur = a.ws.state[record ? ctrl->parity ^ 1u : ctrl->parity];
   if (BY_WARP) {
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * blockDim.x + t) >> 5;
     for (int64_t w = warp; w < n_regen; w += n_warps) {
@@ -813,9 +819,19 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
     s_last = atomicAdd(&ctrl->blocks_done2, 1u) == gridDim.x - 1 ? 1u : 0u;
   }
   __syncthreads();
+  if (s_last && (P.flags & AS_FLAG_GRID_CURRICULUM)) {
+    // this step's episode outcomes (k_reset_rows) join the difficulty-grid histograms of this shard, as the fused
+    // step's finish does
+    for (int i = threadIdx.x; i < kMaxGridBins; i += blockDim.x) {
+      ctrl->grid_attempts[i] += ctrl->grid_delta_att[i];
+      ctrl->grid_successes[i] += ctrl->grid_delta_succ[i];
+      ctrl->grid_delta_att[i] = ctrl->grid_delta_succ[i] = 0u;
+    }
+  }
   if (s_last && threadIdx.x == 0) {
     ctrl->parity ^= 1u;
     ctrl->n_reset_list = 0;
+    ctrl->n_regen_list = 0;
     ctrl->blocks_done2 = 0;
   }
 }

@@ -97,6 +97,10 @@ struct Ctrl {
 static_assert(offsetof(Ctrl, grid_delta_att) == offsetof(Ctrl, stats) + sizeof(AsStats) &&
                   offsetof(Ctrl, grid_delta_succ) == offsetof(Ctrl, grid_delta_att) + sizeof(unsigned int) * kMaxGridBins,
               "Ctrl::stats and the grid outcome arrays form one AsExchange");
+// (mdp.py reads the histograms in place at this distance behind the statistics: _cabi.GRID_HIST_OFFSET)
+static_assert(offsetof(Ctrl, grid_attempts) == offsetof(Ctrl, stats) + sizeof(AsExchange) + 1664 &&
+                  offsetof(Ctrl, grid_successes) == offsetof(Ctrl, grid_attempts) + sizeof(unsigned int) * kMaxGridBins,
+              "the difficulty-grid histograms sit 1664 bytes behind the exchange record");
 
 // Peer exchange buffer of one rank: for each of the two epoch parities one 128-byte slot per sending rank.
 constexpr int kMaxPeers = AS_MAX_PEERS;

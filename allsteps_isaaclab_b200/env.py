@@ -48,6 +48,14 @@ def resolve_robot_tables(robot, cfg: AllstepsCfg):
     return body_rows, limits[0].detach().to(torch.float32).cpu()
 
 
+def write_stone_poses(steps, mdp: AllstepsMDP, env_ids: torch.Tensor):
+    """ENV:119-120: the stones of `env_ids` as the MDP holds them, written to the simulator's stone collection
+    (`RigidObjectCollection.write_object_pose_to_sim`, poses (k,S,7): position + identity quaternion w,x,y,z)."""
+    pos = mdp.export_state(("steps_pos",))["steps_pos"][env_ids]
+    quat = torch.tensor([1.0, 0.0, 0.0, 0.0], device=pos.device).expand(pos.shape[0], NUM_STONES, 4)
+    steps.write_object_pose_to_sim(torch.cat((pos, quat), dim=-1), env_ids)  # ENV:119-120
+
+
 class AllstepsHooksB200:
     """Hook methods of `AllstepsEnv(DirectRLEnv)` (ENV:34) backed by `AllstepsMDP`."""
 
@@ -86,13 +94,13 @@ class AllstepsHooksB200:
     # ------------------------------------------------------------------ ENV:106-123
     def _generate_foot_steps(self, env_ids: Optional[torch.Tensor] = None):
         self.mdp.generate_stones(self.scene.env_origins, env_ids)
+        self._write_stone_poses(env_ids if env_ids is not None else torch.arange(self.num_envs, device=self.device))
+
+    def _write_stone_poses(self, env_ids: torch.Tensor):
+        """The stones of `env_ids` to the `steps` collection, when the env has one (built by `_setup_scene`)."""
         steps = getattr(self, "steps", None)
         if steps is not None and hasattr(steps, "write_object_pose_to_sim"):
-            pos = self.steps_pos
-            quat = torch.tensor([1.0, 0.0, 0.0, 0.0], device=pos.device).expand(self.num_envs, NUM_STONES, 4)
-            pose = torch.cat((pos, quat), dim=-1)  # ENV:119
-            ids = env_ids if env_ids is not None else torch.arange(self.num_envs, device=pos.device)
-            steps.write_object_pose_to_sim(pose[ids], ids)  # ENV:120
+            write_stone_poses(steps, self.mdp, env_ids)
 
     # ------------------------------------------------------------------ the six hooks
     def _pre_physics_step(self, actions: torch.Tensor):  # ENV:257-268 (the clamp is applied inside the kernels)
@@ -124,6 +132,11 @@ class AllstepsHooksB200:
         self.robot.reset(env_ids)
         super()._reset_idx(env_ids)  # scene.reset (contact rows -> 0) and episode_length_buf[env_ids] = 0, DRL:563-584
         self.mdp.reset(self.scene.env_origins, env_ids, self.buf)
+        if self.mdp.regenerates:
+            # ENV:497-500 -> ENV:119-120: stones regenerated by the reset go to PhysX.  All rows of the reset envs are
+            # written, also those intended regeneration left as they were (same values; cheaper than a host sync
+            # to learn which ones changed)
+            self._write_stone_poses(env_ids)
         k = len(env_ids)
         root = self.buf.reset_root_state[:k]
         self.robot.write_root_pose_to_sim(root[:, :7], env_ids)  # ENV:563

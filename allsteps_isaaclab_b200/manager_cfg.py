@@ -7,7 +7,8 @@
                                                     by weight * dt), or the ten terms of ENV:350-375 (`per_term=True`)
     TerminationManager(cfgs["terminations"], env)   fell | so_fast | died, and the time-out with `time_out=True`
     EventManager(cfgs["events"], env)               `reset_allsteps` in mode "reset" (ENV:469-567)
-    CurriculumManager(cfgs["curriculum"], env)      `allsteps_level` (logging; the promotion happens in the reset)
+    CurriculumManager(cfgs["curriculum"], env)      `allsteps_level` (logging; the promotion happens in the reset),
+                                                    and `allsteps_grid` with `grid_curriculum=True`
 
 -- built from the cfg classes of the `isaaclab.managers` module that is passed in (default: the installed Isaac Lab).
 Every term's scene entities are named by `SceneEntityCfg` params, which `ManagerBase._resolve_common_term_cfg`
@@ -24,7 +25,9 @@ from .config import AllstepsCfg
 
 def build_manager_cfgs(managers=None, robot: str = "robot", left_sensor: str = "foot_contacts_left",
                        right_sensor: str = "foot_contacts_right", task_cfg: AllstepsCfg | None = None,
-                       per_term_rewards: bool = False) -> Dict[str, Any]:
+                       per_term_rewards: bool = False, grid_curriculum: bool = False) -> Dict[str, Any]:
+    """grid_curriculum: also log the difficulty-grid curriculum through the `allsteps_grid` curriculum term.  The grid
+    itself is switched on where the MDP is made: `terms.binding(env, grid_bins=B)` before the managers are built."""
     M = managers if managers is not None else importlib.import_module("isaaclab.managers")
     cfg = task_cfg or AllstepsCfg()
 
@@ -53,5 +56,7 @@ def build_manager_cfgs(managers=None, robot: str = "robot", left_sensor: str = "
     }
     events = {"reset_allsteps": M.EventTermCfg(func=terms.reset_allsteps, mode="reset", params=ent())}
     curriculum = {"allsteps_level": M.CurriculumTermCfg(func=terms.allsteps_level, params=ent())}
+    if grid_curriculum:
+        curriculum["allsteps_grid"] = M.CurriculumTermCfg(func=terms.allsteps_grid, params=ent())
     return {"observations": observations, "rewards": rewards, "terminations": terminations, "events": events,
             "curriculum": curriculum}

@@ -207,6 +207,13 @@ class AllstepsMDP:
         # (two uint32 counters per int64 word; the sums cannot carry) -- and hands to `finish_step`
         self.exchange_tensor = self.workspace[off: off + C.sizeof(_cabi.AsExchange)].view(torch.int64)
         self.grid_words = slice(_cabi.STATS_INT64_WORDS, _cabi.EXCHANGE_INT64_WORDS)
+        # ... and of the difficulty-grid histograms: attempts in [:256], successes in [256:] (bin b = pitch bin *
+        # grid_bins + yaw bin; uint32 counters read as int32) -- what a logger reads without a copy or a synchronisation
+        h0 = off + C.sizeof(_cabi.AsExchange) + _cabi.GRID_HIST_OFFSET
+        self.grid_hist_tensor = self.workspace[h0: h0 + 8 * _cabi.MAX_GRID_CELLS].view(torch.int32)
+        # every env that resets may get new stones (grid curriculum, intended regeneration): a host that keeps the
+        # stones in a simulator must write them there after each reset
+        self.regenerates = bool(flags & (_cabi.FLAG_GRID_CURRICULUM | _cabi.FLAG_INTENDED_REGEN))
         self._keepalive = None
 
     # ------------------------------------------------------------------ plumbing
@@ -351,7 +358,8 @@ class AllstepsMDP:
               episode_length: Optional[torch.Tensor] = None):
         """`_reset_idx(env_ids)` minus the PhysX writes.  env_ids None: the envs the preceding `pass1` flagged, taken
         from the id list that pass compacted on the device -- no `.nonzero()`, no host round trip; `out.reset_ids[:n]`
-        / `out.n_reset` (device) name them, rows are in that order."""
+        / `out.n_reset` (device) name them, rows are in that order.  With `regenerates`, the stones of the reset envs
+        may have changed (grid curriculum: new bin and stones for every one of them): write them to the simulator too."""
         if env_ids is None:
             _cabi.check(self.lib.as_reset(self.handle, env_origins.data_ptr(), None, -1, _ptr(episode_length),
                                           C.byref(out.reset_out), self._stream()), "as_reset")

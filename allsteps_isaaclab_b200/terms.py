@@ -55,14 +55,18 @@ class _Binding:
     """Per-env glue shared by all terms: the MDP object, the output buffers and the per-step cache."""
 
     def __init__(self, env, robot="robot", left="foot_contacts_left", right="foot_contacts_right", seed=0,
-                 task_cfg: Optional[AllstepsCfg] = None):
+                 task_cfg: Optional[AllstepsCfg] = None, grid_bins: int = 0, intended_regen: bool = False):
+        """grid_bins / intended_regen: the `AllstepsMDP` extensions (difficulty-grid curriculum with grid_bins per
+        axis; regeneration of the stones of envs that had passed half of them).  Both regenerate stones in
+        `reset_allsteps`, which then writes them to the scene's stone collection."""
         from .env import resolve_robot_tables
 
         self.cfg = task_cfg or AllstepsCfg()
         self.names = (robot, left, right)
         dev = torch.device(env.device)
         self.body_rows, joint_limits = resolve_robot_tables(env.scene[robot], self.cfg)
-        self.mdp = AllstepsMDP(env.num_envs, device=dev, cfg=self.cfg, seed=seed, joint_limits=joint_limits)
+        self.mdp = AllstepsMDP(env.num_envs, device=dev, cfg=self.cfg, seed=seed, joint_limits=joint_limits,
+                               grid_bins=grid_bins, intended_regen=intended_regen)
         self.buf = StepBuffers(env.num_envs, dev, reward_terms=True)
         self.buf.obs.zero_()
         self.buf.reward.zero_()
@@ -177,9 +181,12 @@ def allsteps_time_out(env, asset_cfg=None, left_sensor_cfg=None, right_sensor_cf
 
 # ---------------------------------------------------------------------------------------------- reset event
 def reset_allsteps(env, env_ids, write_to_sim: bool = True, asset_cfg=None, left_sensor_cfg=None,
-                   right_sensor_cfg=None):
+                   right_sensor_cfg=None, stones_cfg="steps"):
     """EventManager `mode="reset"` term, ENV:469-567: MDP reset + start pose + PhysX writes + pass 2.  `env_ids` is
-    what EventManager.apply hands over (event_manager.py:219-240): an index tensor, `slice(None)` or None."""
+    what EventManager.apply hands over (event_manager.py:219-240): an index tensor, `slice(None)` or None.
+    `stones_cfg` names the stones' `RigidObjectCollection`: when the MDP regenerates stones (`binding(env,
+    grid_bins=...)` or `intended_regen=True`), the stones of the reset envs are written to it (ENV:119-120), if the
+    scene has it."""
     b = binding(env, asset_cfg, left_sensor_cfg, right_sensor_cfg)
     b.ensure_pass1(env)
     if env_ids is None or isinstance(env_ids, slice):
@@ -188,6 +195,15 @@ def reset_allsteps(env, env_ids, write_to_sim: bool = True, asset_cfg=None, left
         return
     b.mdp.reset(env.scene.env_origins, env_ids, b.buf, episode_length=env.episode_length_buf)
     k = len(env_ids)
+    if write_to_sim and b.mdp.regenerates:
+        from .env import write_stone_poses
+
+        try:
+            stones = env.scene[_entity_name(stones_cfg, "steps")]
+        except KeyError:  # a scene without stone bodies: nothing to move
+            stones = None
+        if stones is not None:
+            write_stone_poses(stones, b.mdp, env_ids)
     if write_to_sim:
         robot = env.scene[b.names[0]]
         root = b.buf.reset_root_state[:k]
@@ -208,3 +224,19 @@ def allsteps_level(env, env_ids, asset_cfg=None, left_sensor_cfg=None, right_sen
     s = b.mdp.stats_tensor  # int64 view of the device AsStats: 0 n_envs ... 8 sum_target_index ... 10 level
     n = torch.clamp(s[0], min=1).to(torch.float32)
     return {"level": s[10].to(torch.float32), "mean_target_index": s[8].to(torch.float32) / n}
+
+
+def allsteps_grid(env, env_ids, asset_cfg=None, left_sensor_cfg=None, right_sensor_cfg=None) -> Dict[str, torch.Tensor]:
+    """CurriculumManager term of the difficulty-grid curriculum (`binding(env, grid_bins=B)`): episodes ended so far
+    (`attempts`), the share of them that passed half of their stones (`success_rate`) and the number of bins played at
+    least once (`bins_visited`), as 0-dim device tensors read from the histograms in place -- no copy of the per-env
+    bins, no synchronisation, no MDP pass.  The turnover itself happens inside `reset_allsteps`."""
+    b = binding(env, asset_cfg, left_sensor_cfg, right_sensor_cfg)
+    nb = b.mdp.grid_bins * b.mdp.grid_bins
+    h = b.mdp.grid_hist_tensor
+    att = h[:nb].to(torch.int64)
+    succ = h[256:256 + nb].to(torch.int64)
+    total = att.sum()
+    return {"attempts": total.to(torch.float32),
+            "success_rate": succ.sum().to(torch.float32) / torch.clamp(total, min=1).to(torch.float32),
+            "bins_visited": (att > 0).sum().to(torch.float32)}

@@ -52,7 +52,9 @@ enum {
                                        ENV:497 runs after ENV:492 and is never true (SURVEY D3).            */
   AS_FLAG_SKIP_PASS2 = 1u << 1,     /* extension: never run the second `_compute_useful_values` pass
                                        (ENV:567, SURVEY D7) for envs that did not reset.  Off = reference. */
-  AS_FLAG_GRID_CURRICULUM = 1u << 2,/* extension: pitch x yaw difficulty grid sampling at regeneration.   */
+  AS_FLAG_GRID_CURRICULUM = 1u << 2,/* extension: pitch x yaw difficulty grid sampling at regeneration:
+                                       every env that resets -- in as_step_fused or in as_reset -- gets a new
+                                       bin and new stones (see as_grid_state).                              */
   AS_FLAG_MISSED_STEP = 1u << 3     /* extension (BASELINE north_star "missed-step termination"; the reference's
                                        ENV:396-405 has none, SURVEY D4): an env also terminates when its swing foot
                                        has come down below the top of the stone it is heading for, outside that stone's
@@ -231,6 +233,10 @@ int as_step_fused(AsHandle* h, const AsStateIn* in, const float* actions, int64_
  *         Called without a preceding as_step_pass1 (DirectRLEnv.reset() runs `_reset_idx(all ids)` before the first
  *         step, DRL:256-279) it evaluates the promotion rule on the indices as they are and advances the Philox
  *         step counter itself.
+ *         With AS_FLAG_GRID_CURRICULUM or AS_FLAG_INTENDED_REGEN it regenerates stones by the rule of the fused step
+ *         (every listed env with the grid, those past num_steps/2 with intended regeneration; AsStats.n_regenerated
+ *         counts them): the caller writes the stones of the reset envs to its simulator (as_export_state /
+ *         as_export_stone_poses).  Grid outcomes: see as_grid_state.
  * pass2:  the second `_compute_useful_values` over ALL envs + `_get_observations`, on the post-write state.  No
  *         call-order precondition (ENV:567 runs whether or not a pass preceded the reset). */
 int as_step_pass1(AsHandle* h, const AsStateIn* in, const float* actions, int64_t actions_stride,
@@ -349,13 +355,20 @@ int as_export_stone_poses(AsHandle* h, const int32_t* env_ids, int64_t n_ids, fl
 
 /* ---- grid curriculum (EXTENSION: AS_FLAG_GRID_CURRICULUM; no reference counterpart, specification in
  * oracle/grid_curriculum.py) --------------------------------------------------------------------------------------
- * With the flag set, every env that resets in as_step_fused has its episode outcome added to a (grid_bins x
- * grid_bins) pitch x yaw difficulty histogram, is assigned a new bin by inverse-CDF sampling, and gets a stone
- * sequence regenerated at that bin's difficulty.  as_grid_state copies the per-env bins (N bytes) and the two
- * histograms (attempts[256] then successes[256], uint32) out of / into the device state; NULL = skip.
+ * With the flag set, every env that resets -- in as_step_fused, or in as_reset on the 3-call path -- has its episode
+ * outcome added to a (grid_bins x grid_bins) pitch x yaw difficulty histogram, is assigned a new bin by inverse-CDF
+ * sampling, and gets a stone sequence regenerated at that bin's difficulty, its stone window rebuilt at index 1.
+ * as_grid_state copies the per-env bins (N bytes) and the two histograms (attempts[256] then successes[256], uint32)
+ * out of / into the device state; NULL = skip.
  * Bins drawn in step t use the histograms as they stand after step t-1; the outcomes of step t are added when the step
- * is closed (as_finish_step) -- summed over all shards when the step is closed on a global record, so that sharded
- * runs sample from the same CDF as one handle holding all envs. */
+ * is closed: by as_finish_step -- summed over all shards when the step is closed on a global record, so that sharded
+ * runs sample from the same CDF as one handle holding all envs -- or, on the 3-call path, by as_step_pass2.  On the
+ * 3-call path the histograms are shard-local (as its promotion rule is): each shard samples from its own outcomes.
+ * The draws of as_reset are made at the step counter as_step_pass1 advanced to, so bins and stones differ from those
+ * of a fused step on the same inputs.  A step in which nothing resets (as_step_no_reset, or an empty device-side list)
+ * records nothing.  A reset outside a step (as_reset with no as_step_pass1 before it: DirectRLEnv.reset()) ends no
+ * episode: the envs draw new bins and stones but no outcome is recorded -- at start-up that would count every env as a
+ * failure of bin 0 and push the sampler away from the easiest bin before training begins. */
 int as_grid_state(AsHandle* h, uint8_t* bins_dst, const uint8_t* bins_src, uint32_t* hist_dst, const uint32_t* hist_src,
                   void* stream);
 
