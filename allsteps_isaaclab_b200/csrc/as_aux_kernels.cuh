@@ -276,10 +276,25 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
 // (BASELINE config 5: 257 000 of 1 M envs regenerate per step).
 constexpr uint32_t kStreamGrid = 2;
 
+// 1 + 1024 s (a - s) / (a^2 + 1), exact for every s <= a < 2^32: s (a - s) < 2^62 and a^2 + 1 < 2^64 fit 64 bits,
+// the product with 1024 does not.  The quotient has ten bits (every weight is in 1..256), so it is formed by ten
+// steps of binary long division; s (a - s) < a^2 + 1 keeps every partial remainder below the divisor.
 __device__ __forceinline__ unsigned int grid_weight(unsigned int a, unsigned int s) {
   if (a == 0) return 256u;  // unvisited bins are tried
-  const unsigned long long A = a, S = s;
-  return 1u + static_cast<unsigned int>((1024ull * S * (A - S)) / (A * A + 1ull));  // peaks at a 50 % success rate
+  const unsigned long long A = a, S = s, den = A * A + 1ull;
+  unsigned long long rem = S * (A - S);
+  unsigned int q = 0;
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    const bool carry = (rem >> 63) != 0;  // 2 rem passes 2^64: it exceeds den, and the wrapped difference is exact
+    rem <<= 1;
+    q <<= 1;
+    if (carry || rem >= den) {
+      rem -= den;
+      q |= 1u;
+    }
+  }
+  return 1u + q;  // peaks at a 50 % success rate
 }
 
 template <bool BY_WARP>
@@ -823,8 +838,7 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
     // this step's episode outcomes (k_reset_rows) join the difficulty-grid histograms of this shard, as the fused
     // step's finish does
     for (int i = threadIdx.x; i < kMaxGridBins; i += blockDim.x) {
-      ctrl->grid_attempts[i] += ctrl->grid_delta_att[i];
-      ctrl->grid_successes[i] += ctrl->grid_delta_succ[i];
+      grid_fold(ctrl->grid_attempts[i], ctrl->grid_successes[i], ctrl->grid_delta_att[i], ctrl->grid_delta_succ[i]);
       ctrl->grid_delta_att[i] = ctrl->grid_delta_succ[i] = 0u;
     }
   }

@@ -102,6 +102,18 @@ static_assert(offsetof(Ctrl, grid_attempts) == offsetof(Ctrl, stats) + sizeof(As
                   offsetof(Ctrl, grid_successes) == offsetof(Ctrl, grid_attempts) + sizeof(unsigned int) * kMaxGridBins,
               "the difficulty-grid histograms sit 1664 bytes behind the exchange record");
 
+// One bin's step outcomes (da, ds) join its histogram counters (oracle/grid_curriculum.py, "fold"): a bin whose
+// attempts would pass 2^32 - 1 is halved first, which keeps its success ratio and successes <= attempts.  A step's
+// delta is below 2^31 (at most the run's env count), so one halving makes room.  Single writer: the closing CTA.
+__device__ __forceinline__ void grid_fold(unsigned int& att, unsigned int& succ, unsigned int da, unsigned int ds) {
+  if (static_cast<unsigned long long>(att) + da > 0xFFFFFFFFull) {
+    att >>= 1;
+    succ >>= 1;
+  }
+  att += da;
+  succ += ds;
+}
+
 // Peer exchange buffer of one rank: for each of the two epoch parities one 128-byte slot per sending rank.
 constexpr int kMaxPeers = AS_MAX_PEERS;
 constexpr int kPeerCounters = 10;  // the additive head of AsStats

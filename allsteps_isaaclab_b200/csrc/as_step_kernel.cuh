@@ -1736,8 +1736,9 @@ __global__ void __launch_bounds__(kThreads, 2) k_fixup_finish(const __grid_const
   if (a.P.flags & AS_FLAG_GRID_CURRICULUM) {
     // this step's episode outcomes join the difficulty-grid histograms (the sum over all shards when one was handed in)
     for (int i = tid; i < kMaxGridBins; i += blockDim.x) {
-      ctrl->grid_attempts[i] += a.global_stats ? a.global_stats->grid_attempts[i] : ctrl->grid_delta_att[i];
-      ctrl->grid_successes[i] += a.global_stats ? a.global_stats->grid_successes[i] : ctrl->grid_delta_succ[i];
+      grid_fold(ctrl->grid_attempts[i], ctrl->grid_successes[i],
+                a.global_stats ? a.global_stats->grid_attempts[i] : ctrl->grid_delta_att[i],
+                a.global_stats ? a.global_stats->grid_successes[i] : ctrl->grid_delta_succ[i]);
     }
     __syncthreads();
     for (int i = tid; i < kMaxGridBins; i += blockDim.x) ctrl->grid_delta_att[i] = ctrl->grid_delta_succ[i] = 0u;

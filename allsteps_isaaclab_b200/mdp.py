@@ -481,16 +481,38 @@ class AllstepsMDP:
         _cabi.check(self.lib.as_grid_state(self.handle, bins.data_ptr(), None, hist.data_ptr(), None,
                                            self._stream()), "as_grid_state")
         nb = self.grid_bins * self.grid_bins
-        return bins, hist[:nb].long(), hist[256:256 + nb].long()
+        # (uint32 counters: widen, then drop the sign extension)
+        return bins, hist[:nb].long() & 0xFFFFFFFF, hist[256:256 + nb].long() & 0xFFFFFFFF
 
     def set_grid_state(self, bins: Optional[torch.Tensor] = None, attempts=None, successes=None):
-        b = None if bins is None else bins.to(device=self.device, dtype=torch.uint8).contiguous()
+        """bins (N,) with values < B*B; attempts and successes (B*B,) each, 0 <= successes <= attempts < 2^32 (the
+        precondition of oracle/grid_curriculum.py).  Anything else raises ValueError before the handle is touched."""
+        nb = self.grid_bins * self.grid_bins
+        b = None
+        if bins is not None:
+            b64 = torch.as_tensor(bins).detach().to("cpu", torch.int64)
+            if tuple(b64.shape) != (self.num_envs,):
+                raise ValueError(f"bins must have shape ({self.num_envs},), got {tuple(b64.shape)}")
+            if b64.numel() and (int(b64.min()) < 0 or int(b64.max()) >= nb):
+                raise ValueError(f"bins must lie in [0, {nb}) for a {self.grid_bins}x{self.grid_bins} grid")
+            b = b64.to(device=self.device, dtype=torch.uint8)
         hist = None
+        if (attempts is None) != (successes is None):
+            raise ValueError("attempts and successes are set together")
         if attempts is not None:
-            hist = torch.zeros(512, dtype=torch.int32, device=self.device)
-            nb = self.grid_bins * self.grid_bins
-            hist[:nb] = attempts.to(self.device).int()
-            hist[256:256 + nb] = successes.to(self.device).int()
+            att = torch.as_tensor(attempts).detach().to("cpu", torch.int64)
+            succ = torch.as_tensor(successes).detach().to("cpu", torch.int64)
+            for name, x in (("attempts", att), ("successes", succ)):
+                if tuple(x.shape) != (nb,):
+                    raise ValueError(f"{name} must have shape ({nb},), got {tuple(x.shape)}")
+                if nb and (int(x.min()) < 0 or int(x.max()) > 0xFFFFFFFF):
+                    raise ValueError(f"{name} must lie in [0, 2^32): the histogram counters are uint32")
+            if bool((succ > att).any()):
+                raise ValueError("successes must not exceed attempts in any bin")
+            h = torch.zeros(512, dtype=torch.int64)
+            h[:nb] = att
+            h[256:256 + nb] = succ
+            hist = torch.where(h > 0x7FFFFFFF, h - (1 << 32), h).to(device=self.device, dtype=torch.int32)  # uint32 bits
         _cabi.check(self.lib.as_grid_state(self.handle, None, _ptr(b), None, _ptr(hist), self._stream()),
                     "as_grid_state")
         self._keepalive = (b, hist)

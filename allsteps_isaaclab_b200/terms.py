@@ -234,8 +234,8 @@ def allsteps_grid(env, env_ids, asset_cfg=None, left_sensor_cfg=None, right_sens
     b = binding(env, asset_cfg, left_sensor_cfg, right_sensor_cfg)
     nb = b.mdp.grid_bins * b.mdp.grid_bins
     h = b.mdp.grid_hist_tensor
-    att = h[:nb].to(torch.int64)
-    succ = h[256:256 + nb].to(torch.int64)
+    att = h[:nb].to(torch.int64) & 0xFFFFFFFF  # (uint32 counters behind an int32 view)
+    succ = h[256:256 + nb].to(torch.int64) & 0xFFFFFFFF
     total = att.sum()
     return {"attempts": total.to(torch.float32),
             "success_rate": succ.sum().to(torch.float32) / torch.clamp(total, min=1).to(torch.float32),

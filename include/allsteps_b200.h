@@ -359,7 +359,10 @@ int as_export_stone_poses(AsHandle* h, const int32_t* env_ids, int64_t n_ids, fl
  * outcome added to a (grid_bins x grid_bins) pitch x yaw difficulty histogram, is assigned a new bin by inverse-CDF
  * sampling, and gets a stone sequence regenerated at that bin's difficulty, its stone window rebuilt at index 1.
  * as_grid_state copies the per-env bins (N bytes) and the two histograms (attempts[256] then successes[256], uint32)
- * out of / into the device state; NULL = skip.
+ * out of / into the device state; NULL = skip.  Precondition on what is copied in: successes[b] <= attempts[b] for
+ * every bin, and every bin < grid_bins * grid_bins (a larger one would index the difficulty tables past their end);
+ * the library does not check it.  When a step's outcomes would carry a bin's attempts past 2^32 - 1, the bin is
+ * halved first (attempts >> 1, successes >> 1), which keeps its success ratio.
  * Bins drawn in step t use the histograms as they stand after step t-1; the outcomes of step t are added when the step
  * is closed: by as_finish_step -- summed over all shards when the step is closed on a global record, so that sharded
  * runs sample from the same CDF as one handle holding all envs -- or, on the 3-call path, by as_step_pass2.  On the

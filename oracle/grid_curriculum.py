@@ -11,8 +11,17 @@ Definition
   difficulty  ratio_pitch = i / (B-1), ratio_yaw = j / (B-1) scale the +-30 deg / +-20 deg ranges of ENV:42-43 the way
               the scalar ratio does in ENV:131-132; dist upper bound = dist_upper[(max(i,j) * max_level) // (B-1)]
   outcome     an episode that ends (the env resets) is a success iff its curr_target_index had passed S/2
-  histogram   attempts[b] += 1, successes[b] += success for the bin the env was playing
+  histogram   two uint32 counters per bin: attempts (episodes ended in the bin) and successes (of those)
+  fold        a step's outcomes join the histograms as one delta per bin, (da, ds) = episodes of the step that ended in
+              the bin and how many of them were successes.  If a + da > 2^32 - 1 (in mathematical integers), the bin is
+              halved first: (a, s) <- (a >> 1, s >> 1); then (a, s) <- (a + da, s + ds).  Halving keeps the success
+              ratio and s <= a; a step's delta is at most the run's env count (< 2^31), so one halving makes room.  The
+              rule depends on the global sums only, so shards keep identical histograms.  Below 2^32 - 1 - da it is a
+              plain addition.
+  precondition successes[b] <= attempts[b] for every bin, and every env's bin is < B * B
   weights     w_b = 256 if attempts == 0 else 1 + (1024 * s * (a - s)) // (a * a + 1)      (peaks at 50 % success)
+              on mathematical integers (the numerator needs up to 72 bits).  With s <= a every weight is in 1..256,
+              so the CDF total is at most 256 * 256 and fits a uint32 with room to spare.
   sampling    cdf = inclusive prefix sum of w; u24 = 24-bit uniform; target = (u24 * cdf[-1]) >> 24;
               new bin = first b with cdf[b] > target
   each env that resets is assigned a new bin and its stone sequence is regenerated at that bin's difficulty.
@@ -29,13 +38,14 @@ import torch
 from . import philox
 
 STREAM_GRID = 2
+U32_MAX = 0xFFFFFFFF  # the histogram counters are uint32
 
 
 def weights(attempts: np.ndarray, successes: np.ndarray) -> np.ndarray:
-    a = attempts.astype(np.uint64)
-    s = successes.astype(np.uint64)
-    w = np.uint64(1) + (np.uint64(1024) * s * (a - s)) // (a * a + np.uint64(1))
-    return np.where(a == 0, np.uint64(256), w).astype(np.uint32)
+    """The bin weights, evaluated in Python ints (exact; at most 256 bins)."""
+    w = [256 if a == 0 else 1 + (1024 * s * (a - s)) // (a * a + 1)
+         for a, s in zip(np.asarray(attempts).tolist(), np.asarray(successes).tolist())]
+    return np.array(w, dtype=np.uint32)
 
 
 def cdf_of(attempts: np.ndarray, successes: np.ndarray) -> np.ndarray:
@@ -46,6 +56,16 @@ def sample_bins(cdf: np.ndarray, u24: np.ndarray) -> np.ndarray:
     total = np.uint64(cdf[-1])
     target = (u24.astype(np.uint64) * total) >> np.uint64(24)
     return np.searchsorted(cdf.astype(np.uint64), target, side="right").astype(np.uint8)
+
+
+def fold(attempts: np.ndarray, successes: np.ndarray, d_att: np.ndarray, d_succ: np.ndarray) -> None:
+    """A step's per-bin outcomes (d_att, d_succ) join the uint32 histograms in place (see "fold" above)."""
+    for b, (da, ds) in enumerate(zip(np.asarray(d_att).tolist(), np.asarray(d_succ).tolist())):
+        a, s = int(attempts[b]), int(successes[b])
+        if a + da > U32_MAX:
+            a, s = a >> 1, s >> 1
+        attempts[b] = a + da
+        successes[b] = s + ds
 
 
 def grid_draws(seed: int, step: int, env_ids: np.ndarray) -> np.ndarray:
@@ -115,6 +135,7 @@ class GridCurriculum:
         cdf = cdf_of(self.attempts, self.successes)
         u24 = grid_draws(seed, step, env_ids + self.env_id_offset)
         self.bins[env_ids] = sample_bins(cdf, u24)
-        np.add.at(self.attempts, b, 1)
-        np.add.at(self.successes, b, (index_at_end > num_stones // 2).astype(np.uint32))
+        nb = self.attempts.shape[0]
+        ok = np.asarray(index_at_end) > num_stones // 2
+        fold(self.attempts, self.successes, np.bincount(b, minlength=nb), np.bincount(b[ok], minlength=nb))
         return self.bins[env_ids]

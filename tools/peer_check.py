@@ -71,12 +71,23 @@ def main():
                                                 "episode_length_buf", "potentials")})
     nccl_mdp, peer_mdp = mdps
     assert peer_mdp.connect_peers() == (world, rank)
+    # PEER_CHECK_NEAR_TOP=1 (with a grid): every handle starts from histograms a few counts below 2^32 - 1, so the
+    # steps' global outcomes halve bins (the fold of oracle/grid_curriculum.py) -- the same bins on every shard
+    near_top = grid and os.environ.get("PEER_CHECK_NEAR_TOP") == "1"
+    if near_top:
+        nb = grid * grid
+        top = torch.tensor([(1 << 32) - 1 - (b % 64) for b in range(nb)], dtype=torch.int64)
+        hist0 = (top, top * (torch.arange(nb) % 3) // 2)
+        for m in mdps:
+            m.set_grid_state(None, *hist0)
     single = None
     if rank == 0:  # ONE handle with all envs: what every shard has to reproduce
         single = AllstepsMDP(N, device=dev, seed=seed, grid_bins=grid)
         single.generate_stones(sc.env_origins.to(dev))
         single.import_state({k: st0[k] for k in ("curr_target_index", "swing_leg", "target_reach_count",
                                                  "episode_length_buf", "potentials")})
+        if near_top:
+            single.set_grid_state(None, *hist0)
         out_single = StepBuffers(N, dev)
     outs = [StepBuffers(per, dev), StepBuffers(per, dev)]
     g = torch.zeros_like(nccl_mdp.exchange_tensor)
@@ -152,6 +163,9 @@ def main():
         level = int(sb["curriculum"].max())
         promotions += int(level != level_before or grid > 0)
         level_before = level
+    if near_top:
+        att_end = peer_mdp.grid_state()[1].cpu()
+        assert bool((att_end < hist0[0] // 2 + (1 << 20)).any()), "no bin was halved; the check would prove nothing"
     status = peer_mdp.peer_status()
     assert status["timeouts"] == 0 and status["world"] == world, status
     assert promotions > 0, "no promotion happened; the check would prove nothing"
@@ -188,7 +202,8 @@ def main():
     t_peer = timed(lambda: peer_mdp.step(views, d["actions"], outs[1]))
     assert peer_mdp.peer_status()["timeouts"] == 0
     if rank == 0:
-        print(f"peer_check OK: world {world} ({backend}{', grid %dx%d' % (grid, grid) if grid else ''}), {per} envs per rank, {steps} steps, {promotions} promotions, "
+        print(f"peer_check OK: world {world} ({backend}{', grid %dx%d' % (grid, grid) if grid else ''}"
+              f"{' near the top of the counters' if near_top else ''}), {per} envs per rank, {steps} steps, {promotions} promotions, "
               f"shards == single handle; us/step: shard-local {t_local:.1f}, {backend} all-reduce {t_nccl:.1f}, "
               f"peer-memory exchange {t_peer:.1f}", flush=True)
     dist.destroy_process_group()
