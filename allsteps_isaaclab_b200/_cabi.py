@@ -139,6 +139,7 @@ SIGNATURES = {
     "as_peer_connect": (C.c_int, [_ptr, _ptr]),
     "as_peer_status": (C.c_int, [_ptr, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_i64), _ptr]),
     "as_global_stats_device_ptr": (C.c_int, [_ptr, C.POINTER(_ptr)]),
+    "as_peer_three_call": (C.c_int, [_ptr, _i32]),
     "as_exchange_device_ptr": (C.c_int, [_ptr, C.POINTER(_ptr), C.POINTER(_ptr)]),
     "as_export_state": (C.c_int, [_ptr, C.POINTER(AsMdpState), _ptr]),
     "as_export_stone_poses": (C.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _ptr]),

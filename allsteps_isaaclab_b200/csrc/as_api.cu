@@ -31,6 +31,7 @@ struct AsHandle {
   cudaEvent_t ev_start, ev_stop;  // optional timing hook around k_step<fused>
   PeerArgs peer;        // world > 0 after as_peer_create; buf[] complete after as_peer_connect
   bool peer_connected;
+  bool peer_three_call; // as_peer_three_call: the 3-call path decides promotion, any-reset and histograms over all shards
   volatile uint32_t* peer_host_error;  // mapped pinned host word the exchange kernel sets when a peer timed out
   bool pass1_done;
   bool device_list;     // as_reset took the envs from the list pass 1 compacted on the device (no host round trip)
@@ -305,6 +306,14 @@ int launch_regeneration(AsHandle* h, const ResetArgs& r, cudaStream_t s) {
   return check_launch(h, "k_reset_rows");
 }
 
+// k_peer_exchange behind the kernel just launched (ExchangeMode: what it closes).
+int launch_exchange(AsHandle* h, int mode, cudaStream_t s) {
+  const int cells = (h->params.flags & AS_FLAG_GRID_CURRICULUM) ? static_cast<int>(h->params.grid_bins * h->params.grid_bins) : 0;
+  AS_CUDA(launch_dependent(k_peer_exchange, 1u, 128u, 0, s, h->pdl >= 1, h->ws.ctrl, h->peer, h->num_envs, cells,
+                           h->params, mode));
+  return check_launch(h, "k_peer_exchange");
+}
+
 using StepKernel = void (*)(StepArgs);
 
 // The families of k_step instantiations (process_tile describes FAST, PACKED and PRE).
@@ -475,6 +484,7 @@ int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, i
   h->obs_clip_pass1 = 0.0f;
   std::memset(&h->peer, 0, sizeof(h->peer));
   h->peer_connected = false;
+  h->peer_three_call = false;
   h->peer_host_error = nullptr;
   h->pending_valid = false;
   h->ev_start = h->ev_stop = nullptr;
@@ -565,6 +575,7 @@ int as_step_fused(AsHandle* h, const AsStateIn* in, const float* actions, int64_
   AS_REQUIRE(out->obs_clip >= 0.0f, "obs_clip must be >= 0");
   if (int rc = validate_final_obs(h, out)) return rc;
   if (h->pending_valid) return fail(AS_ERR_STATE, "previous fused step was not closed with as_finish_step");
+  if (h->peer_three_call) return fail(AS_ERR_STATE, "the handle is in the global 3-call mode (as_peer_three_call)");
   if (int rc = check_peer(h)) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   StepArgs a = make_step_args(h, in, actions, actions_stride, out);
@@ -665,6 +676,14 @@ int as_peer_connect(AsHandle* h, const void* ipc_handles_in_rank_order) {
   return AS_OK;
 }
 
+int as_peer_three_call(AsHandle* h, int32_t enable) {
+  AS_REQUIRE(h, "handle is null");
+  if (!h->peer_connected) return fail(AS_ERR_STATE, "as_peer_three_call needs connected peers (as_peer_connect)");
+  if (h->pending_valid || h->spec_valid) return fail(AS_ERR_STATE, "a step is open; switch the mode between steps");
+  h->peer_three_call = enable != 0;
+  return AS_OK;
+}
+
 int as_peer_status(AsHandle* h, int* world, int* rank, int64_t* timeouts, void* stream) {
   AS_REQUIRE(h, "handle is null");
   if (world) *world = h->peer_connected ? h->peer.world : 0;
@@ -706,9 +725,7 @@ int as_finish_step(AsHandle* h, const AsExchange* global_stats, void* stream) {
     a.global_stats = &h->ws.ctrl->gx;  // the step kernel's last CTA exchanged the counters and (normally) closed the step
   } else if (h->peer_connected && global_stats == nullptr) {
     // fold + sum over the shards through NVLink peer memory, in one small kernel under the step kernel's tail
-    const int cells = (h->params.flags & AS_FLAG_GRID_CURRICULUM) ? static_cast<int>(h->params.grid_bins * h->params.grid_bins) : 0;
-    AS_CUDA(launch_dependent(k_peer_exchange, 1u, 128u, 0, s, h->pdl >= 1, h->ws.ctrl, h->peer, h->num_envs, cells));
-    if (int rc = check_launch(h, "k_peer_exchange")) return rc;
+    if (int rc = launch_exchange(h, kExchangeFused, s)) return rc;
     a.global_stats = &h->ws.ctrl->gx;
   }
   const int grid = grid_for(a.num_tiles, 1, h->sm_count, 1);
@@ -730,6 +747,8 @@ int as_step_pass1(AsHandle* h, const AsStateIn* in, const float* actions, int64_
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
   AS_REQUIRE(out->obs_clip >= 0.0f, "obs_clip must be >= 0");
   if (int rc = validate_final_obs(h, out)) return rc;
+  if (h->peer_three_call)
+    if (int rc = check_peer(h)) return rc;
   StepArgs a = make_step_args(h, in, actions, actions_stride, out);
   a.ext_episode_length = episode_length;
   h->obs_clip_pass1 = out->obs_clip;  // as_step_pass2 rewrites the same observation buffer: same epilogue
@@ -742,7 +761,10 @@ int as_step_pass1(AsHandle* h, const AsStateIn* in, const float* actions, int64_
   h->pass1_done = true;   // (its last CTA folds the statistics and advances the Philox step counter)
   h->spec_valid = true;
   h->spec_obs = out->obs;
-  return check_launch(h, "k_step<pass1>");
+  if (int rc = check_launch(h, "k_step<pass1>")) return rc;
+  // global 3-call mode: one exchange per step, right here -- everything the step needs from the other shards is known
+  // (flagged count, sum of the indices), and so are the grid outcomes still pending from the previous step
+  return h->peer_three_call ? launch_exchange(h, kExchangePass1, s) : AS_OK;
 }
 
 int as_reset(AsHandle* h, const float* env_origins, const int32_t* env_ids, int64_t n_ids, int64_t* episode_length,
@@ -759,19 +781,26 @@ int as_reset(AsHandle* h, const float* env_origins, const int32_t* env_ids, int6
     AS_REQUIRE(env_origins && env_ids, "env_origins/env_ids is null");
   }
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
+  if (h->peer_three_call)
+    if (int rc = check_peer(h)) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (!h->pass1_done) {
+  // (global 3-call mode: outside a step means "no pass 1 open" on every rank alike, whichever shard reset envs before)
+  if (h->peer_three_call ? !h->spec_valid : !h->pass1_done) {
     // `_reset_idx` outside a step (DirectRLEnv.reset(), DRL:256-279): the promotion rule of ENV:471 looks at the
     // indices as they are now, and the draws must not repeat those of an earlier reset -- sum the indices and
     // advance the Philox step counter, which as_step_pass1 would have done
     k_prepare_reset<<<1, 1024, 0, s>>>(h->ws, h->num_envs);
     if (int rc = check_launch(h, "k_prepare_reset")) return rc;
+    // global 3-call mode: the promotion on the global sum of the indices, pending grid outcomes into the histograms
+    if (h->peer_three_call)
+      if (int rc = launch_exchange(h, kExchangeReset, s)) return rc;
   }
   h->pass1_done = false;  // consumed: a second reset without a pass in between prepares for itself
   ResetArgs r = make_reset_args(h, env_origins);
   // (an explicit id list means `_reset_idx` was entered, i.e. some env reset; with the device-side list that is
   // decided by the count pass 1 folded -- the rule is not evaluated in a step in which nothing resets, DRL:360)
   r.force_any_reset = from_device_list ? 0 : 1;
+  r.peer_decided = h->peer_three_call ? 1 : 0;
   if (compact_out) r.out = *compact_out;
   r.env_ids = from_device_list ? h->ws.reset_ids : env_ids;
   r.n_ids = from_device_list ? -1 : n_ids;
@@ -801,6 +830,8 @@ int as_step_pass2(AsHandle* h, const AsStateIn* in, float* obs, void* stream) {
   // (no call-order precondition: the reference runs `_compute_useful_values` at the end of `_reset_idx` whether or
   // not a pass preceded it -- DirectRLEnv.reset() calls `_reset_idx(all ids)` before the first step, DRL:256-279)
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
+  if (h->peer_three_call)
+    if (int rc = check_peer(h)) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (h->spec_valid) {
     // pass 1 already ran pass 2 for every env that did not reset: redo the envs that did (from the views as they are
@@ -816,6 +847,7 @@ int as_step_pass2(AsHandle* h, const AsStateIn* in, float* obs, void* stream) {
     c.inv_step_dt = h->inv_step_dt;
     c.num_envs = h->num_envs;
     c.revert_if_none = h->device_list ? 1 : 0;
+    c.peer_three_call = h->peer_three_call ? 1 : 0;
     const int grid = grid_for(h->num_envs / 10 + 1, 32, h->sm_count, 3);
     k_pass2_commit<<<grid, 256, 0, s>>>(c);
     h->spec_valid = false;
@@ -835,9 +867,11 @@ int as_step_pass2(AsHandle* h, const AsStateIn* in, float* obs, void* stream) {
 int as_step_no_reset(AsHandle* h, void* stream) {
   AS_REQUIRE(h, "handle is null");
   if (!h->spec_valid) return AS_OK;  // nothing was speculated (no pass 1 since the last pass 2)
+  if (h->peer_three_call)
+    if (int rc = check_peer(h)) return rc;
   const int grid = grid_for(h->num_envs * 11, 256 * 4, h->sm_count, 8);
   k_pass2_revert<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(h->ws, h->spec_obs, h->obs_clip_pass1,
-                                                                        h->num_envs);
+                                                                        h->num_envs, h->peer_three_call ? 1 : 0);
   h->spec_valid = false;
   return check_launch(h, "k_pass2_revert");
 }

@@ -162,10 +162,10 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
   const unsigned long long step = ctrl->step_counter;
   // fused: the step kernel already wrote the start-pose rows; n_ids < 0: the list pass 1 compacted on the device
   const int64_t n_reset = a.fused ? 0 : (a.n_ids < 0 ? static_cast<int64_t>(ctrl->n_reset_list) : a.n_ids);
-  if (!a.fused && blockIdx.x == 0 && threadIdx.x == 0) {
+  if (!a.fused && !a.peer_decided && blockIdx.x == 0 && threadIdx.x == 0) {
     // 3-call path: `_reset_idx` opens with the promotion rule (ENV:471-479) on the statistics pass 1 folded.  The
     // decision is in force from here on: k_reset_rows regenerates at the promoted level (ENV:471 precedes ENV:500),
-    // the next pass 1 applies it to the state words
+    // the next pass 1 applies it to the state words.  (Global 3-call mode: k_peer_exchange decided it on the sums.)
     AsStats s = ctrl->stats;
     if (a.force_any_reset) s.n_reset = s.n_reset > 0 ? s.n_reset : 1;
     ctrl->promote_cur = promotion_decision(P, s);
@@ -260,8 +260,9 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
 // ------------------------------------------------------------------------------------------------ kernels (b) + (c)
 // Everything that happens to the envs listed for regeneration, in ONE launch: behind the fused step the step kernel
 // listed them (fused = 1), on the 3-call path k_reset_list did (fused = 0; there the draws are at the step counter
-// pass 1 or k_prepare_reset advanced to, the outcomes join the histograms when k_pass2_commit closes the step, and a
-// reset outside a step -- into_other = 0 -- records none).
+// pass 1 or k_prepare_reset advanced to, the outcomes join the histograms when k_pass2_commit closes the step -- in
+// the global 3-call mode when the next k_peer_exchange has summed them over the shards -- and a reset outside a step
+// -- into_other = 0 -- records none).
 //   (c) grid-curriculum extension (no reference counterpart; specification = oracle/grid_curriculum.py): the outcome of
 //       the episode that just ended is recorded against the bin the env WAS playing -- a shared-memory histogram per
 //       CTA, flushed with one atomic per touched bin into the step's outcome record (Ctrl::grid_delta_*), which joins
@@ -735,6 +736,8 @@ struct CommitArgs {
   int64_t num_envs;
   int32_t revert_if_none;  // device-side reset list: whether any env reset is only known here -- none did: behave as
                            // k_pass2_revert (DRL:360 would have skipped `_reset_idx`)
+  int32_t peer_three_call; // global 3-call mode: "none did" means none on ANY shard (Ctrl::any_reset), and this step's
+                           // grid outcomes stay in Ctrl::grid_delta_* for the next k_peer_exchange to sum and add
 };
 
 __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ CommitArgs a) {
@@ -745,7 +748,7 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
   const int64_t warp = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
   const int64_t n = ctrl->n_reset_list;
-  if (n == 0 && a.revert_if_none) {
+  if (n == 0 && a.revert_if_none && !(a.peer_three_call && ctrl->any_reset)) {
     if (blockIdx.x == 0 && threadIdx.x == 0) ctrl->stats.n_advanced -= ctrl->last_adv2;  // pass 2 is discarded
     const int64_t total = a.num_envs * 11;
     for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
@@ -834,7 +837,7 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
     s_last = atomicAdd(&ctrl->blocks_done2, 1u) == gridDim.x - 1 ? 1u : 0u;
   }
   __syncthreads();
-  if (s_last && (P.flags & AS_FLAG_GRID_CURRICULUM)) {
+  if (s_last && (P.flags & AS_FLAG_GRID_CURRICULUM) && !a.peer_three_call) {
     // this step's episode outcomes (k_reset_rows) join the difficulty-grid histograms of this shard, as the fused
     // step's finish does
     for (int i = threadIdx.x; i < kMaxGridBins; i += blockDim.x) {
@@ -850,9 +853,12 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
   }
 }
 
+// peer_three_call: global 3-call mode.  When an env of another shard reset, the reference runs pass 2 for every env
+// (DRL:359-360 and ENV:567 look at all envs): keep what pass 1 speculated -- observations, state buffer, advances.
 __global__ void __launch_bounds__(256) k_pass2_revert(Workspace ws, float* __restrict__ obs, float obs_clip,
-                                                      int64_t num_envs) {
-  const int64_t total = num_envs * 11;
+                                                      int64_t num_envs, int32_t peer_three_call) {
+  const bool commit = peer_three_call && ws.ctrl->any_reset;
+  const int64_t total = commit ? 0 : num_envs * 11;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int64_t e = i / 11;
@@ -861,7 +867,8 @@ __global__ void __launch_bounds__(256) k_pass2_revert(Workspace ws, float* __res
   }
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     ws.ctrl->n_reset_list = 0;
-    ws.ctrl->stats.n_advanced -= ws.ctrl->last_adv2;  // the pass-2 advances pass 1 counted are discarded with pass 2
+    if (commit) ws.ctrl->parity ^= 1u;  // the speculated buffer becomes the current state
+    else ws.ctrl->stats.n_advanced -= ws.ctrl->last_adv2;  // the pass-2 advances pass 1 counted are discarded with pass 2
   }
 }
 
@@ -888,8 +895,9 @@ __global__ void __launch_bounds__(1024) k_prepare_reset(Workspace ws, int64_t nu
 }
 
 // as_restore: the fields of a saved control block that are MDP state (parity of the state buffers, pending promotion,
-// Philox step counter, folded statistics, difficulty-grid histograms).  Live bookkeeping stays: the peer-exchange
-// epoch (the peers' slots hold flags of the live epoch), diagnostics counters.
+// Philox step counter, folded statistics, difficulty-grid histograms and the grid outcomes the global 3-call mode keeps
+// pending between steps -- zero between steps in every other mode).  Live bookkeeping stays: the peer-exchange epoch
+// (the peers' slots hold flags of the live epoch), diagnostics counters.
 __global__ void k_restore_ctrl(Ctrl* ctrl, const Ctrl* saved) {
   const int t = threadIdx.x;
   if (t == 0) {
@@ -906,6 +914,8 @@ __global__ void k_restore_ctrl(Ctrl* ctrl, const Ctrl* saved) {
   for (int i = t; i < kMaxGridBins; i += blockDim.x) {
     ctrl->grid_attempts[i] = saved->grid_attempts[i];
     ctrl->grid_successes[i] = saved->grid_successes[i];
+    ctrl->grid_delta_att[i] = saved->grid_delta_att[i];
+    ctrl->grid_delta_succ[i] = saved->grid_delta_succ[i];
   }
   for (int i = t; i < kSlots * kNumCounters; i += blockDim.x) (&ctrl->slots[0][0])[i] = 0u;
   for (int i = t; i < kSlots; i += blockDim.x) ctrl->slot_reward[i] = 0.0f;

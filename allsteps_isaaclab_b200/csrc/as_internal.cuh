@@ -92,7 +92,11 @@ struct Ctrl {
   uint32_t peer_error;                        // != 0: a peer exchange timed out; the shards may have diverged (AS_ERR_PEER)
   uint32_t step_state;                        // written by the LAST CTA of every fused step kernel: 2 = it closed the step itself
                                               // (statistics folded, promotion decided, parity flipped), 1 = k_fixup_finish has to
+  uint32_t any_reset;                         // global 3-call mode: pass 1 flagged an env on some shard this step (written by
+                                              // k_peer_exchange; read by k_pass2_commit / k_pass2_revert, DRL:359-360)
 };
+// (the control block's slot in the workspace and the snapshot stays 8448 bytes: checkpoints keep their layout)
+static_assert(sizeof(Ctrl) <= 8448, "Ctrl must fit its 8448-byte workspace slot");
 
 static_assert(offsetof(Ctrl, grid_delta_att) == offsetof(Ctrl, stats) + sizeof(AsStats) &&
                   offsetof(Ctrl, grid_delta_succ) == offsetof(Ctrl, grid_delta_att) + sizeof(unsigned int) * kMaxGridBins,
@@ -241,6 +245,7 @@ struct ResetArgs {
   int32_t fused;                // 1: state words were already reset by the step kernel, rows go to env's own row
   int32_t into_other;           // 3-call path behind a speculating pass 1: the reset state words go into the OTHER buffer
   int32_t force_any_reset;      // 3-call path: an explicit id list means `_reset_idx` was entered, i.e. some env reset
+  int32_t peer_decided;         // global 3-call mode: k_peer_exchange already decided the promotion on the global sums
 };
 
 }  // namespace as

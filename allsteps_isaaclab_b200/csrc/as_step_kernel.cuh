@@ -1620,21 +1620,34 @@ __global__ void __launch_bounds__(128) k_fold_early(Ctrl* ctrl, int64_t num_envs
   if (threadIdx.x == 0) ctrl->stats_folded = 1;
 }
 
+// What a k_peer_exchange launch closes.
+enum ExchangeMode {
+  kExchangeFused = 0,  // behind k_step<fused>: fold this step's counters first; k_fixup_finish closes on the sums
+  kExchangePass1 = 1,  // global 3-call mode, behind k_step<pass1> (whose last CTA folded already)
+  kExchangeReset = 2,  // global 3-call mode, behind k_prepare_reset: `_reset_idx` outside a step, entered on every rank
+};
+
 // Fold + cross-shard sum in one kernel over NVLink peer memory (replaces k_fold_early + NCCL all-reduce of 80 bytes).
 // One CTA.  Lane r of warp 0 talks to rank r: it stores this shard's ten counters into OUR slot of rank r's buffer,
 // fences, then stores the epoch as the flag; it then polls rank r's slot in OUR buffer for the same epoch and reads
 // the counters.  Two slots per sender (epoch parity): a rank can run at most one step ahead of a peer that has not
 // yet read, because it cannot close step t+1 without that peer's step-t+1 counters.
+// In the global 3-call modes the exchange also decides what needs all shards before `_reset_idx` runs: the promotion
+// of ENV:471 on the global sums, "did any env reset" (DRL:359-360), and it adds the grid outcomes still pending from
+// the previous step (summed over the shards) to the histograms, before anything draws from them.
 __global__ void __launch_bounds__(128) k_peer_exchange(Ctrl* ctrl, const __grid_constant__ PeerArgs peer,
-                                                       int64_t num_envs, int grid_cells) {
+                                                       int64_t num_envs, int grid_cells,
+                                                       const __grid_constant__ AsParams P, int mode) {
   __shared__ unsigned int fold[kNumCounters];
   __shared__ unsigned int s_timeouts;
   asm volatile("griddepcontrol.launch_dependents;");  // the finish kernel may become resident; it waits for us
   asm volatile("griddepcontrol.wait;" ::: "memory");  // the step kernel has completed and flushed
-  fold_stats(ctrl, fold, num_envs);
   const int tid = threadIdx.x;
-  if (tid == 0) ctrl->stats_folded = 1;
-  __syncthreads();
+  if (mode == kExchangeFused) {
+    fold_stats(ctrl, fold, num_envs);
+    if (tid == 0) ctrl->stats_folded = 1;
+    __syncthreads();
+  }
   const unsigned long long epoch = static_cast<unsigned long long>(ctrl->peer_epoch) + 1ull;
   const int par = static_cast<int>(epoch & 1ull);
   auto grid_slot = [&](int owner, int sender) {
@@ -1684,7 +1697,17 @@ __global__ void __launch_bounds__(128) k_peer_exchange(Ctrl* ctrl, const __grid_
       }
       ctrl->gx.grid_attempts[i] = att;
       ctrl->gx.grid_successes[i] = succ;
+      if (mode != kExchangeFused && i < grid_cells) {  // the previous step's outcomes of all shards join the histograms
+        grid_fold(ctrl->grid_attempts[i], ctrl->grid_successes[i], att, succ);
+        ctrl->grid_delta_att[i] = ctrl->grid_delta_succ[i] = 0u;
+      }
     }
+  }
+  if (mode != kExchangeFused && tid == 0) {
+    AsStats g = ctrl->gx.stats;  // (this shard's own record if a peer timed out)
+    if (mode == kExchangeReset) g.n_reset = 1;
+    ctrl->promote_cur = promotion_decision(P, g);  // in force from here on; k_reset_list does not decide again
+    ctrl->any_reset = g.n_reset > 0 ? 1u : 0u;
   }
 }
 

@@ -60,17 +60,28 @@ class AllstepsHooksB200:
     """Hook methods of `AllstepsEnv(DirectRLEnv)` (ENV:34) backed by `AllstepsMDP`."""
 
     def _init_allsteps_b200(self, task_cfg: Optional[AllstepsCfg] = None, seed: int = 0, final_obs: bool = False,
-                            **mdp_kwargs):
+                            distributed: bool = False, **mdp_kwargs):
         """Call at the end of `__init__` (replaces ENV:40-102).
 
         final_obs: publish `extras["final_obs"]` (N,59) every step: for the envs that reset in the step (`reset_buf`),
         the observation of the state their episode ended in -- `obs` holds their start pose -- so that a time-out can
-        be bootstrapped with `gamma * V(final_obs)`.  Rows of the other envs hold whatever an earlier step left there."""
+        be bootstrapped with `gamma * V(final_obs)`.  Rows of the other envs hold whatever an earlier step left there.
+
+        distributed: one process per GPU under torch.distributed (torchrun), this env holding one shard of the run's
+        envs.  The shard's global env ids follow the other ranks' (so draws do not depend on the number of GPUs) and
+        the handle runs in the global 3-call mode: promotion, "did any env reset" and the grid histograms over all
+        shards, bit-identical to one env holding all of them (`AllstepsMDP.connect_peers(three_call=True)`)."""
         self.task_cfg = task_cfg or AllstepsCfg()
         dev = torch.device(self.device)
         body_rows, joint_limits = resolve_robot_tables(self.robot, self.task_cfg)
+        if distributed:
+            from .sharding import global_env_offset
+
+            mdp_kwargs["env_id_offset"] = global_env_offset(self.num_envs, dev)
         self.mdp = AllstepsMDP(self.num_envs, device=dev, cfg=self.task_cfg, seed=seed, joint_limits=joint_limits,
                                **mdp_kwargs)
+        if distributed:
+            self.mdp.connect_peers(three_call=True)
         self.buf = StepBuffers(self.num_envs, dev, reward_terms=True, final_obs=final_obs)
         self.foot_indices = [body_rows[0], body_rows[1]]  # ENV:87
         self.torso_index = body_rows[2]  # ENV:88

@@ -279,12 +279,17 @@ class AllstepsMDP:
         return CapturedStep(self, views, actions, out, global_stats)
 
     # ------------------------------------------------------------------ cross-shard promotion over NVLink peer memory
-    def connect_peers(self, group=None):
+    def connect_peers(self, group=None, three_call: bool = False):
         """One process per GPU, every rank owning one env-id shard: after this call `step()` / `finish_step()` decide
         the promotion rule (ENV:471) and the "did any env reset" test (DRL:359) on the sum over ALL shards.  The sum is
         formed by one small kernel that stores this shard's ten step counters into every peer's exchange buffer
         through NVLink and reads theirs -- no NCCL call on the step path.  torch.distributed is used once, here, to
-        hand round the 64-byte CUDA IPC handles.  Every rank must step in lockstep from now on."""
+        hand round the 64-byte CUDA IPC handles.  Every rank must step in lockstep from now on.
+
+        three_call: the same for the 3-call path (`pass1` / `reset` / `pass2` / `no_reset`, what the Isaac Lab faces
+        drive) instead of `step()`: promotion, "did any env reset" and the grid histograms over all shards, one exchange
+        per `pass1`.  Every rank must make the same sequence of `pass1` calls and resets outside a step;
+        `grid_state()` lags one step behind a single handle between steps (see `set_peer_three_call`)."""
         import torch.distributed as dist
 
         world, rank = dist.get_world_size(group), dist.get_rank(group)
@@ -298,16 +303,27 @@ class AllstepsMDP:
             blob = b"".join(bytes(g.cpu().tolist()) for g in gathered)
             _cabi.check(self.lib.as_peer_connect(self.handle, blob), "as_peer_connect")
         self._bind_global_stats()
+        if three_call:
+            self.set_peer_three_call(True)
         dist.barrier(group)  # nobody steps before every mapping exists
         return world, rank
 
-    def connect_self(self):
+    def connect_self(self, three_call: bool = False):
         """World of one (tests, single-GPU runs of a sharded script): the exchange kernel talks to itself."""
         mine = (C.c_ubyte * _cabi.PEER_HANDLE_BYTES)()
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.as_peer_create(self.handle, 1, 0, mine), "as_peer_create")
             _cabi.check(self.lib.as_peer_connect(self.handle, bytes(mine)), "as_peer_connect")
         self._bind_global_stats()
+        if three_call:
+            self.set_peer_three_call(True)
+
+    def set_peer_three_call(self, enable: bool):
+        """Global 3-call mode on connected peers (`as_peer_three_call`), switched between steps.  In it `step()` is
+        refused, and this step's grid outcomes join the histograms -- summed over the shards -- at the exchange of
+        the next `pass1`: between steps `grid_state()` / `grid_hist_tensor` lag one step behind one handle holding all
+        envs, right after each `pass1` they are equal."""
+        _cabi.check(self.lib.as_peer_three_call(self.handle, 1 if enable else 0), "as_peer_three_call")
 
     def _bind_global_stats(self):
         ptr = C.c_void_p()

@@ -29,6 +29,18 @@ def shard_range(global_envs: int, rank: int, world: int, align: int = SHARD_ALIG
     return start, stop
 
 
+def global_env_offset(num_envs: int, device, group=None) -> int:
+    """This rank's first global env id: the exclusive prefix sum of every rank's `num_envs` (one all_gather; on the
+    GPU for NCCL, on the host for gloo).  Shards may differ in size; ids follow rank order."""
+    import torch.distributed as dist
+
+    dev = torch.device(device) if dist.get_backend(group) == "nccl" else torch.device("cpu")
+    mine = torch.tensor([int(num_envs)], dtype=torch.int64, device=dev)
+    every = [torch.empty_like(mine) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(every, mine, group=group)
+    return int(sum(int(t.item()) for t in every[:dist.get_rank(group)]))
+
+
 def all_reduce_exchange(buf: torch.Tensor, with_grid: bool, group=None) -> torch.Tensor:
     """Sum an `AsExchange` record (int64 view: `AllstepsMDP.exchange_tensor` copied after `fold_stats()`) over the ranks
     where it is additive: the ten leading step counters and -- `with_grid` -- the step's difficulty-grid outcomes (two

@@ -55,18 +55,28 @@ class _Binding:
     """Per-env glue shared by all terms: the MDP object, the output buffers and the per-step cache."""
 
     def __init__(self, env, robot="robot", left="foot_contacts_left", right="foot_contacts_right", seed=0,
-                 task_cfg: Optional[AllstepsCfg] = None, grid_bins: int = 0, intended_regen: bool = False):
+                 task_cfg: Optional[AllstepsCfg] = None, grid_bins: int = 0, intended_regen: bool = False,
+                 distributed: bool = False):
         """grid_bins / intended_regen: the `AllstepsMDP` extensions (difficulty-grid curriculum with grid_bins per
         axis; regeneration of the stones of envs that had passed half of them).  Both regenerate stones in
-        `reset_allsteps`, which then writes them to the scene's stone collection."""
+        `reset_allsteps`, which then writes them to the scene's stone collection.  distributed: this env is one
+        rank's shard of a torchrun job -- global env ids after the other ranks' and the global 3-call mode (see
+        `AllstepsHooksB200._init_allsteps_b200`)."""
         from .env import resolve_robot_tables
 
         self.cfg = task_cfg or AllstepsCfg()
         self.names = (robot, left, right)
         dev = torch.device(env.device)
         self.body_rows, joint_limits = resolve_robot_tables(env.scene[robot], self.cfg)
+        offset = 0
+        if distributed:
+            from .sharding import global_env_offset
+
+            offset = global_env_offset(env.num_envs, dev)
         self.mdp = AllstepsMDP(env.num_envs, device=dev, cfg=self.cfg, seed=seed, joint_limits=joint_limits,
-                               grid_bins=grid_bins, intended_regen=intended_regen)
+                               grid_bins=grid_bins, intended_regen=intended_regen, env_id_offset=offset)
+        if distributed:
+            self.mdp.connect_peers(three_call=True)
         self.buf = StepBuffers(env.num_envs, dev, reward_terms=True)
         self.buf.obs.zero_()
         self.buf.reward.zero_()

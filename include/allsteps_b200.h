@@ -291,6 +291,19 @@ int as_peer_create(AsHandle* h, int world, int rank, void* ipc_handle_out);
 int as_peer_connect(AsHandle* h, const void* ipc_handles_in_rank_order);
 int as_peer_status(AsHandle* h, int* world, int* rank, int64_t* timeouts, void* stream); /* synchronises `stream` */
 int as_global_stats_device_ptr(AsHandle* h, AsStats** device_stats);
+/* Global 3-call mode (enable != 0; 0 switches it off again, between steps).  Valid after as_peer_connect, otherwise
+ * AS_ERR_STATE; also AS_ERR_STATE while a step is open.  With it, a sharded run through the 3-call path (as_step_pass1
+ * -> as_reset -> as_step_pass2 / as_step_no_reset) is bit-identical to one handle holding all envs: outputs, state,
+ * levels, grid bins and stones.  as_step_pass1 launches one exchange behind pass 1 that sums the flagged count and the
+ * indices over the shards and there decides the promotion of ENV:471 and "did any env reset" (DRL:359-360): when an env
+ * of ANY shard reset, as_step_no_reset -- and as_step_pass2 on an empty device-side list -- keep pass 2 for every env
+ * of this shard, as the reference does, instead of taking it back; as_reset uses the exchanged promotion.  A reset
+ * outside a step (no as_step_pass1 open) exchanges too, right before it resets.  So every rank must make the same
+ * sequence of as_step_pass1 / reset-outside-a-step calls (a reset outside a step with a non-empty id list); a rank that
+ * does not meets the sticky AS_ERR_PEER of the exchange's time limit, not a hang.  Grid histograms: see as_grid_state.
+ * Resets the caller adds that pass 1 did not flag (extra termination terms) reset correctly on their own shard but do
+ * not count toward the global any-reset and promotion tests.  as_step_fused on a handle in this mode: AS_ERR_STATE. */
+int as_peer_three_call(AsHandle* h, int32_t enable);
 
 /* ---- action path: ENV:257-274 `_pre_physics_step` + `_apply_action` --------------------------------------
  * efforts[n,j] = applied_gain[level[n]] * joint_gears[j] * clamp(actions[n,j], -1, 1)
@@ -334,7 +347,7 @@ int as_import_state(AsHandle* h, const AsMdpState* src, void* stream);
 
 /* ---- exact checkpoint / resume (SURVEY section 5) -----------------------------------------------------------
  * A snapshot is one opaque device blob: control block (state parity, pending promotion, Philox step counter, folded
- * statistics, difficulty-grid histograms), the packed state words, the stone windows, the grid bins and -- with
+ * statistics, difficulty-grid histograms and the grid outcomes the global 3-call mode keeps pending), the packed state words, the stone windows, the grid bins and -- with
  * include_stones -- the stone rows (needed whenever stones can change: regeneration extensions, or a restore into a
  * fresh handle).  as_restore puts it back; a run continued from a restored snapshot is bit-identical to the
  * uninterrupted one (same seed / env_id_offset / num_envs).  Stream-ordered, no synchronisation. */
@@ -366,7 +379,11 @@ int as_export_stone_poses(AsHandle* h, const int32_t* env_ids, int64_t n_ids, fl
  * Bins drawn in step t use the histograms as they stand after step t-1; the outcomes of step t are added when the step
  * is closed: by as_finish_step -- summed over all shards when the step is closed on a global record, so that sharded
  * runs sample from the same CDF as one handle holding all envs -- or, on the 3-call path, by as_step_pass2.  On the
- * 3-call path the histograms are shard-local (as its promotion rule is): each shard samples from its own outcomes.
+ * 3-call path the histograms are shard-local (as its promotion rule is): each shard samples from its own outcomes --
+ * unless the handle is in the global 3-call mode (as_peer_three_call).  There as_step_pass2 leaves the step's outcomes
+ * pending, and the exchange of the NEXT as_step_pass1 (or reset outside a step) adds them, summed over all shards,
+ * before anything draws from the histograms.  So between steps the histograms as_grid_state copies out lag one step
+ * behind those of one handle holding all envs; right after each as_step_pass1 they are equal.
  * The draws of as_reset are made at the step counter as_step_pass1 advanced to, so bins and stones differ from those
  * of a fused step on the same inputs.  A step in which nothing resets (as_step_no_reset, or an empty device-side list)
  * records nothing.  A reset outside a step (as_reset with no as_step_pass1 before it: DirectRLEnv.reset()) ends no
