@@ -10,14 +10,16 @@ import ctypes as C
 import os
 
 NUM_JOINTS = 21
-NUM_STONES = 20
+NUM_STONES = 20  # AS_NUM_STONES: the default course length (AsParams.num_steps = 0)
+MIN_STONES = 3   # AS_MIN_STONES
+MAX_STONES = 32  # AS_MAX_STONES
 OBS_DIM = 59
 NUM_LEVELS = 10
 ROOT_STATE_DIM = 13
 NUM_REWARD_TERMS = 10
 PEER_HANDLE_BYTES = 64  # AS_PEER_HANDLE_BYTES (sizeof(cudaIpcMemHandle_t))
 TILE_ENVS = 128
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 FLAG_INTENDED_REGEN = 1 << 0
 FLAG_SKIP_PASS2 = 1 << 1
@@ -46,7 +48,8 @@ class AsParams(C.Structure):
         ("clip_lower", _f), ("clip_upper", _f), ("default_root_pos", _f * 3),
         ("joint_lower", _f * NUM_JOINTS), ("joint_upper", _f * NUM_JOINTS), ("joint_gears", _f * NUM_JOINTS),
         ("reset_pose", _f * NUM_JOINTS), ("mirror_src", _i32 * NUM_JOINTS), ("mirror_sign", _f * NUM_JOINTS),
-        ("missed_step_height", _f), ("flags", C.c_uint32), ("grid_bins", C.c_uint32), ("seed", C.c_uint64),
+        ("missed_step_height", _f), ("flags", C.c_uint32), ("grid_bins", C.c_uint32), ("num_steps", C.c_uint32),
+        ("seed", C.c_uint64),
     ]
 
 
@@ -119,6 +122,7 @@ SIGNATURES = {
     "as_abi_version": (C.c_int, []),
     "as_last_error": (C.c_char_p, []),
     "as_workspace_bytes": (_i64, [_i64]),
+    "as_workspace_bytes_for": (_i64, [C.POINTER(AsParams), _i64]),
     "as_create": (C.c_int, [C.POINTER(AsParams), _i64, _i64, C.c_int, _ptr, _i64, _ptr, C.POINTER(_ptr)]),
     "as_destroy": (None, [_ptr]),
     "as_generate_stones": (C.c_int, [_ptr, _ptr, _ptr, _i64, _ptr, _ptr]),

@@ -82,6 +82,13 @@ int check_peer(const AsHandle* h) {
 
 int num_tiles(int64_t n) { return static_cast<int>((n + kTile - 1) / kTile); }
 
+// AsParams.num_steps as the kernels take it: 0 means the default course length; -1 when out of range
+int course_length(const AsParams& P) {
+  const int S = P.num_steps == 0 ? kS : static_cast<int>(P.num_steps);
+  return P.num_steps <= AS_MAX_STONES && S >= AS_MIN_STONES ? S : -1;
+}
+int handle_stones(const AsHandle* h) { return static_cast<int>(h->params.num_steps); }
+
 constexpr int64_t kRegenByWarpMaxEnvs = 1 << 15;  // k_reset_rows: a warp per env up to this batch size (profiles/r02_experiments.txt, 12)
 // From this batch size on the scattered reads of a step go to k_prepare*.  Below it the step is launch-latency bound
 // (working set in L2, a handful of CTAs per SM): one launch fewer beats the better latency hiding of the separate gather
@@ -114,6 +121,7 @@ int launch_prepare(AsHandle* h, const AsStateIn* in, cudaStream_t s, bool gather
   p.lean = contact_in_host_memory(h, in) ? 1 : 0;
   p.stop_frames = h->params.stop_frames;
   p.contact_epsilon = h->params.contact_epsilon;
+  p.num_stones = handle_stones(h);
   const bool aligned = ((reinterpret_cast<uintptr_t>(in->contact_right) | reinterpret_cast<uintptr_t>(in->contact_left)) &
                         15u) == 0 && ((in->contact_right_stride | in->contact_left_stride) & 3) == 0;
   if (aligned) {  // two lanes per env: one memory request per force vector
@@ -138,7 +146,7 @@ int validate_final_obs(const AsHandle* h, const AsStepOut* out) {
   return AS_OK;
 }
 
-int validate_state_in(const AsStateIn* in, bool need_origins) {
+int validate_state_in(const AsHandle* h, const AsStateIn* in, bool need_origins) {
   AS_REQUIRE(in != nullptr, "AsStateIn is null");
   AS_REQUIRE(in->root_pos && in->root_quat && in->root_lin_vel, "root state pointers must be set");
   AS_REQUIRE(in->body_pos, "body_pos must be set");
@@ -147,7 +155,8 @@ int validate_state_in(const AsStateIn* in, bool need_origins) {
   AS_REQUIRE(in->root_pos_stride >= 3 && in->root_quat_stride >= 4 && in->root_lin_vel_stride >= 3,
              "root strides too small");
   AS_REQUIRE(in->joint_pos_stride >= kJ && in->joint_vel_stride >= kJ, "joint strides too small");
-  AS_REQUIRE(in->contact_right_stride >= kS * 3 && in->contact_left_stride >= kS * 3, "contact strides too small");
+  const int S = handle_stones(h);
+  AS_REQUIRE(in->contact_right_stride >= S * 3 && in->contact_left_stride >= S * 3, "contact strides too small");
   AS_REQUIRE(in->body_row_stride >= 3 && in->body_env_stride >= 3, "body strides too small");
   AS_REQUIRE(in->right_foot_row >= 0 && in->left_foot_row >= 0 && in->torso_row >= 0, "negative body row");
   if (need_origins) AS_REQUIRE(in->env_origins != nullptr, "env_origins must be set for the fused step");
@@ -300,9 +309,11 @@ cudaError_t launch_dependent(void (*kernel)(KArgs...), unsigned grid, unsigned b
 // (ALLSTEPS_REGEN_MODE: 1 / 2).
 int launch_regeneration(AsHandle* h, const ResetArgs& r, cudaStream_t s) {
   const bool by_warp = h->regen_mode == 1 || (h->regen_mode == 0 && h->num_envs <= kRegenByWarpMaxEnvs);
+  const bool default_s = handle_stones(h) == kS;
   const int grid_ctas = grid_for(h->num_envs, 64, h->sm_count, 8);
-  AS_CUDA(launch_dependent(by_warp ? k_reset_rows<true> : k_reset_rows<false>, static_cast<unsigned>(grid_ctas), 256u,
-                           0, s, h->pdl >= 1, r));
+  AS_CUDA(launch_dependent(by_warp ? (default_s ? k_reset_rows<true, true> : k_reset_rows<true, false>)
+                                   : (default_s ? k_reset_rows<false, true> : k_reset_rows<false, false>),
+                           static_cast<unsigned>(grid_ctas), 256u, 0, s, h->pdl >= 1, r));
   return check_launch(h, "k_reset_rows");
 }
 
@@ -389,7 +400,8 @@ StepLaunch select_step(AsHandle* h, int mode, const AsStateIn* in, StepArgs& a) 
   // events of a fused step, which time the step kernel alone.
   a.pdl_wait = (hot && h->pdl >= 2 && a.use_pre && !(mode == kModeFused && h->ev_start)) ? 1 : 0;
   // the common launch shape has its own instantiation (process_tile: FAST)
-  const bool fast = !a.in.quat_xyzw && !a.out.reward_terms && a.out.obs_clip == 0.0f && !a.out.final_obs;
+  const bool fast = !a.in.quat_xyzw && !a.out.reward_terms && a.out.obs_clip == 0.0f && !a.out.final_obs &&
+                    handle_stones(h) == kS;
   // root pos / quat / lin vel handed over as slices of one (N,13) root_state_w tensor (Isaac Lab's own layout): the
   // full tiles take the whole rows with one bulk copy (process_tile: PACKED)
   const bool packed = in->root_pos_stride == AS_ROOT_STATE_DIM && in->root_quat_stride == AS_ROOT_STATE_DIM &&
@@ -433,7 +445,12 @@ const char* as_last_error(void) { return g_error.c_str(); }
 
 int64_t as_workspace_bytes(int64_t num_envs) {
   if (num_envs <= 0) return 0;
-  return workspace_layout(num_envs).total;
+  return workspace_layout(num_envs, kS).total;
+}
+
+int64_t as_workspace_bytes_for(const AsParams* params, int64_t num_envs) {
+  if (!params || num_envs <= 0 || course_length(*params) < 0) return 0;
+  return workspace_layout(num_envs, course_length(*params)).total;
 }
 
 int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, int device, void* workspace,
@@ -446,14 +463,16 @@ int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, i
   AS_REQUIRE(params->max_episode_length > 1 && params->max_episode_length < kMaxEpisodeLength,
              "max_episode_length out of range");
   AS_REQUIRE(params->step_dt > 0.0f, "step_dt must be positive");
+  const int S = course_length(*params);
+  AS_REQUIRE(S > 0, "num_steps must be 0 (default) or in 3..32");
   if (params->flags & AS_FLAG_GRID_CURRICULUM)
     AS_REQUIRE(params->grid_bins >= 2 && params->grid_bins <= 16, "grid_bins must be in 2..16");
   for (int j = 0; j < kJ; ++j) {
     AS_REQUIRE(params->joint_upper[j] > params->joint_lower[j], "joint limits must satisfy lower < upper");
     AS_REQUIRE(params->mirror_src[j] >= 0 && params->mirror_src[j] < kJ, "mirror_src out of range");
   }
-  const WorkspaceLayout l = workspace_layout(num_envs);
-  AS_REQUIRE(workspace != nullptr && workspace_bytes >= l.total, "workspace too small (see as_workspace_bytes)");
+  const WorkspaceLayout l = workspace_layout(num_envs, S);
+  AS_REQUIRE(workspace != nullptr && workspace_bytes >= l.total, "workspace too small (see as_workspace_bytes_for)");
   AS_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "workspace must be 256-byte aligned");
   AS_CUDA(cudaSetDevice(device));
   cudaDeviceProp prop;
@@ -470,6 +489,7 @@ int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, i
   AsHandle* h = new (std::nothrow) AsHandle();
   AS_REQUIRE(h != nullptr, "out of host memory");
   h->params = *params;
+  h->params.num_steps = static_cast<uint32_t>(S);  // (the kernels read the course length from here)
   h->num_envs = num_envs;
   h->env_id_offset = env_id_offset;
   h->device = device;
@@ -569,7 +589,7 @@ int as_generate_stones(AsHandle* h, const float* env_origins, const int32_t* env
 int as_step_fused(AsHandle* h, const AsStateIn* in, const float* actions, int64_t actions_stride,
                   const AsStepOut* out, const AsResetOut* reset_out, void* stream) {
   AS_REQUIRE(h && out && actions, "handle/out/actions is null");
-  if (int rc = validate_state_in(in, true)) return rc;
+  if (int rc = validate_state_in(h, in, true)) return rc;
   AS_REQUIRE(actions_stride >= kJ, "actions stride too small");
   AS_REQUIRE(out->obs && out->reward && out->terminated && out->time_out, "step outputs must be set");
   AS_REQUIRE(out->obs_clip >= 0.0f, "obs_clip must be >= 0");
@@ -741,7 +761,7 @@ int as_finish_step(AsHandle* h, const AsExchange* global_stats, void* stream) {
 int as_step_pass1(AsHandle* h, const AsStateIn* in, const float* actions, int64_t actions_stride,
                   const int64_t* episode_length, const AsStepOut* out, void* stream) {
   AS_REQUIRE(h && out && actions, "handle/out/actions is null");
-  if (int rc = validate_state_in(in, false)) return rc;
+  if (int rc = validate_state_in(h, in, false)) return rc;
   AS_REQUIRE(actions_stride >= kJ, "actions stride too small");
   AS_REQUIRE(out->obs && out->reward && out->terminated && out->time_out, "step outputs must be set");
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
@@ -826,7 +846,7 @@ int as_reset(AsHandle* h, const float* env_origins, const int32_t* env_ids, int6
 
 int as_step_pass2(AsHandle* h, const AsStateIn* in, float* obs, void* stream) {
   AS_REQUIRE(h && obs, "handle/obs is null");
-  if (int rc = validate_state_in(in, false)) return rc;
+  if (int rc = validate_state_in(h, in, false)) return rc;
   // (no call-order precondition: the reference runs `_compute_useful_values` at the end of `_reset_idx` whether or
   // not a pass preceded it -- DirectRLEnv.reset() calls `_reset_idx(all ids)` before the first step, DRL:256-279)
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
@@ -953,12 +973,13 @@ int as_export_stone_poses(AsHandle* h, const int32_t* env_ids, int64_t n_ids, fl
                           void* stream) {
   AS_REQUIRE(h && view_poses, "null argument");
   AS_REQUIRE(n_ids >= 0 && n_ids <= h->num_envs, "n_ids out of range");
-  AS_REQUIRE(h->num_envs * kS < (1ll << 31), "view indices must fit 32 bits");
+  const int S = handle_stones(h);
+  AS_REQUIRE(h->num_envs * S < (1ll << 31), "view indices must fit 32 bits");
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
   if (!env_ids) n_ids = h->num_envs;
   if (n_ids == 0) return AS_OK;
-  const int grid = grid_for(n_ids * kS, 256, h->sm_count, 8);
-  k_export_stone_poses<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(h->ws, env_ids, n_ids, h->num_envs,
+  const int grid = grid_for(n_ids * S, 256, h->sm_count, 8);
+  k_export_stone_poses<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(h->ws, env_ids, n_ids, h->num_envs, S,
                                                                              view_poses, view_ids);
   return check_launch(h, "k_export_stone_poses");
 }
@@ -979,8 +1000,8 @@ namespace {
 struct SnapshotLayout {
   int64_t ctrl, state, window, bin, stale, stones, total;
 };
-SnapshotLayout snapshot_layout(int64_t n, bool with_stones) {
-  const WorkspaceLayout w = workspace_layout(n);
+SnapshotLayout snapshot_layout(int64_t n, int S, bool with_stones) {
+  const WorkspaceLayout w = workspace_layout(n, S);
   SnapshotLayout l;
   int64_t off = 0;
   l.ctrl = off;   off += w.state0_off - w.ctrl_off;
@@ -996,15 +1017,15 @@ SnapshotLayout snapshot_layout(int64_t n, bool with_stones) {
 
 int64_t as_snapshot_bytes(const AsHandle* h, int32_t include_stones) {
   if (!h) return 0;
-  return snapshot_layout(h->num_envs, include_stones != 0).total;
+  return snapshot_layout(h->num_envs, handle_stones(h), include_stones != 0).total;
 }
 
 int as_snapshot(AsHandle* h, void* dst, int32_t include_stones, void* stream) {
   AS_REQUIRE(h && dst, "null argument");
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const WorkspaceLayout w = workspace_layout(h->num_envs);
-  const SnapshotLayout l = snapshot_layout(h->num_envs, include_stones != 0);
+  const WorkspaceLayout w = workspace_layout(h->num_envs, handle_stones(h));
+  const SnapshotLayout l = snapshot_layout(h->num_envs, handle_stones(h), include_stones != 0);
   unsigned char* d = static_cast<unsigned char*>(dst);
   const unsigned char* base = reinterpret_cast<const unsigned char*>(h->ws.ctrl);
   AS_CUDA(cudaMemcpyAsync(d + l.ctrl, base + w.ctrl_off, static_cast<size_t>(l.window - l.ctrl), cudaMemcpyDeviceToDevice, s));
@@ -1020,8 +1041,8 @@ int as_restore(AsHandle* h, const void* src, int32_t include_stones, void* strea
   AS_REQUIRE(h && src, "null argument");
   if (h->pending_valid) return fail(AS_ERR_STATE, "a fused step is open; close it with as_finish_step");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const WorkspaceLayout w = workspace_layout(h->num_envs);
-  const SnapshotLayout l = snapshot_layout(h->num_envs, include_stones != 0);
+  const WorkspaceLayout w = workspace_layout(h->num_envs, handle_stones(h));
+  const SnapshotLayout l = snapshot_layout(h->num_envs, handle_stones(h), include_stones != 0);
   const unsigned char* d = static_cast<const unsigned char*>(src);
   unsigned char* base = reinterpret_cast<unsigned char*>(h->ws.ctrl);
   k_restore_ctrl<<<1, 256, 0, s>>>(h->ws.ctrl, reinterpret_cast<const Ctrl*>(d + l.ctrl));

@@ -17,13 +17,13 @@ namespace as {
 
 constexpr unsigned kFullMask = 0xffffffffu;
 
-// Sequential inclusive scan over the first kS lanes, accumulated in double exactly like torch.cumsum on CPU
+// Sequential inclusive scan over the first S lanes, accumulated in double exactly like torch.cumsum on CPU
 // (acc_type<float> is double there) -- a log-step warp scan would re-associate the additions.
-__device__ __forceinline__ float warp_cumsum_sequential(float x, int lane) {
+__device__ __forceinline__ float warp_cumsum_sequential(float x, int lane, int S) {
   double acc = 0.0;
   float mine = 0.0f;
 #pragma unroll
-  for (int s = 0; s < kS; ++s) {
+  for (int s = 0; s < S; ++s) {
     const float vs = __shfl_sync(kFullMask, x, s);
     acc += static_cast<double>(vs);
     if (lane == s) mine = static_cast<float>(acc);
@@ -53,10 +53,11 @@ __device__ __forceinline__ Difficulty difficulty_of_env(const AsParams& P, const
   return (P.flags & AS_FLAG_GRID_CURRICULUM) ? difficulty_of_bin(P, ws.bin[e]) : difficulty_of_level(P, level);
 }
 
-// ENV:125-174 for one env, one stone per lane (lanes >= kS idle).  `u_dr/u_dphi/u_dtheta` are this lane's draws.
+// ENV:125-174 for one env, one stone per lane (lanes >= S idle).  `u_dr/u_dphi/u_dtheta` are this lane's draws.
+// S: the course length (a compile-time constant where the caller knows it is the default).
 __device__ __forceinline__ void generate_stones_warp(const AsParams& P, int lane, const Difficulty& D,
                                                      const Vec3& origin, float u_dr, float u_dphi, float u_dtheta,
-                                                     float4* out_row) {
+                                                     float4* out_row, int S) {
   const float deg2rad = 0.017453292519943295f;  // torch.deg2rad multiplies by float32(pi/180)
   const float half_pi = 1.5707963705062866f;
   const float yaw_lo = (P.yaw_range_deg[0] * D.ratio_yaw) * deg2rad, yaw_hi = (P.yaw_range_deg[1] * D.ratio_yaw) * deg2rad;
@@ -70,34 +71,35 @@ __device__ __forceinline__ void generate_stones_warp(const AsParams& P, int lane
   } else if (lane <= 2) {                                                            // ENV:148-150
     dr = P.init_step_separation; dphi = 0.0f; dth = half_pi;
   }
-  if (lane >= kS) { dr = 0.0f; dphi = 0.0f; dth = half_pi; }
-  const float phi = warp_cumsum_sequential(dphi, lane);                              // ENV:155
+  if (lane >= S) { dr = 0.0f; dphi = 0.0f; dth = half_pi; }
+  const float phi = warp_cumsum_sequential(dphi, lane, S);                              // ENV:155
   const float st = sinf(dth), ct = cosf(dth);
   const float dx = (dr * st) * cosf(phi);                                            // ENV:157
   const float dy = (dr * st) * sinf(phi);                                            // ENV:158
   const float dz = dr * ct;                                                          // ENV:159
-  const float x = warp_cumsum_sequential(dx, lane);                                  // ENV:165-167
-  const float y = warp_cumsum_sequential(dy, lane);
-  const float z = warp_cumsum_sequential(dz, lane);
-  if (lane < kS) out_row[lane] = make_float4(x + origin.x, y + origin.y, z + origin.z, phi);  // ENV:111
+  const float x = warp_cumsum_sequential(dx, lane, S);                               // ENV:165-167
+  const float y = warp_cumsum_sequential(dy, lane, S);
+  const float z = warp_cumsum_sequential(dz, lane, S);
+  if (lane < S) out_row[lane] = make_float4(x + origin.x, y + origin.y, z + origin.z, phi);  // ENV:111
 }
 
-// The same for one env by ONE thread: the twenty stones in sequence, the four cumulative sums as running double
+// The same for one env by ONE thread: the S stones in sequence, the four cumulative sums as running double
 // accumulators (the additions happen in the same order, so the results are those of the warp version bit for bit).
 // `draw(k, s)`: uniform k (0 dr, 1 dphi, 2 dtheta) of stone s.  Used where many envs regenerate at once (the
 // reset-heavy configuration): a thread per env keeps thousands of independent chains in flight where a warp per env
-// spends its time in 4 x 20 dependent shuffle steps with 12 idle lanes.
+// spends its time in 4 x S dependent shuffle steps with 32 - S idle lanes.
 template <typename Draw>
 __device__ __forceinline__ void generate_stones_thread(const AsParams& P, const Difficulty& D, const Vec3& origin,
-                                                       Draw draw, float4* out_row, float4* window_row) {
+                                                       Draw draw, float4* out_row, float4* window_row, int S) {
   const float deg2rad = 0.017453292519943295f;
   const float half_pi = 1.5707963705062866f;
   const float yaw_lo = (P.yaw_range_deg[0] * D.ratio_yaw) * deg2rad, yaw_hi = (P.yaw_range_deg[1] * D.ratio_yaw) * deg2rad;
   const float pit_lo = (P.pitch_range_deg[0] * D.ratio_pitch) * deg2rad + half_pi;
   const float pit_hi = (P.pitch_range_deg[1] * D.ratio_pitch) * deg2rad + half_pi;
   double phi_acc = 0.0, x = 0.0, y = 0.0, z = 0.0;
+  float4 v;
 #pragma unroll 1
-  for (int s = 0; s < kS; ++s) {
+  for (int s = 0; s < S; ++s) {
     float dr = torch_lerp(P.dist_lower, D.dist_upper, draw(0, s));   // ENV:137
     float dphi = torch_lerp(yaw_lo, yaw_hi, draw(1, s));             // ENV:138
     float dth = torch_lerp(pit_lo, pit_hi, draw(2, s));              // ENV:139
@@ -112,7 +114,7 @@ __device__ __forceinline__ void generate_stones_thread(const AsParams& P, const 
     x += static_cast<double>((dr * st) * cosf(phi));                 // ENV:157,165
     y += static_cast<double>((dr * st) * sinf(phi));                 // ENV:158,166
     z += static_cast<double>(dr * ct);                               // ENV:159,167
-    float4 v = make_float4(static_cast<float>(x) + origin.x, static_cast<float>(y) + origin.y,
+    v = make_float4(static_cast<float>(x) + origin.x, static_cast<float>(y) + origin.y,
                            static_cast<float>(z) + origin.z, phi);   // ENV:111
     out_row[s] = v;
     if (s < 4) {  // the env restarts at index 1: window = stones 0..3, tagged
@@ -120,31 +122,33 @@ __device__ __forceinline__ void generate_stones_thread(const AsParams& P, const 
       window_row[s] = v;
     }
   }
+  if (S < 4) window_row[3] = v;  // (slot 3 holds stone min(3, S - 1): the last one)
 }
 
 // Rebuilds one env's stone window from its stone row (lanes 0..3); call after the row was (re)written.
-__device__ __forceinline__ void rebuild_window_warp(const float4* stone_row, float4* window_row, int idx, int lane) {
+__device__ __forceinline__ void rebuild_window_warp(const float4* stone_row, float4* window_row, int idx, int lane,
+                                                    int S) {
   __syncwarp();
   if (lane < 4) {
-    float4 v = stone_row[window_slot_stone(idx, lane)];
+    float4 v = stone_row[window_slot_stone(idx, lane, S)];
     if (lane == 0) v.w = __int_as_float(idx);
     window_row[lane] = v;
   }
 }
 
 __device__ __forceinline__ void stone_draws(const ResetArgs& a, unsigned long long step, int64_t e, uint32_t gid,
-                                            int lane, float& u_dr, float& u_dphi, float& u_dth) {
+                                            int lane, float& u_dr, float& u_dphi, float& u_dth, int S) {
   u_dr = u_dphi = u_dth = 0.0f;
-  if (lane >= kS) return;
+  if (lane >= S) return;
   if (a.stone_uniforms) {  // explicit (5,N,S) tables indexed by local env id
-    const int64_t plane = a.num_envs * kS;
-    u_dr = a.stone_uniforms[0 * plane + e * kS + lane];
-    u_dphi = a.stone_uniforms[1 * plane + e * kS + lane];
-    u_dth = a.stone_uniforms[2 * plane + e * kS + lane];
+    const int64_t plane = a.num_envs * S;
+    u_dr = a.stone_uniforms[0 * plane + e * S + lane];
+    u_dphi = a.stone_uniforms[1 * plane + e * S + lane];
+    u_dth = a.stone_uniforms[2 * plane + e * S + lane];
   } else {
-    u_dr = philox_uniform(a.P.seed, step, kStreamStones, gid, 0 * kS + lane);
-    u_dphi = philox_uniform(a.P.seed, step, kStreamStones, gid, 1 * kS + lane);
-    u_dth = philox_uniform(a.P.seed, step, kStreamStones, gid, 2 * kS + lane);
+    u_dr = philox_uniform(a.P.seed, step, kStreamStones, gid, 0 * S + lane);
+    u_dphi = philox_uniform(a.P.seed, step, kStreamStones, gid, 1 * S + lane);
+    u_dth = philox_uniform(a.P.seed, step, kStreamStones, gid, 2 * S + lane);
   }
 }
 
@@ -155,6 +159,7 @@ __device__ __forceinline__ void stone_draws(const ResetArgs& a, unsigned long lo
 //              decides regeneration and lists the envs that regenerate for k_reset_rows, writes compact rows.
 __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ ResetArgs a) {
   const AsParams& P = a.P;
+  const int S = static_cast<int>(P.num_steps);
   Ctrl* ctrl = a.ws.ctrl;
   const int lane = threadIdx.x & 31;
   const int64_t warp = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
@@ -213,7 +218,7 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
         }
       }
       // the rule of the fused step kernel: every env with the grid curriculum, else those past half of their stones
-      regen = (P.flags & AS_FLAG_GRID_CURRICULUM) || ((P.flags & AS_FLAG_INTENDED_REGEN) && state_idx(word) > kS / 2);
+      regen = (P.flags & AS_FLAG_GRID_CURRICULUM) || ((P.flags & AS_FLAG_INTENDED_REGEN) && state_idx(word) > S / 2);
       if (g == 0) {
         if (a.out.reset_ids) a.out.reset_ids[w] = static_cast<int32_t>(e);
         a.ws.reset_ids[w] = static_cast<int32_t>(e);  // (k_pass2_commit walks this list)
@@ -245,7 +250,7 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
       }
     }
     if (have && !regen && g < 4) {  // the env restarts at index 1 on its stones: its stone window
-      float4 v = a.ws.stones[e * kS + window_slot_stone(1, g)];
+      float4 v = a.ws.stones[e * S + window_slot_stone(1, g, S)];
       if (g == 0) v.w = __int_as_float(1);
       a.ws.window[e * 4 + g] = v;
     }
@@ -272,8 +277,8 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
 //   (b) the stone row (ENV:106-174) and the stone window of the env, at the new difficulty.
 // Two shapes of the same arithmetic (bit-identical: same draws, same order of the additions), chosen by the host from
 // the batch size: one WARP per env for small batches, where the list is a few hundred envs and the kernel is pure
-// latency -- the twenty stones' draws, interpolations and sines run side by side -- and one THREAD per env for large
-// ones, where thousands of independent chains in flight beat 4 x 20 dependent shuffle steps with 12 idle lanes
+// latency -- the S stones' draws, interpolations and sines run side by side -- and one THREAD per env for large
+// ones, where thousands of independent chains in flight beat 4 x S dependent shuffle steps with 32 - S idle lanes
 // (BASELINE config 5: 257 000 of 1 M envs regenerate per step).
 constexpr uint32_t kStreamGrid = 2;
 
@@ -298,13 +303,15 @@ __device__ __forceinline__ unsigned int grid_weight(unsigned int a, unsigned int
   return 1u + q;  // peaks at a 50 % success rate
 }
 
-template <bool BY_WARP>
+// DEFAULT_S: the handle runs courses of the default length, which the generators then take as a constant.
+template <bool BY_WARP, bool DEFAULT_S>
 __global__ void __launch_bounds__(256, 4) k_reset_rows(const __grid_constant__ ResetArgs a) {
   __shared__ unsigned int s_cdf[kMaxGridBins], s_att[kMaxGridBins], s_succ[kMaxGridBins];
   __shared__ unsigned int s_warp_tot[8];
   asm volatile("griddepcontrol.launch_dependents;");  // the finish kernel may become resident; it waits for us
   asm volatile("griddepcontrol.wait;" ::: "memory");  // the step kernel has completed: its id lists are final
   const AsParams& P = a.P;
+  const int S = DEFAULT_S ? kS : static_cast<int>(P.num_steps);
   Ctrl* ctrl = a.ws.ctrl;
   const int t = threadIdx.x, lane = t & 31, warp_in_cta = t >> 5;
   const int64_t n_regen = ctrl->n_regen_list;
@@ -339,10 +346,10 @@ __global__ void __launch_bounds__(256, 4) k_reset_rows(const __grid_constant__ R
     const int b0 = a.ws.bin[e];
     if (record && BY_WARP) {  // a short list spread over many CTAs: straight into the step's outcome record
       atomicAdd(&ctrl->grid_delta_att[b0], 1u);
-      if (a.ws.regen_info[w] > kS / 2) atomicAdd(&ctrl->grid_delta_succ[b0], 1u);
+      if (a.ws.regen_info[w] > S / 2) atomicAdd(&ctrl->grid_delta_succ[b0], 1u);
     } else if (record) {
       atomicAdd(&s_att[b0], 1u);
-      if (a.ws.regen_info[w] > kS / 2) atomicAdd(&s_succ[b0], 1u);
+      if (a.ws.regen_info[w] > S / 2) atomicAdd(&s_succ[b0], 1u);
     }
     const unsigned long long total = s_cdf[nb - 1];
     const uint4 blk = philox_block(P.seed, step, kStreamGrid, static_cast<uint32_t>(e + a.env_id_offset), 0);
@@ -382,9 +389,9 @@ __global__ void __launch_bounds__(256, 4) k_reset_rows(const __grid_constant__ R
       const Vec3 origin{a.env_origins[e * 3], a.env_origins[e * 3 + 1], a.env_origins[e * 3 + 2]};
       const Difficulty D = grid ? difficulty_of_bin(P, bin) : difficulty_of_level(P, level);
       float u0, u1, u2;
-      stone_draws(a, step, e, static_cast<uint32_t>(e + a.env_id_offset), lane, u0, u1, u2);
-      generate_stones_warp(P, lane, D, origin, u0, u1, u2, a.ws.stones + e * kS);
-      rebuild_window_warp(a.ws.stones + e * kS, a.ws.window + e * 4, 1, lane);  // the env restarts at index 1
+      stone_draws(a, step, e, static_cast<uint32_t>(e + a.env_id_offset), lane, u0, u1, u2, S);
+      generate_stones_warp(P, lane, D, origin, u0, u1, u2, a.ws.stones + e * S, S);
+      rebuild_window_warp(a.ws.stones + e * S, a.ws.window + e * 4, 1, lane, S);  // the env restarts at index 1
     }
   } else {
     const int64_t tid = static_cast<int64_t>(blockIdx.x) * blockDim.x + t;
@@ -396,21 +403,21 @@ __global__ void __launch_bounds__(256, 4) k_reset_rows(const __grid_constant__ R
       const Vec3 origin{a.env_origins[e * 3], a.env_origins[e * 3 + 1], a.env_origins[e * 3 + 2]};
       const Difficulty D = grid ? difficulty_of_bin(P, bin) : difficulty_of_level(P, level);
       if (a.stone_uniforms) {
-        const int64_t plane = a.num_envs * kS;
-        const float* tab = a.stone_uniforms + e * kS;
-        generate_stones_thread(P, D, origin, [&](int k, int s) { return tab[k * plane + s]; }, a.ws.stones + e * kS,
-                               a.ws.window + e * 4);
+        const int64_t plane = a.num_envs * S;
+        const float* tab = a.stone_uniforms + e * S;
+        generate_stones_thread(P, D, origin, [&](int k, int s) { return tab[k * plane + s]; }, a.ws.stones + e * S,
+                               a.ws.window + e * 4, S);
       } else {
-        // draw k * S + s is component s & 3 of Philox block 5 k + (s >> 2): three blocks serve four stones
+        // draw d = k * S + s is component d & 3 of Philox block d >> 2.  blk[k] holds the block of draw k * S + s; the
+        // three are fetched together whenever one of them enters a new block (S = 20: every fourth stone, blocks
+        // 5 k + (s >> 2) -- three blocks serve four stones)
         uint4 blk[3];
-        int have = -1;
         generate_stones_thread(P, D, origin, [&](int k, int s) {
-          if ((s >> 2) != have) {
-            have = s >> 2;
+          if (k == 0 && (s == 0 || (s & 3) == 0 || ((S + s) & 3) == 0 || ((2 * S + s) & 3) == 0)) {
 #pragma unroll
-            for (int q = 0; q < 3; ++q) blk[q] = philox_block(P.seed, step, kStreamStones, gid, static_cast<uint32_t>(5 * q + have));
+            for (int q = 0; q < 3; ++q) blk[q] = philox_block(P.seed, step, kStreamStones, gid, static_cast<uint32_t>((q * S + s) >> 2));
           }
-          return u32_to_unit(lane_of(blk[k], s & 3)); }, a.ws.stones + e * kS, a.ws.window + e * 4);
+          return u32_to_unit(lane_of(blk[k], (k * S + s) & 3)); }, a.ws.stones + e * S, a.ws.window + e * 4, S);
       }
     }
   }
@@ -437,9 +444,10 @@ __global__ void __launch_bounds__(256) k_generate_stones(const __grid_constant__
     const int level = min(state_level(st[e].x) + pending, a.P.max_level);
     const Vec3 origin{a.env_origins[e * 3], a.env_origins[e * 3 + 1], a.env_origins[e * 3 + 2]};
     float u0, u1, u2;
-    stone_draws(a, step, e, gid, lane, u0, u1, u2);
-    generate_stones_warp(a.P, lane, difficulty_of_env(a.P, a.ws, e, level), origin, u0, u1, u2, a.ws.stones + e * kS);
-    rebuild_window_warp(a.ws.stones + e * kS, a.ws.window + e * 4, state_idx(st[e].x), lane);
+    const int S = static_cast<int>(a.P.num_steps);
+    stone_draws(a, step, e, gid, lane, u0, u1, u2, S);
+    generate_stones_warp(a.P, lane, difficulty_of_env(a.P, a.ws, e, level), origin, u0, u1, u2, a.ws.stones + e * S, S);
+    rebuild_window_warp(a.ws.stones + e * S, a.ws.window + e * 4, state_idx(st[e].x), lane, S);
   }
 }
 
@@ -610,6 +618,7 @@ __global__ void __launch_bounds__(256) k_export(const __grid_constant__ AsParams
                                                 int64_t num_envs) {
   const uint2* st = ws.state[ws.ctrl->parity];
   const int pending = static_cast<int>(ws.ctrl->promote_cur);
+  const int S = static_cast<int>(P.num_steps);
   for (int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; e < num_envs;
        e += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const uint2 sw = st[e];
@@ -620,14 +629,14 @@ __global__ void __launch_bounds__(256) k_export(const __grid_constant__ AsParams
     if (dst.curriculum) dst.curriculum[e] = min(state_level(sw.x) + pending, P.max_level);
     if (dst.potentials) dst.potentials[e] = __uint_as_float(sw.y);
     if (dst.steps_pos || dst.steps_dphi) {
-      for (int s = 0; s < kS; ++s) {
-        const float4 v = ws.stones[e * kS + s];
+      for (int s = 0; s < S; ++s) {
+        const float4 v = ws.stones[e * S + s];
         if (dst.steps_pos) {
-          dst.steps_pos[(e * kS + s) * 3 + 0] = v.x;
-          dst.steps_pos[(e * kS + s) * 3 + 1] = v.y;
-          dst.steps_pos[(e * kS + s) * 3 + 2] = v.z;
+          dst.steps_pos[(e * S + s) * 3 + 0] = v.x;
+          dst.steps_pos[(e * S + s) * 3 + 1] = v.y;
+          dst.steps_pos[(e * S + s) * 3 + 2] = v.z;
         }
-        if (dst.steps_dphi) dst.steps_dphi[e * kS + s] = v.w;
+        if (dst.steps_dphi) dst.steps_dphi[e * S + s] = v.w;
       }
     }
   }
@@ -637,12 +646,13 @@ __global__ void __launch_bounds__(256) k_import(const __grid_constant__ AsParams
                                                 int64_t num_envs) {
   uint2* st = ws.state[ws.ctrl->parity];
   const int pending = static_cast<int>(ws.ctrl->promote_cur);
+  const int S = static_cast<int>(P.num_steps);
   for (int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; e < num_envs;
        e += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     uint2 sw = st[e];
     int idx = state_idx(sw.x), leg = state_leg(sw.x), cnt = state_count(sw.x), lvl = state_level(sw.x),
         ep = state_ep(sw.x);
-    if (src.curr_target_index) idx = static_cast<int>(min(max(src.curr_target_index[e], (int64_t)0), (int64_t)(kS - 1)));
+    if (src.curr_target_index) idx = static_cast<int>(min(max(src.curr_target_index[e], (int64_t)0), (int64_t)(S - 1)));
     if (src.swing_leg) leg = static_cast<int>(src.swing_leg[e] & 1);
     if (src.target_reach_count) cnt = static_cast<int>(min(max(src.target_reach_count[e], (int64_t)0), (int64_t)3));
     if (src.episode_length) ep = static_cast<int>(min(max(src.episode_length[e], (int64_t)0), (int64_t)kMaxEpisodeLength));
@@ -652,19 +662,19 @@ __global__ void __launch_bounds__(256) k_import(const __grid_constant__ AsParams
     if (src.potentials) sw.y = __float_as_uint(src.potentials[e]);
     st[e] = sw;
     if (src.steps_pos || src.steps_dphi) {
-      for (int s = 0; s < kS; ++s) {
-        float4 v = ws.stones[e * kS + s];
+      for (int s = 0; s < S; ++s) {
+        float4 v = ws.stones[e * S + s];
         if (src.steps_pos) {
-          v.x = src.steps_pos[(e * kS + s) * 3 + 0];
-          v.y = src.steps_pos[(e * kS + s) * 3 + 1];
-          v.z = src.steps_pos[(e * kS + s) * 3 + 2];
+          v.x = src.steps_pos[(e * S + s) * 3 + 0];
+          v.y = src.steps_pos[(e * S + s) * 3 + 1];
+          v.z = src.steps_pos[(e * S + s) * 3 + 2];
         }
-        if (src.steps_dphi) v.w = src.steps_dphi[e * kS + s];
-        ws.stones[e * kS + s] = v;
+        if (src.steps_dphi) v.w = src.steps_dphi[e * S + s];
+        ws.stones[e * S + s] = v;
       }
     }
     for (int k = 0; k < 4; ++k) {  // index and/or stones may have changed: rebuild the window
-      float4 v = ws.stones[e * kS + window_slot_stone(idx, k)];
+      float4 v = ws.stones[e * S + window_slot_stone(idx, k, S)];
       if (k == 0) v.w = __int_as_float(idx);
       ws.window[e * 4 + k] = v;
     }
@@ -677,16 +687,16 @@ __global__ void __launch_bounds__(256) k_import(const __grid_constant__ AsParams
 // (rigid_object_collection.py:295-301,650-659,675).  One thread per (stone, listed env): consecutive threads write
 // consecutive 28-byte rows when the ids are consecutive.
 __global__ void __launch_bounds__(256) k_export_stone_poses(Workspace ws, const int32_t* __restrict__ env_ids,
-                                                            int64_t n_ids, int64_t num_envs,
+                                                            int64_t n_ids, int64_t num_envs, int S,
                                                             float* __restrict__ view_poses,
                                                             int32_t* __restrict__ view_ids) {
-  const int64_t total = n_ids * kS;
+  const int64_t total = n_ids * S;
   for (int64_t w = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; w < total;
        w += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int64_t s = w / n_ids;
     const int64_t i = w - s * n_ids;
     const int64_t e = env_ids ? env_ids[i] : i;
-    const float4 v = ws.stones[e * kS + s];
+    const float4 v = ws.stones[e * S + s];
     const int64_t row = s * num_envs + e;
     float* dst = view_poses + row * 7;
     dst[0] = v.x; dst[1] = v.y; dst[2] = v.z;
@@ -784,9 +794,10 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
       const float* b_l = body + in.left_foot_row * in.body_row_stride;
       const float* b_t = body + in.torso_row * in.body_row_stride;
       const Vec3 rf{b_r[0], b_r[1], b_r[2]}, lf{b_l[0], b_l[1], b_l[2]};
-      const float4* stones = a.ws.stones + e * kS;
-      float4 s_prev = stones[window_slot_stone(m.idx, 0)], s_curr = stones[window_slot_stone(m.idx, 1)],
-             s_next = stones[window_slot_stone(m.idx, 2)];
+      const int S = static_cast<int>(P.num_steps);
+      const float4* stones = a.ws.stones + e * S;
+      float4 s_prev = stones[window_slot_stone(m.idx, 0, S)], s_curr = stones[window_slot_stone(m.idx, 1, S)],
+             s_next = stones[window_slot_stone(m.idx, 2, S)];
       const float f_r = contact_norm(in.contact_right + e * in.contact_right_stride, m.idx, false);
       const float f_l = contact_norm(in.contact_left + e * in.contact_left_stride, m.idx, false);
       const float h = b_t[2] - min_nan(lf.z, rf.z);                       // ENV:281-283
@@ -796,10 +807,10 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
       const Quat inv = quat_inverse(q);
       PassOut po{};
       const FootGeom gm = foot_geometry(P, rf, lf, f_r > P.contact_epsilon, f_l > P.contact_epsilon, s_curr);
-      if (foot_update(P, gm, m, po)) {  // (cannot happen on zeroed contact rows; kept general)
+      if (foot_update(P, gm, m, po, S)) {  // (cannot happen on zeroed contact rows; kept general)
         s_prev = s_curr;
         s_curr = s_next;
-        s_next = stones[min(m.idx + 1, kS - 1)];
+        s_next = stones[min(m.idx + 1, S - 1)];
       }
       targets_and_potential(P, a.inv_step_dt, exact, p, inv, s_prev, s_curr, s_next, m, po);
       if (g == 0) {

@@ -9,7 +9,7 @@
 namespace as {
 
 constexpr int kJ = AS_NUM_JOINTS;
-constexpr int kS = AS_NUM_STONES;
+constexpr int kS = AS_NUM_STONES;  // the default course length; a handle's own is AsParams::num_steps (normalised by as_create)
 constexpr int kObs = AS_OBS_DIM;
 #ifndef AS_KTILE
 #define AS_KTILE AS_TILE_ENVS
@@ -61,10 +61,11 @@ __host__ __device__ inline int state_ep(uint32_t w) { return static_cast<int>(w 
 constexpr int kMaxEpisodeLength = (1 << 20) - 2;
 
 // The stone window: a validated cache of the four stones around `curr_target_index` so that the step reads one
-// coalesced 64-byte record per env instead of three scattered 16-byte gathers out of the 320-byte stone row.
+// coalesced 64-byte record per env instead of three scattered 16-byte gathers out of the S x 16-byte stone row.
 // It is valid iff the tag equals the env's current index; every writer of the index or of the stones rewrites it,
 // and a reader that finds a stale tag falls back to gathering from `stones` (which is always authoritative).
-__device__ __forceinline__ int window_slot_stone(int idx, int slot) { return min(max(idx - 1 + slot, 0), kS - 1); }
+// S: the handle's course length.
+__device__ __forceinline__ int window_slot_stone(int idx, int slot, int S) { return min(max(idx - 1 + slot, 0), S - 1); }
 
 // Device control block at the head of the workspace.
 struct Ctrl {
@@ -143,7 +144,7 @@ struct PeerArgs {
 struct Workspace {
   Ctrl* ctrl;
   uint2* state[2];    // (N) packed state / potentials, ping-pong
-  float4* stones;     // (N,S) x,y,z (world frame), cumulative yaw
+  float4* stones;     // (N,S) x,y,z (world frame), cumulative yaw; S = AsParams::num_steps
   float4* window;     // (N,4) cache of stones idx-1, idx, idx+1, idx+2 (clamped); entry 0's .w holds idx as a tag
   int32_t* reset_ids; // (N)
   int32_t* regen_ids; // (N)
@@ -165,7 +166,8 @@ struct WorkspaceLayout {
 
 inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
 
-inline WorkspaceLayout workspace_layout(int64_t n) {
+// S: the handle's course length (the stone rows are the only part that depends on it)
+inline WorkspaceLayout workspace_layout(int64_t n, int S) {
   WorkspaceLayout l;
   int64_t off = 0;
   l.ctrl_off = off;
@@ -175,7 +177,7 @@ inline WorkspaceLayout workspace_layout(int64_t n) {
   l.state1_off = off;
   off = align_up(off + n * 8, 256);
   l.stones_off = off;
-  off = align_up(off + n * kS * 16, 256);
+  off = align_up(off + n * S * 16, 256);
   l.window_off = off;
   off = align_up(off + n * 4 * 16, 256);
   l.reset_ids_off = off;

@@ -11,7 +11,7 @@
 //   gathers       the packed 8-byte MDP state word and the 64-byte stone-window record are coalesced loads; the two
 //                 contact norms of the current stone come as one coalesced record from k_contact_gather* (large
 //                 batches) or are gathered here (small, launch-bound batches); stones a step has to fetch out of the
-//                 320-byte stone rows travel global -> shared asynchronously (cp.async) when nothing waits for them.
+//                 S x 16-byte stone rows travel global -> shared asynchronously (cp.async) when nothing waits for them.
 //   compute       dones -> pass 1 -> rewards -> masked reset (Philox) -> pass 2 -> observations.  The code of both
 //                 roles is kept STRAIGHT-LINE on purpose: the kernel is bound by how its two instruction streams
 //                 schedule (DESIGN.md section 6), every branch ends a basic block and a taken one refetches
@@ -177,10 +177,10 @@ __device__ __forceinline__ void coop_load(float* dst, const float* base, int64_t
   }
 }
 
-// Scattered reads (one 12/16-byte item out of a 240/320-byte row per env): by default a miss makes L2 pull the whole
-// 128-byte line out of DRAM; the L2::64B qualifier limits the fill to the 64-byte half that holds the item.  These
-// gathers are DRAM-byte bound, so that halves their cost (tools/gather_probe.cu: 259 -> 143 DRAM bytes per env,
-// 44 -> 27 us per 1M envs).  SASS: LDG.E.LTC64B...CONSTANT.
+// Scattered reads (one 12/16-byte item out of a 12 S / 16 S-byte row per env, 240 / 320 bytes at the default S = 20):
+// by default a miss makes L2 pull the whole 128-byte line out of DRAM; the L2::64B qualifier limits the fill to the
+// 64-byte half that holds the item.  These gathers are DRAM-byte bound, so that halves their cost
+// (tools/gather_probe.cu: 259 -> 143 DRAM bytes per env, 44 -> 27 us per 1M envs).  SASS: LDG.E.LTC64B...CONSTANT.
 __device__ __forceinline__ float4 ldg64_f4(const float4* p) {
   float4 r;
   asm("ld.global.nc.L2::64B.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
@@ -284,7 +284,8 @@ __device__ __forceinline__ FootGeom foot_geometry(const AsParams& P, const Vec3&
 }
 
 // ENV:433-457: reach counter, leg flip, index advance.  Returns true when the index changed (window must shift).
-__device__ __forceinline__ bool foot_update(const AsParams& P, const FootGeom& g, Mdp& m, PassOut& o) {
+// S: the course length.
+__device__ __forceinline__ bool foot_update(const AsParams& P, const FootGeom& g, Mdp& m, PassOut& o, int S) {
   o.contact_r = g.press_r ? 1.0f : 0.0f;
   o.contact_l = g.press_l ? 1.0f : 0.0f;
   o.reached = m.leg ? (g.press_l && g.d_l < P.step_radius) : (g.press_r && g.d_r < P.step_radius);
@@ -293,7 +294,7 @@ __device__ __forceinline__ bool foot_update(const AsParams& P, const FootGeom& g
   bool moved = false;
   if (o.advanced) {
     m.leg ^= 1;
-    const int nidx = min(m.idx + 1, kS - 1);
+    const int nidx = min(m.idx + 1, S - 1);
     moved = nidx != m.idx;
     m.idx = nidx;
     m.count = 0;
@@ -671,8 +672,8 @@ __device__ __forceinline__ void close_pass1_by_last_cta(const StepArgs& a, Ctrl*
 // `active` guards it removes are not free: each one ends a basic block, and the step is bound by how well the
 // instruction streams of its two roles schedule, not by DRAM (DESIGN.md section 6).
 // FAST: the launch uses none of the options -- w,x,y,z quaternions, no per-term reward output, no observation clamp,
-// no final observations.  The host checks that (select_step in as_api.cu) and the instantiation drops their uniform
-// branches.
+// no final observations, courses of the default AS_NUM_STONES stones.  The host checks that (select_step in as_api.cu)
+// and the instantiation drops their uniform branches and takes the course length as a constant.
 // (Measured: 179.3 -> 176.7 us per 1M-env step.  Also making the per-array "dense" bits compile-time constants
 // removes 45 more instructions per warp but ptxas then spills 56 instead of 20 bytes in the MDP role: 184 us.)
 // PRE: the launch follows k_prepare* (large batches, two-FMA quotients, contact matrices in device memory): the
@@ -685,6 +686,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
   const AsParams& P = a.P;
   const JointConsts& JC = a.jc;
   const bool exact = use_exact_div<EXACT>(JC);
+  const int S = FAST ? kS : static_cast<int>(P.num_steps);  // stones per course
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int warp = tid >> 5;
@@ -770,7 +772,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
   const uint32_t parity = ctrl->parity;
   const uint2* st_in = a.ws.state[parity];
   uint2* st_out = (kPingPong || kSpec) ? a.ws.state[parity ^ 1u] : a.ws.state[parity];
-  const float4* stones = a.ws.stones + e * kS;
+  const float4* stones = a.ws.stones + e * S;
   auto stone_at = [&](int i) -> float4 { return ldg64_f4(stones + i); };
   float4* wrow = a.ws.window + e * 4;
   const bool contact_aligned = ((reinterpret_cast<uintptr_t>(a.in.contact_right) | reinterpret_cast<uintptr_t>(
@@ -820,9 +822,9 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
     if (win_valid) {
       s_prev = w0; s_curr = w1; s_next = w2;
     } else {  // stale cache (first use, or the fix-up re-reading an env the step already advanced): gather
-      s_prev = stone_at(window_slot_stone(m.idx, 0));
-      s_curr = stone_at(window_slot_stone(m.idx, 1));
-      s_next = stone_at(window_slot_stone(m.idx, 2));
+      s_prev = stone_at(window_slot_stone(m.idx, 0, S));
+      s_curr = stone_at(window_slot_stone(m.idx, 1, S));
+      s_next = stone_at(window_slot_stone(m.idx, 2, S));
     }
   }
   // the index advanced by one: slide the window (the stone entering at the far end is fetched when written back)
@@ -833,7 +835,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
     // load is answered by L1/L2; gathering it from the stone row instead is a DRAM miss in the middle of the MDP
     // role's critical path (almost every warp has a lane that slides).  A second slide in one step (possible only
     // with stop_frames == 1) or a stale record falls back to the gather.
-    s_next = (win_valid && !win_dirty) ? wrow[3] : stone_at(min(m.idx + 1, kS - 1));
+    s_next = (win_valid && !win_dirty) ? wrow[3] : stone_at(min(m.idx + 1, S - 1));
     win_dirty = true;
   };
 
@@ -937,7 +939,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
     if (active) {
       h = torso_z - min_nan(lf.z, rf.z);   // ENV:281-283
       geom = foot_geometry(P, rf, lf, f_r, f_l, s_curr);
-      moved1 = foot_update(P, geom, m, po);
+      moved1 = foot_update(P, geom, m, po, S);
       if (moved1) slide_window();
     }
     orient_wait();  // roll / pitch / quat_inv of this env were computed by the joint role (ENV:285, MATH:238-248)
@@ -955,9 +957,9 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
           float* rt = a.out.reward_terms + e * AS_NUM_REWARD_TERMS;
           rt[0] = P.alive_reward_scale; rt[1] = r_progress; rt[4] = r_speed;
         }
-        const bool pays_step = po.reached && m.count == 1 && m.idx < kS - 1;
+        const bool pays_step = po.reached && m.count == 1 && m.idx < S - 1;
         r_step = pays_step ? 50.0f * expf((-po.d_swing) / 0.25f) : 0.0f;
-        r_bonus = (m.idx == kS - 1 && po.body_dist < 0.15f) ? 10.0f : 0.0f;
+        r_bonus = (m.idx == S - 1 && po.body_dist < 0.15f) ? 10.0f : 0.0f;
       }
     }
 
@@ -989,7 +991,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
         // ---- masked reset, ENV:487-538.  Pass 2 on the post-reset state: identity orientation (vector part +-0),
         // zero velocity, zero contacts (contact_sensor.py:155), stale body positions; so roll = pitch = v_b = 0 and
         // targets_b = stone - root.  The start-pose joints are produced by the joint-role warps.
-        regen = ((P.flags & AS_FLAG_INTENDED_REGEN) && m.idx > kS / 2) || (P.flags & AS_FLAG_GRID_CURRICULUM);
+        regen = ((P.flags & AS_FLAG_INTENDED_REGEN) && m.idx > S / 2) || (P.flags & AS_FLAG_GRID_CURRICULUM);
         const Vec3 org{s_org[t * 3], s_org[t * 3 + 1], s_org[t * 3 + 2]};
         p = Vec3{P.default_root_pos[0] + org.x, P.default_root_pos[1] + org.y, P.default_root_pos[2] + org.z};
         if (regen) {
@@ -1024,7 +1026,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
           }
           geom = foot_geometry(P, rf, lf, f_r, f_l, s_curr);
         }
-        const bool moved = foot_update(P, geom, m, po);
+        const bool moved = foot_update(P, geom, m, po, S);
         adv2 = po.advanced;  // (taken back with pass 2 by k_fixup_finish, k_pass2_revert or k_pass2_commit)
         if (moved) {
           slide_window();
@@ -1051,7 +1053,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
         // and storing it would park the warp on the store until DRAM answers (in-order issue), in the middle of the
         // MDP role's critical path and for nearly every warp; instead it travels global -> shared asynchronously
         // and is written back at the very end of the tile.
-        cp_async16(smem_u32(s_w3 + t), stones + window_slot_stone(m.idx, 3));
+        cp_async16(smem_u32(s_w3 + t), stones + window_slot_stone(m.idx, 3, S));
         w3_pending = true;
       }
     }
@@ -1441,7 +1443,7 @@ __device__ __forceinline__ void process_tile(const StepArgs& a, int tile, uint32
 //     one pass 2 looks at when pass 1 advances the index) out of the two (N,1,S,3) PhysX matrices, ENV:421-425 -- the
 //     two vectors are neighbours in the row, so the second one rides in the same 64-byte fills as the first;
 //   * the stone window of every env whose record went stale (the index moved or the env reset in the last step):
-//     stones idx-1 .. idx+2 out of its 320-byte stone row, tagged with idx -- the step kernel only reads windows;
+//     stones idx-1 .. idx+2 out of its S x 16-byte stone row, tagged with idx -- the step kernel only reads windows;
 //   * optionally the three body rows the task reads (right foot, left foot, torso: 12 bytes each) out of a strided
 //     (N,B,13) body_state_w tensor into a dense (N,3,3) array the step kernel takes by bulk copy.
 // These random DRAM reads are what floors the step (profiles/r01_membound_probe.txt); issued from inside the step
@@ -1457,10 +1459,11 @@ struct PrepareArgs {
                       // pass 1 advances the index
   int32_t stop_frames;  // ENV:56: pass 1 can advance the index only if the reach counter is one short of this
   float contact_epsilon;  // ENV:425
+  int32_t num_stones;     // S, the course length
 };
 
-__device__ __forceinline__ void refresh_window_entry(const Workspace& ws, int64_t e, int idx, int slot) {
-  float4 v = ldg64_f4(ws.stones + e * kS + window_slot_stone(idx, slot));
+__device__ __forceinline__ void refresh_window_entry(const Workspace& ws, int64_t e, int idx, int slot, int S) {
+  float4 v = ldg64_f4(ws.stones + e * S + window_slot_stone(idx, slot, S));
   if (slot == 0) v.w = __int_as_float(idx);  // tag
   ws.window[e * 4 + slot] = v;
 }
@@ -1473,7 +1476,7 @@ __global__ void __launch_bounds__(256) k_prepare(const __grid_constant__ Prepare
   const AsStateIn& in = a.in;
   const uint32_t word = a.ws.state[a.ws.ctrl->parity][e].x;
   const int idx = state_idx(word);
-  const int nxt = min(idx + 1, kS - 1);
+  const int nxt = min(idx + 1, a.num_stones - 1);
   const bool stale = (a.ws.win_stale[e >> 5] >> (e & 31)) & 1u;
   const float* rr = in.contact_right + e * in.contact_right_stride;
   const float* lr = in.contact_left + e * in.contact_left_stride;
@@ -1486,7 +1489,7 @@ __global__ void __launch_bounds__(256) k_prepare(const __grid_constant__ Prepare
       ((want_next && contact_norm(lr, nxt, false) > eps) ? 8u : 0u));
   if (stale) {
 #pragma unroll
-    for (int k = 0; k < 4; ++k) refresh_window_entry(a.ws, e, idx, k);
+    for (int k = 0; k < 4; ++k) refresh_window_entry(a.ws, e, idx, k, a.num_stones);
   }
   if (a.body_dense) {
 #pragma unroll
@@ -1520,7 +1523,7 @@ __global__ void __launch_bounds__(256) k_prepare_paired(const __grid_constant__ 
   // The next stone's vectors are needed only if pass 1 can advance the index at all (ENV:433-441: the reach counter is
   // one short of stop_frames) -- known from the state word alone, before any contact data: most envs fetch the 12 bytes
   // of the current stone only, which straddle a 64-byte fill boundary half as often as the 24 bytes of both stones.
-  const bool has_next = idx < kS - 1 && state_count(word) + 1 >= a.stop_frames;
+  const bool has_next = idx < a.num_stones - 1 && state_count(word) + 1 >= a.stop_frames;
   float4 r = make_float4(0.f, 0.f, 0.f, 0.f), l = r, r2 = r, l2 = r;
   const uint64_t once = policy_evict_first(), keep = policy_evict_last();
   if (live) {
@@ -1553,8 +1556,8 @@ __global__ void __launch_bounds__(256) k_prepare_paired(const __grid_constant__ 
   lc[8] = l2.x; lc[9] = 0.f; lc[10] = 0.f; lc[11] = 0.f;
   if (live) {
     if (stale) {  // lane h rewrites entries 2h, 2h+1 of the record
-      refresh_window_entry(a.ws, e, idx, 2 * half);
-      refresh_window_entry(a.ws, e, idx, 2 * half + 1);
+      refresh_window_entry(a.ws, e, idx, 2 * half, a.num_stones);
+      refresh_window_entry(a.ws, e, idx, 2 * half + 1, a.num_stones);
     }
     if (a.body_dense) {  // even lane: the two feet, odd lane: the torso
       const int b0 = half ? 2 : 0, b1 = half ? 3 : 2;

@@ -18,7 +18,7 @@ from typing import Dict, Optional
 
 import torch
 
-from .config import AllstepsCfg, JOINT_NAMES, NUM_JOINTS, NUM_STONES
+from .config import AllstepsCfg, JOINT_NAMES, NUM_JOINTS
 from .mdp import AllstepsMDP, PhysicsViews, StepBuffers
 
 
@@ -50,9 +50,10 @@ def resolve_robot_tables(robot, cfg: AllstepsCfg):
 
 def write_stone_poses(steps, mdp: AllstepsMDP, env_ids: torch.Tensor):
     """ENV:119-120: the stones of `env_ids` as the MDP holds them, written to the simulator's stone collection
-    (`RigidObjectCollection.write_object_pose_to_sim`, poses (k,S,7): position + identity quaternion w,x,y,z)."""
+    (`RigidObjectCollection.write_object_pose_to_sim`, poses (k,S,7): position + identity quaternion w,x,y,z; S is the
+    course length `mdp.num_steps`)."""
     pos = mdp.export_state(("steps_pos",))["steps_pos"][env_ids]
-    quat = torch.tensor([1.0, 0.0, 0.0, 0.0], device=pos.device).expand(pos.shape[0], NUM_STONES, 4)
+    quat = torch.tensor([1.0, 0.0, 0.0, 0.0], device=pos.device).expand(pos.shape[0], mdp.num_steps, 4)
     steps.write_object_pose_to_sim(torch.cat((pos, quat), dim=-1), env_ids)  # ENV:119-120
 
 
@@ -90,7 +91,7 @@ class AllstepsHooksB200:
         self.right_body_indices = as_idx(self.task_cfg.right_body_names)  # ENV:90
         self.left_body_indices = as_idx(self.task_cfg.left_body_names)  # ENV:91
         self.negation_body_indices = as_idx(self.task_cfg.negation_body_names)  # ENV:92
-        self.num_steps = self.task_cfg.num_steps
+        self.num_steps = self.mdp.num_steps  # CFG:90, the course length the kernels run
         self.actions = torch.zeros(self.num_envs, 21, device=dev)
         self._pass_epoch = -1
         self._generate_foot_steps()  # ENV:71

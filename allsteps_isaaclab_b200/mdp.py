@@ -13,7 +13,7 @@ from typing import Dict, Optional, Tuple
 import torch
 
 from . import _cabi
-from .config import AllstepsCfg, NUM_JOINTS, NUM_STONES, OBS_DIM
+from .config import AllstepsCfg, NUM_JOINTS, OBS_DIM
 from .params import make_params
 
 
@@ -33,6 +33,9 @@ class PhysicsViews:
 
     Accepts the tensors the reference reads (`robot.data.root_pos_w`, ..., `sensor_left.data.force_matrix_w`);
     strided views such as slices of `root_state_w (N,13)` / `body_state_w (N,B,13)` are taken as they are.
+
+    The contact matrices are (N,1,S,3), S the course length (`AllstepsCfg.num_steps`, 3..32); `num_steps` records it,
+    and the MDP refuses views whose S is not its own.
 
     The two contact matrices may also be PINNED HOST tensors: under unified addressing they are device-accessible,
     and since the step needs only the current stone's 12-byte vector per foot and env (24 of 480 bytes), letting the
@@ -71,23 +74,27 @@ class PhysicsViews:
         s.quat_xyzw = 1 if quat_xyzw else 0  # PhysX' own order; Isaac Lab's root_quat_w is w,x,y,z
         if max(body_rows) >= B:
             raise ValueError("body row index out of range")
+        S = force_matrix_right.shape[-2] if force_matrix_right.dim() >= 3 else -1
         for name, t in (("force_matrix_right", force_matrix_right), ("force_matrix_left", force_matrix_left)):
-            if t.dtype != torch.float32 or t.shape[0] != N or t.shape[-1] != 3 or t.shape[-2] != NUM_STONES:
-                raise ValueError(f"{name} must be float32 (N,1,{NUM_STONES},3)")
+            if (t.dtype != torch.float32 or t.dim() < 3 or t.shape[0] != N or t.shape[-1] != 3 or t.shape[-2] != S
+                    or not _cabi.MIN_STONES <= S <= _cabi.MAX_STONES):
+                raise ValueError(f"{name} must be float32 (N,1,S,3) with S in {_cabi.MIN_STONES}..{_cabi.MAX_STONES}, "
+                                 f"the same S for both feet; got {tuple(t.shape)}")
             if not t[0].is_contiguous():
                 raise ValueError(f"{name}: the per-env (1,S,3) block must be contiguous")
             if t.device.type == "cpu" and root_pos_w.device.type == "cuda" and not t.is_pinned():
                 raise ValueError(f"{name}: a host tensor must be pinned (page-locked) to be read by the device")
         s.contact_right = force_matrix_right.data_ptr()
-        s.contact_right_stride = force_matrix_right.stride(0) if N > 1 else NUM_STONES * 3
+        s.contact_right_stride = force_matrix_right.stride(0) if N > 1 else S * 3
         s.contact_left = force_matrix_left.data_ptr()
-        s.contact_left_stride = force_matrix_left.stride(0) if N > 1 else NUM_STONES * 3
+        s.contact_left_stride = force_matrix_left.stride(0) if N > 1 else S * 3
         if env_origins is not None:
             if env_origins.dtype != torch.float32 or tuple(env_origins.shape) != (N, 3) or not env_origins.is_contiguous():
                 raise ValueError("env_origins must be contiguous float32 (N,3)")
             s.env_origins = env_origins.data_ptr()
         self.struct = s
         self.num_envs = N
+        self.num_steps = S
         self.device = root_pos_w.device
 
     _FIELDS = ("root_pos_w", "root_quat_w", "root_lin_vel_w", "body_pos_w", "joint_pos", "joint_vel",
@@ -188,7 +195,8 @@ class AllstepsMDP:
         self.seed = int(seed)
         self.params = make_params(self.cfg, seed=seed, flags=flags, grid_bins=self.grid_bins,
                                   joint_limits=joint_limits)
-        nbytes = self.lib.as_workspace_bytes(self.num_envs)
+        self.num_steps = int(self.params.num_steps) or _cabi.NUM_STONES  # S, stones per course (CFG:90; 0: default)
+        nbytes = self.lib.as_workspace_bytes_for(C.byref(self.params), self.num_envs)
         with torch.cuda.device(self.device):
             self.workspace = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
             assert self.workspace.data_ptr() % 256 == 0
@@ -235,6 +243,13 @@ class AllstepsMDP:
     def launch_count(self) -> int:
         return int(self.lib.as_launch_count(self.handle))
 
+    def _check_views(self, views: PhysicsViews):
+        if views.num_envs != self.num_envs:
+            raise ValueError("views belong to a different number of envs")
+        if views.num_steps != self.num_steps:
+            raise ValueError(f"contact matrices are (N,1,{views.num_steps},3); this MDP runs courses of "
+                             f"num_steps={self.num_steps} stones")
+
     # ------------------------------------------------------------------ stones (ENV:106-174)
     def generate_stones(self, env_origins: torch.Tensor, env_ids: Optional[torch.Tensor] = None,
                         uniforms: Optional[torch.Tensor] = None):
@@ -245,9 +260,8 @@ class AllstepsMDP:
             ids_ptr, n_ids = env_ids.data_ptr(), env_ids.numel()
         if uniforms is not None:
             _require(uniforms, torch.float32, self.device, "uniforms")
-            if tuple(uniforms.shape) != (5, self.num_envs, NUM_STONES) and tuple(uniforms.shape) != (
-                    3, self.num_envs, NUM_STONES):
-                raise ValueError("uniforms must be (5|3, N, S)")
+            if tuple(uniforms.shape) not in ((5, self.num_envs, self.num_steps), (3, self.num_envs, self.num_steps)):
+                raise ValueError(f"uniforms must be (5|3, N, S) with S = num_steps = {self.num_steps}")
             uniforms = uniforms.contiguous()
         _cabi.check(self.lib.as_generate_stones(self.handle, env_origins.data_ptr(), ids_ptr, n_ids,
                                                 _ptr(uniforms), self._stream()), "as_generate_stones")
@@ -256,8 +270,7 @@ class AllstepsMDP:
     def step(self, views: PhysicsViews, actions: torch.Tensor, out: StepBuffers,
              global_stats: Optional[torch.Tensor] = None, finish: bool = True):
         """One MDP step in one fused launch. Results land in `out`; nothing is synchronised."""
-        if views.num_envs != self.num_envs:
-            raise ValueError("views belong to a different number of envs")
+        self._check_views(views)
         _require(actions, torch.float32, self.device, "actions")
         if actions.dim() != 2 or actions.shape != (self.num_envs, NUM_JOINTS) or actions.stride(1) != 1:
             raise ValueError("actions must be (N,21) with unit inner stride")
@@ -362,6 +375,7 @@ class AllstepsMDP:
     # ------------------------------------------------------------------ 3-call path
     def pass1(self, views: PhysicsViews, actions: torch.Tensor, out: StepBuffers,
               episode_length: Optional[torch.Tensor] = None):
+        self._check_views(views)
         _require(actions, torch.float32, self.device, "actions")
         stride = actions.stride(0) if self.num_envs > 1 else NUM_JOINTS
         if episode_length is not None:
@@ -388,6 +402,7 @@ class AllstepsMDP:
 
     def pass2(self, views: PhysicsViews, out: StepBuffers):
         """ENV:567 after the PhysX writes of `_reset_idx`: makes `out.obs` final for a step in which envs reset."""
+        self._check_views(views)
         _cabi.check(self.lib.as_step_pass2(self.handle, C.byref(views.struct), out.obs.data_ptr(), self._stream()),
                     "as_step_pass2")
         self._keepalive = (views, out)
@@ -425,24 +440,24 @@ class AllstepsMDP:
 
     def export_state(self, fields: Optional[Tuple[str, ...]] = None) -> Dict[str, torch.Tensor]:
         """The MDP state in the reference's own buffers (ENV:48,74-78, DRL:179).  `fields`: only these (default all;
-        `prev_target_index` / `next_target_index` come with `curr_target_index`) -- the 320-byte stone rows are the
+        `prev_target_index` / `next_target_index` come with `curr_target_index`) -- the S x 16-byte stone rows are the
         bulk of a full export, a caller that logs one counter per step should not pay for them."""
-        N, dev = self.num_envs, self.device
+        N, S, dev = self.num_envs, self.num_steps, self.device
         want = set(self._STATE_FIELDS if fields is None else fields)
         if want & {"prev_target_index", "next_target_index"}:
             want.add("curr_target_index")
         unknown = want - set(self._STATE_FIELDS) - {"prev_target_index", "next_target_index"}
         if unknown:
             raise KeyError(f"unknown state fields: {sorted(unknown)}")
-        shapes = {"potentials": ((N,), torch.float32), "steps_pos": ((N, NUM_STONES, 3), torch.float32),
-                  "steps_dphi": ((N, NUM_STONES), torch.float32)}
+        shapes = {"potentials": ((N,), torch.float32), "steps_pos": ((N, S, 3), torch.float32),
+                  "steps_dphi": ((N, S), torch.float32)}
         d = {k: torch.empty(*shapes.get(k, ((N,), torch.int64))[0], dtype=shapes.get(k, ((N,), torch.int64))[1], device=dev)
              for k in self._STATE_FIELDS if k in want}
         st = _cabi.AsMdpState(*[_ptr(d.get(k)) for k in self._STATE_FIELDS])
         _cabi.check(self.lib.as_export_state(self.handle, C.byref(st), self._stream()), "as_export_state")
         if "curr_target_index" in d:
-            d["prev_target_index"] = torch.clamp(d["curr_target_index"] - 1, 0, NUM_STONES - 1)  # ENV:76
-            d["next_target_index"] = torch.clamp(d["curr_target_index"] + 1, 0, NUM_STONES - 1)  # ENV:77
+            d["prev_target_index"] = torch.clamp(d["curr_target_index"] - 1, 0, S - 1)  # ENV:76
+            d["next_target_index"] = torch.clamp(d["curr_target_index"] + 1, 0, S - 1)  # ENV:77
         return d
 
     def export_stone_poses(self, env_ids: Optional[torch.Tensor] = None, view_poses: Optional[torch.Tensor] = None):
@@ -450,17 +465,17 @@ class AllstepsMDP:
         (S*N,7) x,y,z,w tensor plus their view indices -- `steps.root_physx_view.set_transforms(view_poses,
         indices=view_ids)` replaces ENV:119-120 + rigid_object_collection.py:295-301 (no whole-tensor clone, quaternion
         conversion or transpose).  `view_poses` may be a persistent buffer; rows of other envs are left untouched."""
-        N, dev = self.num_envs, self.device
+        N, S, dev = self.num_envs, self.num_steps, self.device
         if view_poses is None:
-            view_poses = torch.zeros(NUM_STONES * N, 7, dtype=torch.float32, device=dev)
+            view_poses = torch.zeros(S * N, 7, dtype=torch.float32, device=dev)
         _require(view_poses, torch.float32, dev, "view_poses")
-        if tuple(view_poses.shape) != (NUM_STONES * N, 7) or not view_poses.is_contiguous():
+        if tuple(view_poses.shape) != (S * N, 7) or not view_poses.is_contiguous():
             raise ValueError("view_poses must be a contiguous (S*N,7) tensor")
         ids_ptr, k = None, N
         if env_ids is not None:
             env_ids = env_ids.to(device=dev, dtype=torch.int32).contiguous()
             ids_ptr, k = env_ids.data_ptr(), env_ids.numel()
-        view_ids = torch.empty(NUM_STONES * k, dtype=torch.int32, device=dev)
+        view_ids = torch.empty(S * k, dtype=torch.int32, device=dev)
         if k:
             _cabi.check(self.lib.as_export_stone_poses(self.handle, ids_ptr, k, view_poses.data_ptr(),
                                                        view_ids.data_ptr(), self._stream()), "as_export_stone_poses")
@@ -480,12 +495,12 @@ class AllstepsMDP:
             keep[name] = t
             return t.data_ptr()
 
-        N = self.num_envs
+        N, S = self.num_envs, self.num_steps
         st = _cabi.AsMdpState(
             get("curr_target_index", torch.int64, (N,)), get("swing_leg", torch.int64, (N,)),
             get("target_reach_count", torch.int64, (N,)), get("episode_length_buf", torch.int64, (N,)),
             get("curriculum", torch.int64, (N,)), get("potentials", torch.float32, (N,)),
-            get("steps_pos", torch.float32, (N, NUM_STONES, 3)), get("steps_dphi", torch.float32, (N, NUM_STONES)))
+            get("steps_pos", torch.float32, (N, S, 3)), get("steps_dphi", torch.float32, (N, S)))
         _cabi.check(self.lib.as_import_state(self.handle, C.byref(st), self._stream()), "as_import_state")
         self._keepalive = keep
 
@@ -563,13 +578,14 @@ class AllstepsMDP:
         d = {k: v.cpu() for k, v in self.export_state().items()}
         d["snapshot"] = self.snapshot(include_stones=True).cpu()
         d["meta"] = torch.tensor([_cabi.ABI_VERSION, self.num_envs, self.env_id_offset, self.seed,
-                                  int(self.params.flags), self.grid_bins], dtype=torch.int64)
+                                  int(self.params.flags), self.grid_bins, self.num_steps], dtype=torch.int64)
         return d
 
     def load_state_dict(self, d: Dict[str, torch.Tensor]):
         meta = [int(x) for x in d["meta"].tolist()]
-        mine = [_cabi.ABI_VERSION, self.num_envs, self.env_id_offset, self.seed, int(self.params.flags), self.grid_bins]
-        names = ["abi", "num_envs", "env_id_offset", "seed", "flags", "grid_bins"]
+        mine = [_cabi.ABI_VERSION, self.num_envs, self.env_id_offset, self.seed, int(self.params.flags), self.grid_bins,
+                self.num_steps]
+        names = ["abi", "num_envs", "env_id_offset", "seed", "flags", "grid_bins", "num_steps"]
         for name, a, b in zip(names, meta, mine):
             if a != b:
                 raise ValueError(f"checkpoint was taken with {name}={a}, this handle has {name}={b}")

@@ -5,6 +5,8 @@ fp32 values are identical to the reference's.
 """
 from __future__ import annotations
 
+import numbers
+
 import torch
 
 from . import _cabi
@@ -19,7 +21,11 @@ def make_params(cfg: AllstepsCfg, seed: int = 0, flags: int = 0, grid_bins: int 
                 joint_limits=None) -> _cabi.AsParams:
     """joint_limits: optional (J,2) tensor / nested list [lower, upper] in radians, as the simulator reports them
     (`robot.data.joint_pos_limits[0]`); default: the MJCF ranges converted in double (config.py)."""
+    S = cfg.num_steps
+    if isinstance(S, bool) or not isinstance(S, numbers.Integral) or not _cabi.MIN_STONES <= S <= _cabi.MAX_STONES:
+        raise ValueError(f"num_steps must be an integer in {_cabi.MIN_STONES}..{_cabi.MAX_STONES} (CFG:90), got {S!r}")
     p = _cabi.AsParams()
+    p.num_steps = int(S)
     n_levels = cfg.max_curriculum + 1
     assert n_levels <= _cabi.NUM_LEVELS
     p.step_dt = cfg.step_dt

@@ -27,10 +27,12 @@
 extern "C" {
 #endif
 
-#define AS_ABI_VERSION 4
+#define AS_ABI_VERSION 5
 
 #define AS_NUM_JOINTS 21  /* CFG:57  action_space            */
-#define AS_NUM_STONES 20  /* CFG:90  num_steps               */
+#define AS_NUM_STONES 20  /* CFG:90  num_steps: the default course length (AsParams.num_steps = 0) */
+#define AS_MIN_STONES 3   /* stones 0..2 are the fixed start stones, ENV:144-150 */
+#define AS_MAX_STONES 32  /* the packed state word holds curr_target_index in 5 bits */
 #define AS_OBS_DIM 59     /* CFG:58  observation_space       */
 #define AS_NUM_LEVELS 10  /* ENV:45  max_curriculum + 1      */
 #define AS_ROOT_STATE_DIM 13
@@ -97,6 +99,8 @@ typedef struct AsParams {
                                       foot's body origin counts as "down" (extension, no reference counterpart) */
   uint32_t flags;
   uint32_t grid_bins;              /* AS_FLAG_GRID_CURRICULUM: bins per axis (<= 16), else 0            */
+  uint32_t num_steps;              /* CFG:90: stones per course, S, in AS_MIN_STONES..AS_MAX_STONES; 0 = AS_NUM_STONES.
+                                      Every "S" below is this value of the handle.                      */
   uint64_t seed;                   /* Philox key                                                        */
 } AsParams;
 
@@ -114,8 +118,9 @@ typedef struct AsStateIn {
                          articulation_data.py:372-379); 0: w,x,y,z as robot.data.root_quat_w                        */
   const float* joint_pos;     int64_t joint_pos_stride;    /* robot.data.joint_pos       (N,21)             */
   const float* joint_vel;     int64_t joint_vel_stride;    /* robot.data.joint_vel       (N,21)             */
-  const float* contact_right; int64_t contact_right_stride;/* sensor_right.data.force_matrix_w (N,1,S,3)    */
-  const float* contact_left;  int64_t contact_left_stride; /* sensor_left.data.force_matrix_w  (N,1,S,3)    */
+  const float* contact_right; int64_t contact_right_stride;/* sensor_right.data.force_matrix_w (N,1,S,3),   */
+  const float* contact_left;  int64_t contact_left_stride; /* sensor_left.data.force_matrix_w  (N,1,S,3),   */
+                                                            /* S = AsParams.num_steps; strides >= 3 S         */
   const float* env_origins;                                 /* scene.env_origins (N,3) contiguous            */
 } AsStateIn;
 
@@ -195,9 +200,12 @@ typedef struct AsHandle AsHandle;
 /* ---- lifetime --------------------------------------------------------------------------------------- */
 int as_abi_version(void);
 const char* as_last_error(void);
-/* Bytes of device workspace needed for `num_envs` envs (MDP state: stones, packed state, control block). */
+/* Bytes of device workspace needed for `num_envs` envs (MDP state: stones, packed state, control block) with courses
+ * of AS_NUM_STONES stones. */
 int64_t as_workspace_bytes(int64_t num_envs);
-/* `workspace`: device memory of as_workspace_bytes() bytes, 256-byte aligned, zero-initialised by this call.
+/* The same for the course length of `params` (params->num_steps); 0 when num_envs <= 0 or num_steps is out of range. */
+int64_t as_workspace_bytes_for(const AsParams* params, int64_t num_envs);
+/* `workspace`: device memory of as_workspace_bytes_for(params, num_envs) bytes, 256-byte aligned, zero-initialised by this call.
  * `env_id_offset`: global id of local env 0 (env-id sharding; Philox is keyed by global id).
  * Replaces AllstepsEnv.__init__ buffer allocation, ENV:41-96. */
 int as_create(const AsParams* params, int64_t num_envs, int64_t env_id_offset, int device,
@@ -206,7 +214,8 @@ void as_destroy(AsHandle* h);
 
 /* ---- stones: ENV:106-174 `_generate_foot_steps` -------------------------------------------------------
  * env_ids: NULL = all envs, else `n_ids` local ids (device, int32).  uniforms: NULL = in-kernel Philox at the
- * current step counter, else device (5,N,S) floats indexed by LOCAL env id (replay of external draws).
+ * current step counter, else device (5,N,S) floats indexed by LOCAL env id (replay of external draws); S is
+ * AsParams.num_steps.
  * levels are taken from the per-env state. */
 int as_generate_stones(AsHandle* h, const float* env_origins, const int32_t* env_ids, int64_t n_ids,
                        const float* uniforms, void* stream);
@@ -339,7 +348,7 @@ typedef struct AsMdpState {
   int64_t* episode_length;    /* (N) */
   int64_t* curriculum;        /* (N) */
   float* potentials;          /* (N) */
-  float* steps_pos;           /* (N,S,3) */
+  float* steps_pos;           /* (N,S,3), S = AsParams.num_steps */
   float* steps_dphi;          /* (N,S)   */
 } AsMdpState;
 int as_export_state(AsHandle* h, const AsMdpState* dst, void* stream);
@@ -360,7 +369,7 @@ int as_restore(AsHandle* h, const void* src, int32_t include_stones, void* strea
  * cat((steps_pos, [1,0,0,0])) -> scatter into object_state_w -> clone + convert_quat(to="xyzw") of the WHOLE (N,S,7)
  * tensor -> einsum transpose (reshape_data_to_view, :650-659), the kernel writes, for the k listed envs only, the rows
  * `view_poses[s*N + e] = (x, y, z, 0, 0, 0, 1)` of the object-major (S*N,7) x,y,z,w tensor and the index list
- * `view_ids[s*k + i] = s*N + env_ids[i]` (_env_obj_ids_to_view_ids, :675) -- the two arguments of
+ * `view_ids[s*k + i] = s*N + env_ids[i]` (_env_obj_ids_to_view_ids, :675), S = AsParams.num_steps -- the two arguments of
  * root_physx_view.set_transforms(view_poses, indices=view_ids).  env_ids == NULL: all envs (k = N, in order).
  * view_ids may be NULL. */
 int as_export_stone_poses(AsHandle* h, const int32_t* env_ids, int64_t n_ids, float* view_poses, int32_t* view_ids,

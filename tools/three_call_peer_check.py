@@ -1,6 +1,7 @@
 """The global 3-call mode across shards against one handle holding all envs (run under torchrun, one rank per GPU).
 
-    python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 tools/three_call_peer_check.py
+    python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 tools/three_call_peer_check.py \
+        [--num-steps S]
 
 Every rank owns one env-id shard of the same seeded scenario and drives it through the 3-call path (`pass1` ->
 `reset` -> `pass2`, or `no_reset`) in the global 3-call mode (`connect_peers(three_call=True)`); rank 0 also drives ONE
@@ -15,7 +16,10 @@ The tool asserts that it met each of these.  Then the same through `StandaloneAl
 THREE_CALL_CHECK_BACKEND=gloo runs the ranks as processes sharing GPU (rank % device_count), as tools/peer_check.py
 does.  THREE_CALL_CHECK_MODE=local runs the shards shard-local (no peers: the 3-call path's behaviour before the
 global mode) and reports the first step at which they part from the single handle, and what differs there.
+--num-steps runs courses of S stones (default 20); the promotion threshold is scaled to 12 S / 20, so that the scenario
+still promotes.
 """
+import argparse
 import os
 import sys
 import types
@@ -27,6 +31,7 @@ import torch
 import torch.distributed as dist
 
 from allsteps_isaaclab_b200 import synthetic as syn
+from allsteps_isaaclab_b200.config import AllstepsCfg
 from allsteps_isaaclab_b200.mdp import AllstepsMDP, PhysicsViews, StepBuffers
 from allsteps_isaaclab_b200.sharding import STATS_ADDITIVE_FIELDS
 from scenario import Scenario
@@ -38,6 +43,11 @@ FALLS = ("all", "first", "last", "none")
 
 
 def main():
+    ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
+    ap.add_argument("--num-steps", type=int, default=20, help="stones per course (AllstepsCfg.num_steps)")
+    S = ap.parse_args().num_steps
+    cfg = AllstepsCfg(num_steps=S, curriculum_progress_threshold=AllstepsCfg().curriculum_progress_threshold * S / 20)
+    lo = 9 * S // 20  # (indices from here up sit above the promotion threshold on average)
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     backend = os.environ.get("THREE_CALL_CHECK_BACKEND", "nccl")
     local = int(os.environ.get("LOCAL_RANK", rank)) if backend == "nccl" else rank % torch.cuda.device_count()
@@ -60,13 +70,13 @@ def main():
     steps = int(os.environ.get("THREE_CALL_CHECK_STEPS", "24"))
     B = int(os.environ.get("THREE_CALL_CHECK_GRID", "5"))
     N, seed = per * world, 29
-    sc = Scenario(N, seed=seed)  # same seed on every rank: identical CPU-side scenario
+    sc = Scenario(N, seed=seed, cfg=cfg)  # same seed on every rank: identical CPU-side scenario
     st0 = sc.initial_mdp_state()
-    st0["curr_target_index"] = torch.randint(9, 20, (N,), generator=sc.gen)  # above the promotion threshold
+    st0["curr_target_index"] = torch.randint(lo, S, (N,), generator=sc.gen)  # above the promotion threshold
     st0["episode_length_buf"] = torch.randint(0, 600, (N,), generator=sc.gen)  # no time-outs during the run
     sl = slice(rank * per, (rank + 1) * per)
     origins = sc.env_origins[sl].to(dev)
-    shard = AllstepsMDP(per, device=dev, seed=seed, env_id_offset=rank * per, grid_bins=B)
+    shard = AllstepsMDP(per, device=dev, cfg=cfg, seed=seed, env_id_offset=rank * per, grid_bins=B)
     shard.generate_stones(origins)
     shard.import_state({k: st0[k][sl] for k in STATE_KEYS})
     if mode == "global":
@@ -75,7 +85,7 @@ def main():
     ep = st0["episode_length_buf"][sl].to(dev)
     single = out_s = ep_s = None
     if rank == 0:
-        single = AllstepsMDP(N, device=dev, seed=seed, grid_bins=B)
+        single = AllstepsMDP(N, device=dev, cfg=cfg, seed=seed, grid_bins=B)
         single.generate_stones(sc.env_origins.to(dev))
         single.import_state({k: st0[k] for k in STATE_KEYS})
         out_s = StepBuffers(N, dev, final_obs=True)
@@ -137,7 +147,7 @@ def main():
     if bad and rank == 0:
         print(f"three_call_peer_check LOCAL DIFFERS at the reset outside a step: {', '.join(bad)}", flush=True)
     # the reset put every env back at index 1: indices above the promotion threshold again, so that steps promote
-    high = {"curr_target_index": torch.randint(9, 20, (N,), generator=sc.gen)}
+    high = {"curr_target_index": torch.randint(lo, S, (N,), generator=sc.gen)}
     shard.import_state({k: v[sl] for k, v in high.items()})
     if rank == 0:
         single.import_state(high)
@@ -202,14 +212,14 @@ def main():
         return
     assert all(v > 0 for v in met.values()), f"the scenario missed a case it must contain: {met}"
     assert shard.peer_status()["timeouts"] == 0
-    standalone_env_check(rank, world, dev, gather_cat)
+    standalone_env_check(rank, world, dev, gather_cat, cfg)
     if rank == 0:
-        print(f"three_call_peer_check OK: world {world} ({backend}, grid {B}x{B}), {per} envs per rank, {steps} steps "
+        print(f"three_call_peer_check OK: world {world} ({backend}, grid {B}x{B}), {S} stones, {per} envs per rank, {steps} steps "
               f"+ a reset outside a step, shards == single handle; {met}", flush=True)
     dist.destroy_process_group()
 
 
-def standalone_env_check(rank, world, dev, gather_cat):
+def standalone_env_check(rank, world, dev, gather_cat, cfg):
     """`StandaloneAllstepsEnv(..., distributed=True)` on every rank against one plain env holding all envs (rank 0):
     reset() then steps through the hooks; observations, rewards, masks, levels and stones must be equal."""
     from allsteps_isaaclab_b200.env import StandaloneAllstepsEnv
@@ -217,7 +227,7 @@ def standalone_env_check(rank, world, dev, gather_cat):
 
     per, seed, B = 640, 37, 7
     N = per * world
-    sc = Scenario(N, seed=seed, full_bodies=True, fall_fraction=0.08)
+    sc = Scenario(N, seed=seed, full_bodies=True, fall_fraction=0.08, cfg=cfg)
     sl = slice(rank * per, (rank + 1) * per)
     shard_sc = types.SimpleNamespace(N=per, joint_limits=sc.joint_limits, cfg=sc.cfg)
 
@@ -226,7 +236,7 @@ def standalone_env_check(rank, world, dev, gather_cat):
         scene = types.SimpleNamespace(env_origins=origins.to(dev))
         return StandaloneAllstepsEnv(robot, left, right, scene, str(dev), sc.cfg, seed=seed, grid_bins=B, **kw)
 
-    zero = sc.physics(torch.zeros(N, 20, 3), torch.ones(N, dtype=torch.int64), torch.zeros(N, dtype=torch.int64))
+    zero = sc.physics(torch.zeros(N, cfg.num_steps, 3), torch.ones(N, dtype=torch.int64), torch.zeros(N, dtype=torch.int64))
     env = make(shard_sc, {k: v[sl] for k, v in zero.items()}, sc.env_origins[sl], distributed=True)
     assert env.mdp.env_id_offset == rank * per
     ref = make(sc, zero, sc.env_origins) if rank == 0 else None
