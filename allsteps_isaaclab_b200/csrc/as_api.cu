@@ -631,7 +631,7 @@ int as_step_fused(AsHandle* h, const AsStateIn* in, const float* actions, int64_
 int as_fold_stats(AsHandle* h, void* stream) {
   AS_REQUIRE(h, "handle is null");
   if (!h->pending_valid) return fail(AS_ERR_STATE, "as_fold_stats belongs between as_step_fused and as_finish_step");
-  k_fold_early<<<1, 128, 0, static_cast<cudaStream_t>(stream)>>>(h->ws.ctrl, h->num_envs);
+  k_fold_early<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(h->ws.ctrl, h->num_envs);
   return check_launch(h, "k_fold_early");
 }
 

@@ -152,11 +152,9 @@ __device__ __forceinline__ void stone_draws(const ResetArgs& a, unsigned long lo
   }
 }
 
-// Kernel (b).  One warp per listed env.
-//   fused = 1: lists were compacted by the step kernel (ws.reset_ids / ws.regen_ids), MDP words already reset;
-//              PhysX rows are written at the env's own row of full-size buffers.
-//   fused = 0: explicit `env_ids` (3-call path): also resets the MDP word and the DirectRLEnv episode counter,
-//              decides regeneration and lists the envs that regenerate for k_reset_rows, writes compact rows.
+// Kernel (b) of the 3-call path (as_reset; behind the fused step the step kernel resets its envs itself).  For the
+// explicit `env_ids`: resets the MDP word and the DirectRLEnv episode counter, writes the compact PhysX rows, decides
+// regeneration and lists the envs that regenerate for k_reset_rows.
 __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ ResetArgs a) {
   const AsParams& P = a.P;
   const int S = static_cast<int>(P.num_steps);
@@ -165,9 +163,9 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
   const int64_t warp = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
   const unsigned long long step = ctrl->step_counter;
-  // fused: the step kernel already wrote the start-pose rows; n_ids < 0: the list pass 1 compacted on the device
-  const int64_t n_reset = a.fused ? 0 : (a.n_ids < 0 ? static_cast<int64_t>(ctrl->n_reset_list) : a.n_ids);
-  if (!a.fused && !a.peer_decided && blockIdx.x == 0 && threadIdx.x == 0) {
+  // n_ids < 0: the list pass 1 compacted on the device
+  const int64_t n_reset = a.n_ids < 0 ? static_cast<int64_t>(ctrl->n_reset_list) : a.n_ids;
+  if (!a.peer_decided && blockIdx.x == 0 && threadIdx.x == 0) {
     // 3-call path: `_reset_idx` opens with the promotion rule (ENV:471-479) on the statistics pass 1 folded.  The
     // decision is in force from here on: k_reset_rows regenerates at the promoted level (ENV:471 precedes ENV:500),
     // the next pass 1 applies it to the state words.  (Global 3-call mode: k_peer_exchange decided it on the sums.)
@@ -176,8 +174,8 @@ __global__ void __launch_bounds__(256, 3) k_reset_list(const __grid_constant__ R
     ctrl->promote_cur = promotion_decision(P, s);
   }
   const uint32_t parity = ctrl->parity;
-  // fused: the step wrote the other buffer; 3-call path after a speculating pass 1: so did that pass
-  uint2* st_cur = (a.fused || a.into_other) ? a.ws.state[parity ^ 1u] : a.ws.state[parity];
+  // after a speculating pass 1 the step continues in the other state buffer
+  uint2* st_cur = a.into_other ? a.ws.state[parity ^ 1u] : a.ws.state[parity];
   // Explicit id list (3-call path).  FOUR envs per warp, eight lanes each: a reset env is a chain of dependent loads
   // (id -> state word -> origins -> stones) with a little arithmetic in between, so a warp per env leaves the kernel
   // latency-bound at a few thousand resident warps; four independent chains per warp quadruple the loads in flight.
@@ -750,6 +748,20 @@ struct CommitArgs {
                            // grid outcomes stay in Ctrl::grid_delta_* for the next k_peer_exchange to sum and add
 };
 
+// Takes the speculated pass 2 back (grid-stride over the whole launch): the observation tails of pass 1 return to the
+// observation rows, and the pass-2 advances pass 1 counted leave the statistics.  The state buffer of pass 1 stays.
+__device__ __forceinline__ void revert_pass2(const Workspace& ws, float* __restrict__ obs, float obs_clip,
+                                             int64_t num_envs) {
+  const int64_t total = num_envs * 11;
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int64_t e = i / 11;
+    const int c = static_cast<int>(i - e * 11);
+    obs[e * kObs + 48 + c] = clip_obs(reinterpret_cast<const float*>(ws.tail1 + e * 3)[c], obs_clip);
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) ws.ctrl->stats.n_advanced -= ws.ctrl->last_adv2;
+}
+
 __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ CommitArgs a) {
   __shared__ float s_row[8][4][20];
   const AsParams& P = a.P;
@@ -759,14 +771,7 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
   const int64_t n = ctrl->n_reset_list;
   if (n == 0 && a.revert_if_none && !(a.peer_three_call && ctrl->any_reset)) {
-    if (blockIdx.x == 0 && threadIdx.x == 0) ctrl->stats.n_advanced -= ctrl->last_adv2;  // pass 2 is discarded
-    const int64_t total = a.num_envs * 11;
-    for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
-         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-      const int64_t e = i / 11;
-      const int c = static_cast<int>(i - e * 11);
-      a.obs[e * kObs + 48 + c] = clip_obs(reinterpret_cast<const float*>(a.ws.tail1 + e * 3)[c], a.obs_clip);
-    }
+    revert_pass2(a.ws, a.obs, a.obs_clip, a.num_envs);
     return;
   }
   uint2* st = a.ws.state[ctrl->parity ^ 1u];  // the buffer pass 1 speculated into and as_reset wrote
@@ -869,17 +874,10 @@ __global__ void __launch_bounds__(256) k_pass2_commit(const __grid_constant__ Co
 __global__ void __launch_bounds__(256) k_pass2_revert(Workspace ws, float* __restrict__ obs, float obs_clip,
                                                       int64_t num_envs, int32_t peer_three_call) {
   const bool commit = peer_three_call && ws.ctrl->any_reset;
-  const int64_t total = commit ? 0 : num_envs * 11;
-  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int64_t e = i / 11;
-    const int c = static_cast<int>(i - e * 11);
-    obs[e * kObs + 48 + c] = clip_obs(reinterpret_cast<const float*>(ws.tail1 + e * 3)[c], obs_clip);
-  }
+  if (!commit) revert_pass2(ws, obs, obs_clip, num_envs);
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     ws.ctrl->n_reset_list = 0;
     if (commit) ws.ctrl->parity ^= 1u;  // the speculated buffer becomes the current state
-    else ws.ctrl->stats.n_advanced -= ws.ctrl->last_adv2;  // the pass-2 advances pass 1 counted are discarded with pass 2
   }
 }
 

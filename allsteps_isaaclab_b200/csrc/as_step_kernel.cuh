@@ -76,7 +76,6 @@ struct Misc {  // lives at kOffMisc, never aliased
   unsigned int wcnt[kTile / 32][kNumCounters];  // per-warp step counters
   float wreward[kTile / 32];
   unsigned int is_last;
-  unsigned int fold[kNumCounters];
   ResetTables rt;
   // exchanged between the two roles at the CTA barrier
   float red_energy[kTile];   // sum_j |joint_vel * action|, ENV:365
@@ -405,45 +404,41 @@ __device__ __forceinline__ unsigned slot_sum(const Ctrl* ctrl, int which) {
   return __reduce_add_sync(0xffffffffu, v);
 }
 
-// Folds the slots into ctrl->stats and clears them.  Called by one CTA (>= 64 threads) after the step kernel.
-__device__ __forceinline__ void fold_stats(Ctrl* ctrl, unsigned int* fold, int64_t num_envs) {
-  const int t = threadIdx.x;
-  const int lane = t & 31;
-  // one warp per counter, one lane per slot.  No kernel is adding to the slots any more (stream order), so plain
-  // L2 loads followed by independent zeroing stores do: one memory round trip for the whole fold.
-  for (int c = t >> 5; c < kNumCounters; c += blockDim.x >> 5) {
+// Folds the slots into ctrl->stats and clears them: one warp, one lane per slot, lane 0 writes the totals.  Nobody may
+// still be adding to the slots (the caller is the last CTA of the step kernel, or a kernel behind it in stream order),
+// so plain L2 loads followed by independent zeroing stores do: one memory round trip for the whole fold.  Returns the
+// step's reset count in every lane.
+__device__ __forceinline__ unsigned fold_stats_warp(Ctrl* ctrl, int64_t num_envs, int lane) {
+  unsigned tot[kNumCounters];
+#pragma unroll
+  for (int c = 0; c < kNumCounters; ++c) {
     const unsigned v = __ldcg(&ctrl->slots[lane][c]);
     __stcg(&ctrl->slots[lane][c], 0u);
-    const unsigned r = c == kCntLevelMax ? __reduce_max_sync(0xffffffffu, v) : __reduce_add_sync(0xffffffffu, v);
-    if (lane == 0) fold[c] = r;
+    tot[c] = c == kCntLevelMax ? __reduce_max_sync(0xffffffffu, v) : __reduce_add_sync(0xffffffffu, v);
   }
-  float rsum = 0.0f;
-  if (t >= 32 && t < 64) {
-    rsum = __ldcg(&ctrl->slot_reward[lane]);
-    __stcg(&ctrl->slot_reward[lane], 0.0f);
+  float rsum = __ldcg(&ctrl->slot_reward[lane]);
+  __stcg(&ctrl->slot_reward[lane], 0.0f);
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) rsum += __shfl_xor_sync(0xffffffffu, rsum, o);
-  }
-  __syncthreads();
-  if (t == 0) {
+  for (int o = 16; o > 0; o >>= 1) rsum += __shfl_xor_sync(0xffffffffu, rsum, o);
+  if (lane == 0) {
     AsStats& st = ctrl->stats;
     st.n_envs = num_envs;
-    st.n_reset = fold[kCntReset];
-    st.n_terminated = fold[kCntTerminated];
-    st.n_time_out = fold[kCntTimeOut];
-    st.n_fell = fold[kCntFell];
-    st.n_so_fast = fold[kCntSoFast];
-    st.n_died = fold[kCntDied];
-    st.n_advanced = static_cast<int64_t>(fold[kCntAdvanced1]) + fold[kCntAdvanced2];
-    st.sum_target_index = fold[kCntSumIndex];
-    st.n_regenerated = fold[kCntRegen];
-    st.level = fold[kCntLevelMax];
+    st.n_reset = tot[kCntReset];
+    st.n_terminated = tot[kCntTerminated];
+    st.n_time_out = tot[kCntTimeOut];
+    st.n_fell = tot[kCntFell];
+    st.n_so_fast = tot[kCntSoFast];
+    st.n_died = tot[kCntDied];
+    st.n_advanced = static_cast<int64_t>(tot[kCntAdvanced1]) + tot[kCntAdvanced2];
+    st.sum_target_index = tot[kCntSumIndex];
+    st.n_regenerated = tot[kCntRegen];
+    st.level = tot[kCntLevelMax];
     st.step_counter = static_cast<int64_t>(ctrl->step_counter);
-    st.n_missed = fold[kCntMissed];
-    ctrl->last_adv2 = fold[kCntAdvanced2];
+    st.sum_reward = static_cast<double>(rsum);
+    st.n_missed = tot[kCntMissed];
+    ctrl->last_adv2 = tot[kCntAdvanced2];
   }
-  if (t == 32) ctrl->stats.sum_reward = static_cast<double>(rsum);
-  __syncthreads();
+  return tot[kCntReset];
 }
 
 // ENV:471-472 promotion rule on step statistics (this shard's, or summed over ranks).
@@ -539,55 +534,35 @@ __device__ __forceinline__ void peer_publish(Ctrl* ctrl, const PeerArgs& peer, c
   ctrl->peer_epoch = static_cast<uint32_t>(epoch == 0xFFFFFFFFull ? 0ull : epoch);
 }
 
-// One-warp version of fold_stats (the last CTA of the fused step kernel folds with the warp that took the ticket).
-__device__ __forceinline__ void fold_stats_warp(Ctrl* ctrl, int64_t num_envs, int lane, unsigned& n_reset_out) {
-  unsigned tot[kNumCounters];
-#pragma unroll
-  for (int c = 0; c < kNumCounters; ++c) {
-    const unsigned v = __ldcg(&ctrl->slots[lane][c]);
-    __stcg(&ctrl->slots[lane][c], 0u);
-    tot[c] = c == kCntLevelMax ? __reduce_max_sync(0xffffffffu, v) : __reduce_add_sync(0xffffffffu, v);
-  }
-  float rsum = __ldcg(&ctrl->slot_reward[lane]);
-  __stcg(&ctrl->slot_reward[lane], 0.0f);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) rsum += __shfl_xor_sync(0xffffffffu, rsum, o);
-  n_reset_out = tot[kCntReset];
-  if (lane == 0) {
-    AsStats& st = ctrl->stats;
-    st.n_envs = num_envs;
-    st.n_reset = tot[kCntReset];
-    st.n_terminated = tot[kCntTerminated];
-    st.n_time_out = tot[kCntTimeOut];
-    st.n_fell = tot[kCntFell];
-    st.n_so_fast = tot[kCntSoFast];
-    st.n_died = tot[kCntDied];
-    st.n_advanced = static_cast<int64_t>(tot[kCntAdvanced1]) + tot[kCntAdvanced2];
-    st.sum_target_index = tot[kCntSumIndex];
-    st.n_regenerated = tot[kCntRegen];
-    st.level = tot[kCntLevelMax];
-    st.step_counter = static_cast<int64_t>(ctrl->step_counter);
-    st.sum_reward = static_cast<double>(rsum);
-    st.n_missed = tot[kCntMissed];
-    ctrl->last_adv2 = tot[kCntAdvanced2];
-  }
+// Closes a fused step (one thread, after the fold): decides the promotion of ENV:471 for the next step on `promote_on`
+// (this shard's statistics, or their sum over the shards), reports the step's reset count, flips the state parity,
+// advances the Philox step counter and empties the reset and regeneration lists for the next step.
+__device__ __forceinline__ void close_step(const StepArgs& a, Ctrl* ctrl, const AsStats& promote_on, unsigned n_reset) {
+  ctrl->stats_folded = 0;
+  ctrl->promote_cur = promotion_decision(a.P, promote_on);
+  if (a.rows.n_reset) *a.rows.n_reset = static_cast<int32_t>(a.want_reset_list ? ctrl->n_reset_list : n_reset);
+  ctrl->parity ^= 1u;
+  ctrl->step_counter += 1ull;
+  ctrl->n_reset_list = 0;
+  ctrl->n_regen_list = 0;
 }
 
 // The last CTA of a fused step kernel (every CTA takes a ticket once its counters are out).  When the launch is
-// allowed to close its own step (StepArgs::self_finish: shard-local promotion, no regeneration kernels behind it) and
-// at least one env reset -- so that pass 2 for everybody was the right assumption (DRL:360) -- it does what
-// k_fixup_finish's finisher does: fold the statistics, decide the promotion of ENV:471 for the next step, flip the state
-// parity, advance the Philox step counter.  k_fixup_finish then finds step_state == 2 and returns at once.
+// allowed to close its own step (StepArgs::self_finish: no regeneration kernels behind it, no all-reduce announced) and
+// at least one env reset -- so that pass 2 for everybody was the right assumption (DRL:360) -- it folds the statistics
+// and closes the step; k_fixup_finish then finds step_state == 2 and returns at once.  Without peers the reset count is
+// read before anything is folded: a step in which nobody reset leaves its counters in the slots for k_fixup_finish.
+// (The two branches stay apart: merged into one, they change the register allocation of the fused instantiations, and
+// the launch-bound small batches, whose step ends with this CTA, measured slower.)
 __device__ __forceinline__ void close_step_by_last_cta(const StepArgs& a, Ctrl* ctrl, int lane) {
   __threadfence();
   unsigned state = 1u;
   if (a.self_finish) {
-    unsigned nr;
     if (a.peer.world > 0) {
       // sharded, promotion on the global mean: fold, exchange the ten counters with every peer over NVLink (this warp;
       // a peer's last CTA answers when ITS step kernel gets there), then decide on the sums -- the exchange and the
       // finish ride in the step kernel's last CTA instead of two more launches
-      fold_stats_warp(ctrl, a.num_envs, lane, nr);
+      const unsigned nr = fold_stats_warp(ctrl, a.num_envs, lane);
       __syncwarp();
       __threadfence();
       long long got[kPeerCounters];
@@ -600,33 +575,14 @@ __device__ __forceinline__ void close_step_by_last_cta(const StepArgs& a, Ctrl* 
       __syncwarp();
       const long long global_resets = __shfl_sync(0xffffffffu, n_to == 0 ? got[1] /* AsStats::n_reset */ : static_cast<long long>(nr), 0);
       if (global_resets > 0 || (a.P.flags & AS_FLAG_SKIP_PASS2)) {
-        if (lane == 0) {
-          ctrl->stats_folded = 0;
-          ctrl->promote_cur = promotion_decision(a.P, ctrl->gx.stats);
-          if (a.rows.n_reset) *a.rows.n_reset = static_cast<int32_t>(a.want_reset_list ? ctrl->n_reset_list : nr);
-          ctrl->parity ^= 1u;
-          ctrl->step_counter += 1ull;
-          ctrl->n_reset_list = 0;
-          ctrl->n_regen_list = 0;
-        }
+        if (lane == 0) close_step(a, ctrl, ctrl->gx.stats, nr);
         state = 2u;
       }  // else: nobody reset anywhere -- k_fixup_finish redoes the step without pass 2, on ctrl->gx (already folded)
-    } else {
-      const unsigned n_reset = slot_sum(ctrl, kCntReset);
-      if (n_reset > 0 || (a.P.flags & AS_FLAG_SKIP_PASS2)) {
-        fold_stats_warp(ctrl, a.num_envs, lane, nr);
-        __syncwarp();
-        if (lane == 0) {
-          ctrl->stats_folded = 0;
-          ctrl->promote_cur = promotion_decision(a.P, ctrl->stats);
-          if (a.rows.n_reset) *a.rows.n_reset = static_cast<int32_t>(a.want_reset_list ? ctrl->n_reset_list : nr);
-          ctrl->parity ^= 1u;
-          ctrl->step_counter += 1ull;
-          ctrl->n_reset_list = 0;
-          ctrl->n_regen_list = 0;
-        }
-        state = 2u;
-      }
+    } else if (slot_sum(ctrl, kCntReset) > 0 || (a.P.flags & AS_FLAG_SKIP_PASS2)) {
+      const unsigned nr = fold_stats_warp(ctrl, a.num_envs, lane);
+      __syncwarp();
+      if (lane == 0) close_step(a, ctrl, ctrl->stats, nr);
+      state = 2u;
     }
   }
   if (lane == 0) {
@@ -639,8 +595,7 @@ __device__ __forceinline__ void close_step_by_last_cta(const StepArgs& a, Ctrl* 
 // promotion every CTA applied, advances the Philox step counter -- a reset that follows draws at the advanced counter.
 __device__ __forceinline__ void close_pass1_by_last_cta(const StepArgs& a, Ctrl* ctrl, int lane) {
   __threadfence();
-  unsigned nr;
-  fold_stats_warp(ctrl, a.num_envs, lane, nr);
+  fold_stats_warp(ctrl, a.num_envs, lane);
   __syncwarp();
   if (lane == 0) {
     ctrl->promote_cur = 0;
@@ -1615,11 +1570,12 @@ __global__ void __launch_bounds__(kThreads, AS_STEP_MIN_CTAS) k_step(const __gri
   process_tile<MODE, FULL, EXACT, FAST, PACKED, PRE>(a, tile, phase_root, phase_joint, smem);
 }
 
-// as_fold_stats: fold early so that the caller can all-reduce the statistics before as_finish_step.
-__global__ void __launch_bounds__(128) k_fold_early(Ctrl* ctrl, int64_t num_envs) {
-  __shared__ unsigned int fold[kNumCounters];
-  if (__ldcg(&ctrl->step_state) == 2u) return;  // (the step closed itself: the totals are in ctrl->stats already)
-  fold_stats(ctrl, fold, num_envs);
+// as_fold_stats: fold early so that the caller can all-reduce the statistics before as_finish_step.  One warp.  At most
+// once per step: when the step closed itself, or its last CTA folded for the peer exchange, the totals are in
+// ctrl->stats already and the slots are empty.
+__global__ void __launch_bounds__(32) k_fold_early(Ctrl* ctrl, int64_t num_envs) {
+  if (__ldcg(&ctrl->step_state) == 2u || __ldcg(&ctrl->stats_folded) != 0u) return;
+  fold_stats_warp(ctrl, num_envs, threadIdx.x);
   if (threadIdx.x == 0) ctrl->stats_folded = 1;
 }
 
@@ -1641,13 +1597,12 @@ enum ExchangeMode {
 __global__ void __launch_bounds__(128) k_peer_exchange(Ctrl* ctrl, const __grid_constant__ PeerArgs peer,
                                                        int64_t num_envs, int grid_cells,
                                                        const __grid_constant__ AsParams P, int mode) {
-  __shared__ unsigned int fold[kNumCounters];
   __shared__ unsigned int s_timeouts;
   asm volatile("griddepcontrol.launch_dependents;");  // the finish kernel may become resident; it waits for us
   asm volatile("griddepcontrol.wait;" ::: "memory");  // the step kernel has completed and flushed
   const int tid = threadIdx.x;
   if (mode == kExchangeFused) {
-    fold_stats(ctrl, fold, num_envs);
+    if (tid < 32 && __ldcg(&ctrl->stats_folded) == 0u) fold_stats_warp(ctrl, num_envs, tid);  // (unless as_fold_stats did)
     if (tid == 0) ctrl->stats_folded = 1;
     __syncthreads();
   }
@@ -1758,7 +1713,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_fixup_finish(const __grid_const
   __syncthreads();
   if (misc->is_last == 0) return;
   __threadfence();
-  if (!prefolded) fold_stats(ctrl, misc->fold, a.num_envs);
+  if (!prefolded && tid < 32) fold_stats_warp(ctrl, a.num_envs, tid);
   if (a.P.flags & AS_FLAG_GRID_CURRICULUM) {
     // this step's episode outcomes join the difficulty-grid histograms (the sum over all shards when one was handed in)
     for (int i = tid; i < kMaxGridBins; i += blockDim.x) {
@@ -1770,14 +1725,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_fixup_finish(const __grid_const
     for (int i = tid; i < kMaxGridBins; i += blockDim.x) ctrl->grid_delta_att[i] = ctrl->grid_delta_succ[i] = 0u;
   }
   if (tid == 0) {
-    ctrl->stats_folded = 0;
-    const AsStats* g = a.global_stats ? &a.global_stats->stats : &ctrl->stats;
-    ctrl->promote_cur = promotion_decision(a.P, *g);
-    if (a.rows.n_reset) *a.rows.n_reset = static_cast<int32_t>(a.want_reset_list ? ctrl->n_reset_list : ctrl->stats.n_reset);
-    ctrl->parity ^= 1u;
-    ctrl->step_counter += 1ull;
-    ctrl->n_reset_list = 0;
-    ctrl->n_regen_list = 0;
+    close_step(a, ctrl, a.global_stats ? a.global_stats->stats : ctrl->stats, static_cast<unsigned>(ctrl->stats.n_reset));
     ctrl->blocks_done2 = 0;
     if (need_fixup) {
       ctrl->fixup_ran += 1;

@@ -286,14 +286,17 @@ int as_read_stats(AsHandle* h, AsStats* host_out, void* stream); /* synchronises
  * path, `mean(curr_target_index) > 12` over ALL envs, ENV:471) --------------------------------------------------
  * One process per GPU.  as_peer_create allocates this shard's 4-KB exchange buffer and returns its CUDA IPC handle
  * (AS_PEER_HANDLE_BYTES bytes); the caller gathers the handles of all ranks (any transport, e.g.
- * torch.distributed.all_gather) and hands them, in rank order, to as_peer_connect.  From then on
- * as_finish_step(h, NULL, stream) launches ONE small kernel that folds this shard's step counters, stores them into
- * every peer's buffer through NVLink, waits for the peers' stores of the same step and sums them, followed by the
- * finish kernel deciding on that global sum -- the fused replacement of as_fold_stats + NCCL all-reduce +
- * as_finish_step(global).  Every rank must call as_step_fused / as_finish_step the same number of times.  A peer that
- * does not show up within 2 s is counted in AsStats-independent `*timeouts` of as_peer_status and its counters are
- * taken as zero (no hang).  world == 1 is allowed (self-exchange).  as_global_stats_device_ptr: the summed AsStats
- * (first 10 fields; the rest is this shard's). */
+ * torch.distributed.all_gather) and hands them, in rank order, to as_peer_connect.  From then on the last CTA of the
+ * fused step kernel folds this shard's step counters, stores them into every peer's buffer through NVLink, waits for
+ * the peers' stores of the same step, sums them and closes the step on that global sum (as_finish_step(h, NULL,
+ * stream) is left with a step in which no env of any shard reset).  When the step kernel leaves the step open
+ * (AS_STEP_DEFER_FINISH, or the regeneration kernels behind it), as_finish_step(h, NULL, stream) launches ONE small
+ * kernel for the fold and the exchange, followed by the finish kernel deciding on the sum.  Either way this is the
+ * fused replacement of as_fold_stats + NCCL all-reduce + as_finish_step(global).  Every rank must call as_step_fused /
+ * as_finish_step the same number of times.  A peer that does not deliver within ALLSTEPS_PEER_TIMEOUT_MS (default
+ * 10 s; 0 = no limit) is counted in `*timeouts` of as_peer_status; the step closes on this shard's own record (a partial
+ * sum is never used) and every later step is refused with the sticky AS_ERR_PEER (no hang).  world == 1 is allowed
+ * (self-exchange).  as_global_stats_device_ptr: the summed AsStats (first 10 fields; the rest is this shard's). */
 #define AS_PEER_HANDLE_BYTES 64
 #define AS_MAX_PEERS 16
 int as_peer_create(AsHandle* h, int world, int rank, void* ipc_handle_out);
